@@ -259,6 +259,34 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+def dump_outputs(sim, out_dir):
+    """Write what a caller of the device-resident step holds after the last timed tick, as float32 .npy files under
+    `out_dir` (at most about 45 MB, whatever the size): the per-agent vectors, and the observation records (raw
+    bytes), episode infos and next built-in-policy actions, each for a fixed seeded sample of agent slots (all slots
+    for the per-agent vectors up to 2^19 of them).  The sampled slots are written beside them as float64 index arrays,
+    so that two builds can be compared output for output."""
+    import torch
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    n = sim.E * sim.P
+    perm = np.random.default_rng(0).permutation(n)
+    slots = {"slots": np.sort(perm[:1 << 19]), "wide_slots": np.sort(perm[:1 << 14]), "obs_slots": np.sort(perm[:256])}
+    idx = {k: torch.from_numpy(v).to(sim.obs.device) for k, v in slots.items()}
+    arrays = {"rewards": sim.rewards[idx["slots"]], "terminated": sim.terminated[idx["slots"]],
+              "truncated": sim.truncated[idx["slots"]], "mask": sim.mask[idx["slots"]],
+              "info_valid": sim.info_valid[idx["slots"]], "episode_done": sim.episode_done,
+              "info": sim.info[idx["wide_slots"]], "actions": sim.actions.view(n, 12)[idx["wide_slots"]],
+              "obs": sim.obs[idx["obs_slots"]]}
+    # the max-level columns of an episode info are NaN where the key is absent; levels are >= 0, so the dump, whose
+    # arrays are all finite, writes -1 there instead
+    levels = slice(SPEC["IN_MAXLVL_ARMOR"], SPEC["IN_MAXLVL_CONSUMABLE"] + 1)
+    arrays["info"][:, levels] = torch.nan_to_num(arrays["info"][:, levels], nan=-1.0)
+    for name, t in arrays.items():
+        np.save(out / f"{name}.npy", t.cpu().numpy().astype(np.float32))
+    for name, v in slots.items():
+        np.save(out / f"{name}.npy", v.astype(np.float64))
+
+
 def run_native(args):
     import torch
     import torch.distributed as dist
@@ -332,6 +360,8 @@ def run_native(args):
     step_ms, obs_ms, n_timed = sim.timing_read()
     sim.timing(False)
     sums, counts, counters = sim.stats(clear=False)
+    if args.dump_outputs and rank == 0:          # rank 0's envs only: one dump within the size bound at any world size
+        dump_outputs(sim, args.dump_outputs)
     # ---- survival leg (SURVEY.md 8d "run 1024 ticks from reset so the alive-fraction decay is included"): a whole
     # episode under the scripted forager policy (nmmo_forage_actions: walk to water / foliage when hungry), whose
     # population decays like the published trained-policy runs (BASELINE.md 2: alive 0.83 / 0.53 / 0.25 / 0.13 at ticks
@@ -741,7 +771,11 @@ def main():
     ap.add_argument("--tf32", type=int, default=0, help="config4: allow TF32 in the policy's matmuls / convolutions (the reference runs fp32)")
     ap.add_argument("--rollout-batch", type=int, default=131072)
     ap.add_argument("--steady-steps", type=int, default=1023, help="ticks of the survival leg (one episode under the scripted forager policy; 0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of their last step to DIR/<name>.npy (native step benchmark only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.what != "step" or args.impl != "native"):
+        ap.error("--dump-outputs applies to the native step benchmark only")
     if args.what == "rollout":
         run_rollout(args)
     elif args.what == "config4":

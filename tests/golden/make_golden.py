@@ -7,8 +7,8 @@ What is pinned.  The reference's stat / reward wrapper stack
     agent_zoo/takeru/reward_wrapper.py          RewardWrapper.observation / reward_terminated_truncated_info
     agent_zoo/neurips23_start_kit/reward_wrapper.py   same + RewardWrapper.action
     agent_zoo/yaofeng/reward_wrapper.py         same (hp / exp / defense / attack / gold bonuses, dangerous-NPC mask)
-is imported UNMODIFIED from /root/reference (only the missing third-party modules pettingzoo and
-nmmo are replaced by minimal stubs: a BaseParallelWrapper that stores `env`, the EventCode
+is imported UNMODIFIED from the reference checkout named by $NMMO_REFERENCE (only the missing
+third-party modules pettingzoo and nmmo are replaced by minimal stubs: a BaseParallelWrapper that stores `env`, the EventCode
 constants, the item class lists) and driven through whole episodes by a fake `nmmo.Env` that
 replays an engine trajectory.  Its outputs -- reward, terminated, truncated, episode info dict and
 the edited ActionTargets masks -- are stored; tests/test_golden.py requires the CPU oracle's wrapper
@@ -17,7 +17,7 @@ part to reproduce them bit for bit, and the GPU tests require the CUDA path to e
 What is NOT pinned.  The engine trajectory itself comes from oracle/nmmo_oracle.c (the nmmo 2.1
 engine is not available here), so these vectors pin rows a-4..a-10 of SURVEY.md section 8, not a-3/a-16.
 
-Run in the build container (needs /root/reference):  python tests/golden/make_golden.py
+Run with a checkout of the reference baselines repository:  NMMO_REFERENCE=<checkout> python tests/golden/make_golden.py
 """
 from __future__ import annotations
 
@@ -30,11 +30,13 @@ import numpy as np
 
 HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent.parent
-REF = Path("/root/reference")
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
 
 from nmmo_b200.config import SPEC, ObsLayout  # noqa: E402
+from util import reference_file  # noqa: E402
+
+REF = reference_file()
 
 INFO_KEYS = {  # episode-info key -> column of the nm_info record (include/nmmo_spec.h)
     "length": "IN_LENGTH", "return": "IN_RETURN",
@@ -310,7 +312,7 @@ def run_case(name, agent, ticks, seed, wrapper_over=None, **engine_over):
 
 
 def main():
-    assert REF.exists(), "needs the reference checkout at /root/reference"
+    assert REF is not None, "set NMMO_REFERENCE to a checkout of the reference baselines repository"
     install_stubs()
     sys.path.insert(0, str(REF))
     run_case("takeru_small", "takeru", 140, 3, NC_HORIZON=120, NC_RES_DEPLETION=2, NC_SPAWN_IMMUNITY=3, NC_WEAPON_DROP_THR=1 << 30)

@@ -3,7 +3,7 @@
 
 `clean_pufferl.evaluate` and `clean_pufferl.train` cannot be imported here (pufferlib is absent) and the
 code in question is inline in those two functions, so this script cuts the exact statements out of
-/root/reference/reinforcement_learning/clean_pufferl.py by their first/last lines --
+reinforcement_learning/clean_pufferl.py of the reference checkout ($NMMO_REFERENCE) by their first/last lines --
     the masked append   "learner_mask = torch.Tensor(mask * data.policy_pool.mask)" ... "ptr += len(indices)"   (:333-349)
     the sort            "idxs = sorted(range(len(data.sort_keys)), key=data.sort_keys.__getitem__)"            (:413)
     the GAE loop        "advantages = torch.zeros(config.batch_size, device=data.device)" ... end of the loop  (:425-436)
@@ -11,7 +11,7 @@ code in question is inline in those two functions, so this script cuts the exact
 outputs are stored in tests/golden/rollout_*.npz; tests/test_rollout.py requires oracle/rollout_oracle.py to
 reproduce them bit for bit, and the GPU tests require the CUDA path to equal the oracle bit for bit.
 
-Run in the build container (needs /root/reference):  python tests/golden/make_golden_rollout.py
+Run with a checkout of the reference baselines repository:  NMMO_REFERENCE=<checkout> python tests/golden/make_golden_rollout.py
 """
 from __future__ import annotations
 
@@ -24,9 +24,11 @@ import torch
 
 HERE = Path(__file__).resolve().parent
 import sys
+sys.path.insert(0, str(HERE.parent.parent))
 sys.path.insert(0, str(HERE.parent))
 from rollout_inputs import step_stream  # noqa: E402
-SRC = Path("/root/reference/reinforcement_learning/clean_pufferl.py")
+from util import reference_file  # noqa: E402
+SRC = reference_file("reinforcement_learning", "clean_pufferl.py")
 
 
 def cut(lines, first, last_pred):
@@ -84,7 +86,7 @@ def run_case(name, seed, batch_size, n_slots, stride, p_alive, p_done, p_learner
 
 
 def main():
-    assert SRC.exists(), "needs the reference checkout at /root/reference"
+    assert SRC is not None, "set NMMO_REFERENCE to a checkout of the reference baselines repository"
     run_case("rollout_small", 1, batch_size=256, n_slots=96, stride=32, p_alive=0.9, p_done=0.05, p_learner=1.0, gamma=0.99, lam=0.95)
     run_case("rollout_pool", 2, batch_size=700, n_slots=128, stride=48, p_alive=0.8, p_done=0.1, p_learner=0.7, gamma=0.99, lam=0.95)
     run_case("rollout_nodone", 3, batch_size=300, n_slots=64, stride=16, p_alive=0.95, p_done=0.0, p_learner=1.0, gamma=0.97, lam=0.9)

@@ -1,10 +1,10 @@
 """The reference's real curricula -> device task tables (nmmo_b200/curriculum.py), and team-task semantics on the oracle.
 
-The spec modules and the embedding pickles live under /root/reference; the translated tables are committed under
-nmmo_b200/data/ (tools/make_task_tables.py).  Tests that need the reference checkout skip without it.
+The spec modules and the embedding pickles live in the reference baselines repository; the translated tables are
+committed under nmmo_b200/data/ (tools/make_task_tables.py).  Tests that need a checkout of the reference (named by
+$NMMO_REFERENCE) skip without it.
 """
 import textwrap
-from pathlib import Path
 
 import numpy as np
 import pytest
@@ -12,10 +12,10 @@ import pytest
 from nmmo_b200.config import SPEC
 from nmmo_b200.curriculum import (Unsupported, load_spec_module, load_spec_pickle, load_table, spec_name, spec_to_row, translate)
 from nmmo_b200.tasks import EVENT, ITEM, PRED, SKILL, TF_RELATIVE_TARGET, TF_TEAM, task_row
-from util import SMALL, build_world
+from util import SMALL, build_world, reference_file
 
-REF = Path("/root/reference")
-needs_ref = pytest.mark.skipif(not (REF / "neurips23_evaluation").exists(), reason="reference checkout not present")
+REF = reference_file("neurips23_evaluation")
+needs_ref = pytest.mark.skipif(REF is None, reason="no reference checkout: set NMMO_REFERENCE")
 
 
 def test_committed_tables():
@@ -24,6 +24,11 @@ def test_committed_tables():
     assert h["unsupported"] == [] and len(set(h["names"])) == 63
     assert h["names"][0] == "Task_TickGE_(num_tick:1024)_reward_to:agent" and h["rows"][0].tolist()[:2] == [PRED["TICK_GE"], 1024]
     assert np.isfinite(h["embed"].astype(np.float32)).all() and np.abs(h["embed"].astype(np.float32)).max() > 0.1
+    # spot checks against the source (heldout_evaluation_task.py:43-50, :112-119)
+    r = dict(zip(h["names"], h["rows"].tolist()))
+    assert r["Task_DefeatEntity_(agent_type:npc_level:3_num_agent:20)_reward_to:agent"][:4] == [PRED["DEFEAT_ENTITY"], 0, 3, 20]
+    assert r["Task_FullyArmed_(combat_style:Mage_level:3_num_agent:1)_reward_to:agent"][:3] == [PRED["FULLY_ARMED"], SKILL["MAGE"], 3]
+    assert r["Task_CountEvent_(event:EARN_GOLD_N:20)_reward_to:agent"][:3] == [PRED["COUNT_EVENT"], EVENT["EARN_GOLD"], 20]
     s = load_table("sample_eval")
     assert s["rows"].shape[0] == 24 and s["embed"].shape == (24, 2048) and s["unsupported"] == []
     m = load_table("manual")
@@ -41,8 +46,8 @@ def test_committed_tables():
 
 @needs_ref
 def test_spec_module_and_pickle_agree_and_match_the_committed_table():
-    py = load_spec_module(REF / "neurips23_evaluation" / "heldout_evaluation_task.py")
-    pk = load_spec_pickle(REF / "neurips23_evaluation" / "heldout_task_with_embedding.pkl")
+    py = load_spec_module(REF / "heldout_evaluation_task.py")
+    pk = load_spec_pickle(REF / "heldout_task_with_embedding.pkl")
     assert [spec_name(s) for s in py] == [spec_name(s) for s in pk]
     rows_py, names, _, _, bad_py = translate(py)
     rows_pk, _, _, emb, bad_pk = translate(pk)

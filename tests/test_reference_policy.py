@@ -1,27 +1,26 @@
 """Rows a-14 / a-15 of SURVEY.md section 8: the reference's own policy consumes our observation record.
 
-agent_zoo/takeru/policy.py is loaded UNMODIFIED from /root/reference (the two absent third-party packages
-are stubbed: pufferlib.models.Policy -> torch.nn.Module, pufferlib.emulation.unpack_batched_obs -> the
-record unpacker of nmmo_b200/emulation.py, nmmo's EntityState column names -> include/nmmo_spec.h) and run
+agent_zoo/takeru/policy.py is loaded UNMODIFIED from the reference checkout named by $NMMO_REFERENCE (the two
+absent third-party packages are stubbed: pufferlib.models.Policy -> torch.nn.Module,
+pufferlib.emulation.unpack_batched_obs -> the record unpacker of nmmo_b200/emulation.py, nmmo's EntityState column names -> include/nmmo_spec.h) and run
 on observation records produced by the oracle.  It must find every alive agent's own row, produce one
 logit vector per action head with the width of the matching ActionTargets mask, mask exactly the invalid
-entries, and its greedy actions must be accepted by the engine step.  Skipped where the reference checkout
-is absent (the GPU box).
+entries, and its greedy actions must be accepted by the engine step.  Skipped where no reference checkout
+is at hand.
 """
 import importlib.util
 import sys
 import types
-from pathlib import Path
 
 import numpy as np
 import pytest
 
 from nmmo_b200.config import SPEC, ObsLayout
 from nmmo_b200.emulation import UnflattenContext, unpack_batched_obs
-from util import SMALL, build_world
+from util import SMALL, build_world, reference_file
 
-REF = Path("/root/reference/agent_zoo/takeru/policy.py")
-pytestmark = pytest.mark.skipif(not REF.exists(), reason="reference checkout not present")
+REF = reference_file("agent_zoo", "takeru", "policy.py")
+pytestmark = pytest.mark.skipif(REF is None, reason="no reference checkout: set NMMO_REFERENCE")
 
 
 def _load_reference_policy():

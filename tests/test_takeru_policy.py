@@ -2,7 +2,8 @@
 
 The reference module is loaded unmodified (third-party imports stubbed, see test_reference_policy.py), both networks get
 the same weights through ``state_dict`` (same parameter names), and logits / values are compared on oracle records --
-with and without the per-environment Market de-duplication.  Skipped where the reference checkout is absent."""
+with and without the per-environment Market de-duplication.  No outputs of the reference module are stored in this
+repository, so the test is skipped where no reference checkout ($NMMO_REFERENCE) is at hand."""
 import types
 
 import numpy as np
@@ -26,7 +27,7 @@ def _records(world, ticks=12, seed=4):
     return torch.from_numpy(np.concatenate(recs))
 
 
-@pytest.mark.skipif(not REF.exists(), reason="reference checkout not present")
+@pytest.mark.skipif(REF is None, reason="no reference checkout: set NMMO_REFERENCE")
 @pytest.mark.parametrize("dedup,sparse", [(False, False), (True, False), (True, True)])
 def test_same_weights_same_outputs_as_the_reference_module(dedup, sparse):
     torch.manual_seed(0)

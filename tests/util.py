@@ -1,6 +1,9 @@
 """Shared parity harness: drive the CUDA simulator and the CPU oracle with identical inputs."""
 from __future__ import annotations
 
+import os
+from pathlib import Path
+
 import numpy as np
 
 from nmmo_b200.config import SPEC, ObsLayout, make_config
@@ -8,6 +11,14 @@ from nmmo_b200.mapgen import generate_maps
 from nmmo_b200.tasks import default_curriculum, make_task_table
 
 SMALL = dict(NC_N_PLAYERS=16, NC_N_NPCS=32, NC_MAP_CENTER=32)
+
+
+def reference_file(*parts):
+    """A path in the checkout of the reference baselines repository (Meeso1/nmmo) named by $NMMO_REFERENCE, or None
+    when that variable is unset or the path does not exist there."""
+    root = os.environ.get("NMMO_REFERENCE")
+    path = Path(root, *parts) if root else None
+    return path if path is not None and path.exists() else None
 
 
 def build_world(agent="takeru", n_maps=4, map_seed=7, task_dim=None, env_over=None, wrapper_over=None, **engine_over):
