@@ -103,6 +103,21 @@ static size_t step_smem_bytes(const NmParams &p, bool items_in_place = false) {
   s += a16(1024); s += a16((size_t)p.P * 16); s += a16((size_t)p.P * 8); s += a16(std::max<size_t>(4096, (size_t)p.R * 8) + 128); s += a16((size_t)p.R * 4); s += a16(NM_DEPL_CAP * 2); s += 4096; s += a16(p.P); s += a16((size_t)p.P * 4) + 64;
   return s + 128;
 }
+// four environments per CTA (VSmall4): shared memory of one environment, and its HBM workspace (the carve_ws arrays of
+// step_body<VSmall4>, incl. the event ring); the scratch also holds the Move position index, and the depleted-tile
+// list is used in place
+static size_t step4_smem_bytes(const NmParams &p) {
+  size_t s = 0;
+  s += a16((size_t)EA_N * p.R * 2); s += a16((size_t)p.S * p.S / 2);
+  s += a16((size_t)((p.S * p.S + 31) / 32) * 4); s += 2 * a16((size_t)((p.CAP + 31) / 32) * 4);
+  s += a16(p.P); s += a16(p.N); s += a16((size_t)p.N * 2); s += a16((size_t)VSmall4::kNpcHash * 2);
+  s += a16(std::max<size_t>(4096, (size_t)p.R * 8)); s += a16((size_t)p.R * 4); s += a16(32 * 4); s += 16;
+  return s + 128;
+}
+static size_t step4_ws_bytes(const NmParams &p) {
+  return a16((size_t)p.P * p.cfg[NC_N_INV] * 2) + a16((size_t)12 * p.P * 2) + a16((size_t)NM_EV_CAP * 8) + a16((size_t)p.P * 4) +
+         a16((size_t)p.P * 16) + a16((size_t)p.P * 8) + a16(p.P);
+}
 static size_t obs_smem_bytes(const NmParams &p) {
   size_t s = 0;
   int NINV = p.cfg[NC_N_INV];
@@ -184,12 +199,14 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   // the small step kernel runs two environments per CTA (they walk the code together) when both fit
   p.half_smem = (int)((h->step_smem + 127) & ~(size_t)127);
   p.envs_per_cta = (!p.big && 2 * p.half_smem <= max_smem) ? 2 : 1;
-  // three environments per CTA (item table and event ring in place in HBM / L2) when they fit
-  int want3 = 1;
-  if (const char *ov = getenv("NMMO_B200_ENVS_PER_CTA")) want3 = atoi(ov) == 3;      // test hook: 1 / 2 / 3
-  if (!p.big && want3) {
-    const size_t s3 = (step_smem_bytes(p, true) + 127) & ~(size_t)127;
-    if (3 * s3 <= (size_t)max_smem) { p.envs_per_cta = 3; p.half_smem = (int)s3; h->step_smem = s3; }
+  // four environments per CTA (VSmall4) when they fit, else three (item table and event ring in place in HBM / L2)
+  int want = 4;
+  if (const char *ov = getenv("NMMO_B200_ENVS_PER_CTA")) want = atoi(ov);      // test hook: 1 / 2 / 3 / 4
+  const size_t s4 = (step4_smem_bytes(p) + 127) & ~(size_t)127, s3 = (step_smem_bytes(p, true) + 127) & ~(size_t)127;
+  if (!p.big && want == 4 && p.P <= VSmall4::kThreads && p.R <= 2 * VSmall4::kThreads && 4 * s4 <= (size_t)max_smem) {
+    p.envs_per_cta = 4; p.half_smem = (int)s4; h->step_smem = s4;
+  } else if (!p.big && want >= 3 && 3 * s3 <= (size_t)max_smem) {
+    p.envs_per_cta = 3; p.half_smem = (int)s3; h->step_smem = s3;
   }
   if (getenv("NMMO_B200_NO_DEPL_LIST")) p.no_depl_list = 1;      // test hook
   p.ev_cap = p.big ? VBig::kEvCap : VSmall::kEvCap;
@@ -199,12 +216,13 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   }
   {   // the opt-in limit is a property of the kernel, not of the handle: several handles of different shapes may
       // be alive in one process, so it only ever grows (per device)
-    static int step_attr[3][64] = {{0}}, obs_attr[2][64] = {{0}};
+    static int step_attr[4][64] = {{0}}, obs_attr[2][64] = {{0}};
     const int need_step = p.envs_per_cta * p.half_smem, need_obs = (int)h->obs_smem, d = device & 63, b = p.big;
-    const int sk = b ? 1 : (p.envs_per_cta == 3 ? 2 : 0);
+    const int sk = b ? 1 : (p.envs_per_cta == 3 ? 2 : p.envs_per_cta == 4 ? 3 : 0);
     if (need_step > step_attr[sk][d]) {
       if (sk == 1) CU(cudaFuncSetAttribute(nmmo_step_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
       else if (sk == 2) CU(cudaFuncSetAttribute(nmmo_step3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
+      else if (sk == 3) CU(cudaFuncSetAttribute(nmmo_step4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
       else CU(cudaFuncSetAttribute(nmmo_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
       step_attr[sk][d] = need_step;
     }
@@ -224,10 +242,11 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
       const bool std_shape = std_cfg && !b && memcmp(&p.L, &sl, sizeof(sl)) == 0 && p.P == StdShape::P && p.N == StdShape::N && p.R == StdShape::R &&
                              p.S == StdShape::S && p.CAP == StdShape::CAP && p.cfg[NC_N_INV] == StdShape::NINV;
       h->obs_std = std_shape && p.ICAP == StdShape::ICAP && p.cfg[NC_VISION] == StdShape::VIS;
-      h->step_std = std_shape && p.envs_per_cta == 3;
+      h->step_std = std_shape && p.envs_per_cta >= 3;
       if (const char *ov = getenv("NMMO_B200_NO_STD_OBS")) { if (atoi(ov) == 1) h->obs_std = false; }      // test hooks: the generic kernels on the default shape
       if (const char *ov = getenv("NMMO_B200_NO_STD_STEP")) { if (atoi(ov) == 1) h->step_std = false; }
-      if (h->step_std) CU(cudaFuncSetAttribute(nmmo_step3_std_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
+      if (h->step_std) CU(cudaFuncSetAttribute(p.envs_per_cta == 4 ? nmmo_step4_std_kernel : nmmo_step3_std_kernel,
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
       // big family: the configs[4] shape
       h->big_std = std_cfg && b && memcmp(&p.L, &sl, sizeof(sl)) == 0 && p.P == StdShape5::P && p.N == StdShape5::N && p.R == StdShape5::R &&
                    p.S == StdShape5::S && p.CAP == StdShape5::CAP && p.cfg[NC_N_INV] == StdShape5::NINV && p.cfg[NC_VISION] == StdShape5::VIS;
@@ -242,6 +261,7 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   const size_t ent_i16 = p.big ? (size_t)NM_BIG_ENT_STRIDE * p.R : (size_t)EA_N * p.R;      // int16 per env
   DA(p.ent, E * ent_i16); DA(p.item, E * IS_N * p.CAP); DA(p.map, E * p.S * p.S / 2);
   if (p.big) { p.ws_bytes = step_big_ws_bytes(p); DA(p.ws, E * p.ws_bytes); }
+  else if (p.envs_per_cta == 4) { p.ws_bytes = step4_ws_bytes(p); DA(p.ws, E * p.ws_bytes); }
   else if (p.envs_per_cta == 3) { p.ws_bytes = a16((size_t)NM_EV_CAP * 8); DA(p.ws, E * p.ws_bytes); }
   uint8_t *dmaps; DA(dmaps, (size_t)n_maps * p.S * p.S); p.maps = dmaps;
   CU(cudaMemcpy(dmaps, maps, (size_t)n_maps * p.S * p.S, cudaMemcpyHostToDevice));
@@ -295,6 +315,8 @@ static int launch_step_kernel(nmmo_handle *h, NmParams &prm, cudaStream_t st, in
   const bool lean_ok = !prm.prof && !prm.inj_off;
   if (prm.big && h->big_std && lean_ok) nmmo_step_big_std_kernel<<<n, NM_BIG_THREADS, (size_t)prm.half_smem, st>>>(prm);
   else if (prm.big) nmmo_step_big_kernel<<<n, NM_BIG_THREADS, (size_t)prm.half_smem, st>>>(prm);
+  else if (epc == 4 && h->step_std && lean_ok) nmmo_step4_std_kernel<<<(n + 3) / 4, 4 * NM_STEP4_THREADS, (size_t)4 * prm.half_smem, st>>>(prm);
+  else if (epc == 4) nmmo_step4_kernel<<<(n + 3) / 4, 4 * NM_STEP4_THREADS, (size_t)4 * prm.half_smem, st>>>(prm);
   else if (epc == 3 && h->step_std && lean_ok) nmmo_step3_std_kernel<<<(n + 2) / 3, 3 * NM_STEP_THREADS, (size_t)3 * prm.half_smem, st>>>(prm);
   else if (epc == 3) nmmo_step3_kernel<<<(n + 2) / 3, 3 * NM_STEP_THREADS, (size_t)3 * prm.half_smem, st>>>(prm);
   else nmmo_step_kernel<<<(n + epc - 1) / epc, epc * NM_STEP_THREADS, (size_t)epc * prm.half_smem, st>>>(prm);
@@ -568,6 +590,7 @@ extern "C" void *nmmo_task_embed_ptr(nmmo_handle *h) { return (void *)h->prm.emb
 extern "C" const char *nmmo_step_kernel_name(nmmo_handle *h) {
   const bool lean_ok = !h->prm.prof && !h->prm.inj_off;      // same rule as launch_step
   if (h->prm.big) return (h->big_std && lean_ok) ? "nmmo_step_big_std_kernel" : "nmmo_step_big_kernel";
+  if (h->prm.envs_per_cta == 4) return (h->step_std && lean_ok) ? "nmmo_step4_std_kernel" : "nmmo_step4_kernel";
   if (h->prm.envs_per_cta == 3) return (h->step_std && lean_ok) ? "nmmo_step3_std_kernel" : "nmmo_step3_kernel";
   return "nmmo_step_kernel";
 }

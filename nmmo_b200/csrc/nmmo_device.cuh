@@ -16,6 +16,9 @@
 
 #define NM_EV_CAP 1024          // per-env per-tick event ring (shared memory)
 #define NM_STEP_THREADS 256
+#ifndef NM_STEP4_THREADS
+#define NM_STEP4_THREADS 192      // step kernel, four environments per CTA: threads per environment (768 per CTA, 80 registers)
+#endif
 #ifndef NM_OBS_THREADS
 #define NM_OBS_THREADS 512         // observation kernels: 16 warps per CTA ...
 #define NM_OBS_CTAS_PER_SM 2       // ... two CTAs per SM
@@ -94,7 +97,7 @@ struct NmParams {
   unsigned long long *prof;    // optional [32] per-phase clock accumulators (NULL = off)
   int half_smem;               // step kernel: dynamic shared memory of one environment
   int no_depl_list;            // test hook: never trust the depleted-tile list (always rebuild it from a map scan)
-  int envs_per_cta;            // step kernel: 2 when two environments fit in one CTA's shared memory, else 1
+  int envs_per_cta;            // step kernel: environments per CTA (4, 3, 2 or 1: as many as fit in shared memory)
   int mode;                    // 0 step (auto-reset finished envs), 1 reset flagged envs only
   int env_lo, env_hi;          // step kernel: the environments this launch covers (the host-buffer path launches it per copied range)
   int env_base;                // global env index of env 0 (multi-GPU sharding; seeds derive from it)

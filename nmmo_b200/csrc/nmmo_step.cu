@@ -3,6 +3,7 @@
 // Two instantiations of the same phases (struct VSmall / VBig below):
 //   nmmo_step_kernel      256 threads per environment, two environments per CTA, every table in shared memory
 //                         (PLAYER_N <= 256, P + N <= 512, map <= 255^2: BASELINE.json configs 1-4);
+//                         nmmo_step3_kernel / nmmo_step4_kernel run three / four environments per CTA (VSmall3 / VSmall4);
 //   nmmo_step_big_kernel  1024 threads per environment, one environment per CTA; the entity table (row-major), the
 //                         item table and the tile map stay in HBM / L2 and only the hot indices (occupancy bitmap,
 //                         position index, attack lists, inventories) live in shared memory
@@ -40,6 +41,7 @@ struct VSmall {
   static constexpr int kEvCap = NM_EV_CAP, kDeplCap = NM_DEPL_CAP, kNpcHash = 512, kTblSlots = 1024;
   static constexpr bool kGlobalTables = false;          // tables are staged in shared memory by TMA bulk copies
   static constexpr bool kItemsInPlace = false;          // ... including the live prefix of the item table and the event ring
+  static constexpr bool kScratchInWs = false;           // true: the per-tick arrays of VSmall4 below live in the HBM workspace
   static constexpr bool kStd = false;                   // true: a known shape (Shape) as compile-time constants
   typedef StdShape Shape;
   typedef uint16_t tile_t;                              // a tile index r * S + c
@@ -55,6 +57,20 @@ struct VSmall3 : VSmall {
 struct VSmall3Std : VSmall3 {
   static constexpr bool kStd = true;
 };
+// ... four environments per CTA, NM_STEP4_THREADS threads each (P <= kThreads, P + N <= 2 * kThreads): a 4096-env
+// tick is 1024 CTAs, seven full rounds of 148 SMs.  An environment gets 58 KB of shared memory (227 KB / 4), so the
+// arrays that are rebuilt every tick and read off the critical path also go to the per-env workspace in HBM / L2
+// (actions, task rows and accumulators, inventory lists, unique-event counts, window-scan results), the depleted-tile
+// list is used in place, and the Move position index, the player list and the alive-player list share scratch arrays
+// that are idle in the phases using them.  The NPC id hash stays: it is rebuilt and probed in the bookkeeping phase,
+// which is on every tick's critical path (in HBM it cost 5 K cycles per env-tick late in an episode).
+struct VSmall4 : VSmall3 {
+  static constexpr int kThreads = NM_STEP4_THREADS;
+  static constexpr bool kScratchInWs = true;
+};
+struct VSmall4Std : VSmall4 {
+  static constexpr bool kStd = true;
+};
 struct VBig {
   static constexpr int kThreads = NM_BIG_THREADS;
   static constexpr int kRowsPerThread = 3;
@@ -62,6 +78,7 @@ struct VBig {
   static constexpr int kEvCap = NM_BIG_EV_CAP, kDeplCap = NM_BIG_DEPL_CAP, kNpcHash = 4096, kTblSlots = 8192;
   static constexpr bool kGlobalTables = true;           // tables are used where they live (HBM, served from L2)
   static constexpr bool kItemsInPlace = true;
+  static constexpr bool kScratchInWs = false;
   static constexpr bool kStd = false;
   typedef StdShape5 Shape;
   typedef uint32_t tile_t;
@@ -1308,8 +1325,9 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
   auto carve = [&](size_t bytes) { uint8_t *q = smem + off; off = (off + bytes + 15) & ~(size_t)15; return q; };
   // big family: the arrays that are touched a few times per tick live in a per-env workspace in HBM / L2
   uint8_t *const gws = V::kItemsInPlace ? prm.ws + (size_t)env * prm.ws_bytes : nullptr;
-  auto carve_ws = [&](size_t bytes) {
-    if (!V::kGlobalTables) return carve(bytes);
+  // in_ws: the array goes to the workspace (big family and VSmall4: act / task / acc; VSmall4 only: the rest)
+  auto carve_ws = [&](size_t bytes, bool in_ws = V::kGlobalTables || V::kScratchInWs) {
+    if (!in_ws) return carve(bytes);
     uint8_t *q = gws + goff; goff = (goff + bytes + 15) & ~(size_t)15; return q;
   };
   const uint32_t ent_bytes = (uint32_t)(EA_N * R * 2), item_bytes = (uint32_t)(IS_N * CAP * 2), map_bytes = (uint32_t)(S * S / 2);
@@ -1329,31 +1347,40 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
   ctx.occ = (uint32_t *)carve(occ_words * 4);
   ctx.used = (uint32_t *)carve(cap_words * 4);
   ctx.fresh = (uint32_t *)carve(cap_words * 4);
-  ctx.inv = (uint16_t *)carve((size_t)P * NINV * 2);
+  ctx.inv = (uint16_t *)carve_ws((size_t)P * NINV * 2, V::kScratchInWs);
   ctx.invn = carve(P);
   ctx.act = (int16_t *)carve_ws((size_t)A_N * P * 2);
   ctx.npc_move = (int8_t *)carve(N);
   ctx.npc_att = (int16_t *)carve((size_t)N * 2);
   if (V::kItemsInPlace && !V::kGlobalTables) { ctx.ev = (uint2 *)(gws + goff); goff += (size_t)V::kEvCap * 8; }      // (VSmall3: the only workspace array)
   else ctx.ev = (uint2 *)carve_ws((size_t)V::kEvCap * 8);
-  ctx.duniq = (int *)carve((size_t)P * 4);
-  int *s_list = (int *)carve((size_t)P * 4);
+  ctx.duniq = (int *)carve_ws((size_t)P * 4, V::kScratchInWs);
+  int *s_list = V::kScratchInWs ? nullptr : (int *)carve((size_t)P * 4);      // (VSmall4: in the scratch, below)
   ctx.npc_hash = (unsigned short *)carve((size_t)V::kNpcHash * 2);
   ctx.task = (int *)carve_ws((size_t)P * 16);
   ctx.acc = (int *)carve_ws((size_t)P * 8);
   // 4 KB scratch reused phase by phase: attack list + registrations, move tile hash,
   // respawn worklist, NPC-spawn pre-drawn values
   const size_t scratch_bytes = max((size_t)4096, (size_t)R * 8);
-  uint32_t *s_scratch = (uint32_t *)carve(scratch_bytes + 32 * V::kChunkIters * 4);      // + the per-chunk counts behind the two attack arrays
+  // + the per-chunk counts behind the two attack arrays (VSmall4: R <= 384, they fit in the 4 KB)
+  uint32_t *s_scratch = (uint32_t *)carve(scratch_bytes + (V::kScratchInWs ? 0 : 32 * V::kChunkIters * 4));
   uint8_t *s_mv = carve((size_t)R * (sizeof(tile_t) + 2));     // Move phase: destination (tile_t) + verdict (u16) per row; >= R * 4 bytes
-  // depleted-tile list: staged in shared memory (small) / used in place in HBM (big)
+  // depleted-tile list: staged in shared memory (small) / used in place in HBM (big, VSmall4)
+  constexpr bool kDeplInPlace = V::kGlobalTables || V::kScratchInWs;
   tile_t *const gdepl = (tile_t *)prm.depl + (size_t)env * V::kDeplCap;
-  ctx.dlist = V::kGlobalTables ? gdepl : (tile_t *)carve((size_t)V::kDeplCap * sizeof(tile_t));
-  uint32_t *s_tbl = (uint32_t *)carve((size_t)V::kTblSlots * 4);           // Move phase: position index (tile -> row)
+  ctx.dlist = kDeplInPlace ? gdepl : (tile_t *)carve((size_t)V::kDeplCap * sizeof(tile_t));
+  // Move phase: position index (tile -> row).  VSmall4: in the scratch, which the attack phase leaves before the Move
+  uint32_t *s_tbl = V::kScratchInWs ? s_scratch : (uint32_t *)carve((size_t)V::kTblSlots * 4);
+  static_assert(!V::kScratchInWs || V::kTblSlots * 4 <= 4096, "the position index must fit the scratch");
+  // VSmall4: the player list of the update / harvest / Buy phases and of the window scans sits in the scratch behind
+  // the first 2 KB (idle in those phases; the depleted-tile list the writeback copies out of it is <= 2 KB)
+  if (V::kScratchInWs) s_list = (int *)(s_scratch + 512);
+  static_assert(!V::kScratchInWs || (V::kThreads + 512) * 4 <= 4096, "the player list must fit the scratch");
   uint32_t *s_att = s_scratch;
   int *s_first = (int *)(s_scratch + R);
-  ctx.slow = (int8_t *)carve((size_t)P);
-  uint32_t *s_plist = (uint32_t *)carve((size_t)P * 4);
+  ctx.slow = (int8_t *)carve_ws((size_t)P, V::kScratchInWs);
+  // alive players for the NPC target scans (phases 0-1).  VSmall4: in the Move scratch, which the attack phase is first to use
+  uint32_t *s_plist = V::kScratchInWs ? (uint32_t *)s_mv : (uint32_t *)carve((size_t)P * 4);
   ctx.sc = (int *)carve(32 * 4);
   uint64_t *bar = (uint64_t *)carve(16);
   // ---- load: three bulk copies on one mbarrier, issued before anything else touches HBM ----
@@ -1377,7 +1404,7 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
     // the prefix below the high-water mark moves between HBM and shared memory.  Rows above it are
     // never read before they are allocated (the in-use bitmap is built from the prefix).
     const uint32_t col_bytes = (uint32_t)item_hi0 * 2;
-    const uint32_t dl_bytes = n_depl0 > 0 ? (uint32_t)((n_depl0 * (int)sizeof(tile_t) + 15) & ~15) : 0u;
+    const uint32_t dl_bytes = n_depl0 > 0 && !kDeplInPlace ? (uint32_t)((n_depl0 * (int)sizeof(tile_t) + 15) & ~15) : 0u;
     mbar_expect_tx(bar + 1, (V::kItemsInPlace ? 0u : col_bytes * IS_N) + dl_bytes);
     if (dl_bytes) bulk_g2s(ctx.dlist, gdepl, dl_bytes, bar + 1);
     if (col_bytes && !V::kItemsInPlace)
@@ -1420,7 +1447,7 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
   #pragma unroll 1
   for (int i = tid; i < V::kNpcHash / 2; i += T) ((uint32_t *)ctx.npc_hash)[i] = 0;
   #pragma unroll 1
-  for (int i = tid; i < V::kTblSlots; i += T) s_tbl[i] = 0;
+  for (int i = tid; i < (V::kScratchInWs ? 0 : V::kTblSlots); i += T) s_tbl[i] = 0;
   if (tid < P) {
     ctx.task[tid * 4] = my_t[0]; ctx.task[tid * 4 + 1] = my_t[1]; ctx.task[tid * 4 + 2] = my_t[2]; ctx.task[tid * 4 + 3] = 0;
     ctx.acc[tid * 2] = my_acc0; ctx.acc[tid * 2 + 1] = my_acc1;
@@ -1819,6 +1846,9 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
       PCOUNT(46, clock64() - ta2);
     }
   }
+  // VSmall4: the position index takes over the scratch (every read of the attack list is behind the last barrier above)
+  #pragma unroll 1
+  for (int i = tid; i < (V::kScratchInWs ? V::kTblSlots : 0); i += T) s_tbl[i] = 0;
   HSYNC();
   PHASE();
   // Move (60): with one entity per tile the reference resolves moves in entity-id order.
@@ -2154,7 +2184,7 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
     if (col_bytes && !V::kItemsInPlace)
       for (int k = 0; k < IS_N; k++) bulk_s2g(gitem + (size_t)k * CAP, ctx.item + k * CAP, col_bytes);
     bulk_s2g(prm.map + (size_t)env * map_bytes, ctx.map, map_bytes);
-    if (ctx.sc[21] > 0)
+    if (ctx.sc[21] > 0 && !(kDeplInPlace && ctx.sc[22]))      // (in place: a list rebuilt into dlist is already there)
       bulk_s2g(gdepl, ctx.sc[22] ? (const void *)ctx.dlist : (const void *)s_scratch, (uint32_t)((ctx.sc[21] * (int)sizeof(tile_t) + 15) & ~15));
     bulk_commit();
   }
@@ -2339,6 +2369,12 @@ nmmo_step3_kernel(const __grid_constant__ NmParams prm) { step_body<VSmall3>(prm
 
 extern "C" __global__ void __launch_bounds__(3 * VSmall3Std::kThreads, 1)
 nmmo_step3_std_kernel(const __grid_constant__ NmParams prm) { step_body<VSmall3Std>(prm); }
+
+extern "C" __global__ void __launch_bounds__(4 * VSmall4::kThreads, 1)
+nmmo_step4_kernel(const __grid_constant__ NmParams prm) { step_body<VSmall4>(prm); }
+
+extern "C" __global__ void __launch_bounds__(4 * VSmall4Std::kThreads, 1)
+nmmo_step4_std_kernel(const __grid_constant__ NmParams prm) { step_body<VSmall4Std>(prm); }
 
 extern "C" __global__ void __launch_bounds__(VBig::kThreads, 1)
 nmmo_step_big_kernel(const __grid_constant__ NmParams prm) { step_body<VBig>(prm); }
