@@ -60,6 +60,16 @@ int nmmo_reset(nmmo_handle *h, const uint64_t *seeds, const int32_t *map_ids, co
  * Launches 2 kernels on `stream`; results are in the buffers returned by the accessors. */
 int nmmo_step(nmmo_handle *h, const int32_t *actions_dev, void *stream);
 
+/* Replaces: send(actions) of one batch of an env pool (clean_pufferl.py:357 with envs_per_batch < num_envs): steps
+ * envs [env_lo, env_hi) only.  actions: DEVICE int32 [env_hi - env_lo][P][12], row 0 = env env_lo, 16-byte aligned.
+ * Launches the step and observation kernels of the range on `stream`; envs of the range whose episode ended on their
+ * previous step are reset instead of stepped, as in nmmo_step.  The built-in random policy (nmmo_set_autosample) writes
+ * the range's rows of its buffer.  Ranges on different streams may run at the same time when they do not overlap; calls
+ * that touch the whole handle (nmmo_reset, nmmo_step) must be ordered after every range step in flight.
+ * NM_ERR_ARG for an empty or out-of-bounds range or misaligned actions; NM_ERR_STATE while per-kernel timing or the
+ * phase profiler is on (both describe whole-handle launches). */
+int nmmo_step_envs(nmmo_handle *h, int env_lo, int env_hi, const int32_t *actions_dev, void *stream);
+
 /* Same call with HOST buffers (the copy-in / copy-out path the reference pays today,
  * clean_pufferl.py:302-304,329): H2D of actions, step, D2H of reward/terminated/truncated/mask;
  * obs_out may be NULL (observations stay on the device for the policy) or a host buffer of
@@ -171,8 +181,8 @@ enum nm_rollout_buffer {     /* nmmo_rollout_buffer(which): rows = batch_size + 
   NM_RB_IDXS,                /* int32 [rows]: sample indices sorted by (slot, step)  (clean_pufferl.py:413) */
   NM_RB_ADVANTAGES,          /* float32 [rows]: advantages[t] for t < ptr - 1, in sorted order (:424-436) */
   /* compact mode only */
-  NM_RB_MARKET,              /* uint8 [max_steps][n_envs][market_bytes]: the Market block of an env in a step, stored once */
-  NM_RB_MARKET_SLOT,         /* int32 [rows]: step_index * n_envs + env of the row's Market block */
+  NM_RB_MARKET,              /* uint8 [max_steps * n_envs][market_bytes]: the Market block of an env in a call, stored once, in call order */
+  NM_RB_MARKET_SLOT,         /* int32 [rows]: the row's Market block (blocks of earlier calls + env of the call; step_index * n_envs + env for whole-handle calls) */
   NM_RB_TASK_ID              /* int32 [rows]: the row's task id (its Task block is the embedding of that task) */
 };
 int nmmo_rollout_create(int device, int batch_size, int n_slots, int obs_stride, nmmo_rollout **out);
@@ -202,6 +212,15 @@ int nmmo_rollout_reset(nmmo_rollout *r, void *stream);
 int nmmo_rollout_store(nmmo_rollout *r, const uint8_t *obs, const int32_t *actions, const float *logprob,
                        const float *value, const float *reward, const float *done, const uint8_t *mask,
                        const uint8_t *learner_mask, int step, void *stream);
+/* The same for the slots [slot_lo, slot_lo + n) of one call, e.g. one batch of an env pool: every argument covers
+ * the call's n slots (obs uint8 [n][obs_stride], ...), the sort key is slot_lo + i and the running counts are kept per
+ * global slot, so calls over different ranges sort and chain like one call over all slots.  task_id: NULL for a plain
+ * rollout, DEVICE int32 [n] for a compact one, whose range must cover whole envs; there the Market block is stored once
+ * per (call, env of the call), up to max_steps * n_slots / agents_per_env blocks between two resets (NM_ERR_LIMIT when
+ * full).  nmmo_rollout_store / _store_compact are this call with slot_lo = 0, n = n_slots. */
+int nmmo_rollout_store_range(nmmo_rollout *r, int slot_lo, int n, const uint8_t *obs, const int32_t *actions,
+                             const float *logprob, const float *value, const float *reward, const float *done,
+                             const uint8_t *mask, const uint8_t *learner_mask, const int32_t *task_id, int step, void *stream);
 /* Rows stored so far (synchronises `stream`). */
 int nmmo_rollout_ptr(nmmo_rollout *r, void *stream, int *ptr_out);
 /* Sorted order + advantages of the stored rows; float32 arithmetic of the reference in its order. */

@@ -324,6 +324,20 @@ static int launch_step_kernel(nmmo_handle *h, NmParams &prm, cudaStream_t st, in
   return NM_OK;
 }
 
+// observation kernel over env range [lo, hi) on `st`
+static int launch_obs_kernel(nmmo_handle *h, NmParams &prm, cudaStream_t st, int lo, int hi) {
+  const int n = hi - lo;
+  prm.env_lo = lo; prm.env_hi = hi;
+  if (prm.big) {
+    const int ap = std::min(prm.P, NM_BIG_OBS_AGENTS), parts = (prm.P + ap - 1) / ap;
+    if (h->big_std && !prm.prof) nmmo_obs_big_std_kernel<<<n * parts, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
+    else nmmo_obs_big_kernel<<<n * parts, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
+  } else if (h->obs_std && !prm.prof) nmmo_obs_std_kernel<<<n, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
+  else nmmo_obs_kernel<<<n, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
+  CU(cudaGetLastError());
+  return NM_OK;
+}
+
 // step_done = true: the step kernel of this tick was already launched (in env ranges, by the caller)
 static int launch_step(nmmo_handle *h, int mode, cudaStream_t st, cudaEvent_t after_step = nullptr, bool step_done = false) {
   NmParams prm = h->prm;
@@ -340,13 +354,7 @@ static int launch_step(nmmo_handle *h, int mode, cudaStream_t st, cudaEvent_t af
   if (!step_done) { int rc = launch_step_kernel(h, prm, st, 0, prm.E); if (rc) return rc; }
   if (e3) CU(cudaEventRecord(e3[1], st));
   if (after_step) CU(cudaEventRecord(after_step, st));      // rewards / flags / mask are final here
-  if (prm.big) {
-    const int ap = std::min(prm.P, NM_BIG_OBS_AGENTS), parts = (prm.P + ap - 1) / ap;
-    if (h->big_std && !prm.prof) nmmo_obs_big_std_kernel<<<prm.E * parts, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
-    else nmmo_obs_big_kernel<<<prm.E * parts, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
-  } else if (h->obs_std && !prm.prof) nmmo_obs_std_kernel<<<prm.E, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
-  else nmmo_obs_kernel<<<prm.E, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
-  CU(cudaGetLastError());
+  { int rc = launch_obs_kernel(h, prm, st, 0, prm.E); if (rc) return rc; }
   if (e3) CU(cudaEventRecord(e3[2], st));
   return NM_OK;
 }
@@ -401,6 +409,22 @@ extern "C" int nmmo_step(nmmo_handle *h, const int32_t *actions_dev, void *strea
   CU(cudaSetDevice(h->device));
   h->prm.actions = actions_dev;
   return launch_step(h, 0, (cudaStream_t)stream);
+}
+
+extern "C" int nmmo_step_envs(nmmo_handle *h, int env_lo, int env_hi, const int32_t *actions_dev, void *stream) {
+  if (!h || !actions_dev) return fail(NM_ERR_ARG, "null argument");
+  if (env_lo < 0 || env_hi > h->prm.E || env_lo >= env_hi) return fail(NM_ERR_ARG, "env range must satisfy 0 <= env_lo < env_hi <= E");
+  if ((uintptr_t)actions_dev & 15) return fail(NM_ERR_ARG, "actions must be 16-byte aligned");
+  if (h->timing || h->prm.prof)
+    return fail(NM_ERR_STATE, "per-kernel timing and the phase profiler describe whole-handle launches: switch them off for range steps");
+  CU(cudaSetDevice(h->device));
+  NmParams prm = h->prm;
+  prm.mode = 0;
+  prm.actions = actions_dev; prm.act_env_lo = env_lo;
+  const cudaStream_t st = (cudaStream_t)stream;
+  int rc = launch_step_kernel(h, prm, st, env_lo, env_hi);
+  if (rc) return rc;
+  return launch_obs_kernel(h, prm, st, env_lo, env_hi);
 }
 
 static int finish_step_host(nmmo_handle *h, float *rew_out, uint8_t *term_out, uint8_t *trunc_out, uint8_t *mask_out,

@@ -99,7 +99,8 @@ struct NmParams {
   int no_depl_list;            // test hook: never trust the depleted-tile list (always rebuild it from a map scan)
   int envs_per_cta;            // step kernel: environments per CTA (4, 3, 2 or 1: as many as fit in shared memory)
   int mode;                    // 0 step (auto-reset finished envs), 1 reset flagged envs only
-  int env_lo, env_hi;          // step kernel: the environments this launch covers (the host-buffer path launches it per copied range)
+  int env_lo, env_hi;          // step and observation kernels: the environments this launch covers
+  int act_env_lo;              // env whose actions are row 0 of `actions` (0 = a whole-handle buffer; nmmo_step_envs: its env_lo)
   int env_base;                // global env index of env 0 (multi-GPU sharding; seeds derive from it)
 };
 

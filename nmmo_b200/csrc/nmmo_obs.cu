@@ -105,9 +105,9 @@ __device__ __forceinline__ void obs_body(const NmParams &prm) {
   const int NINV = V::kStd ? SH::NINV : c[NC_N_INV], vis = V::kStd ? SH::VIS : c[NC_VISION];
   const int AP = V::kStage ? P : min(P, NM_BIG_OBS_AGENTS);
   const int parts = V::kStage ? 1 : (P + AP - 1) / AP;
-  // small family: highest env first -- the tables the step kernel wrote last are still in L2, and the records this kernel
-  // writes last are the ones the next step kernel (lowest env first) reads first
-  const int env = V::kStage ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x / parts;
+  // small family: highest env of [env_lo, env_hi) first -- the tables the step kernel wrote last are still in L2, and the
+  // records this kernel writes last are the ones the next step kernel (lowest env first) reads first
+  const int env = V::kStage ? prm.env_hi - 1 - (int)blockIdx.x : prm.env_lo + (int)blockIdx.x / parts;
   const int p_lo = V::kStage ? 0 : ((int)blockIdx.x % parts) * AP, p_hi = min(P, p_lo + AP);
   const int tick = prm.scalars[(size_t)env * NM_SC_N + SC_TICK];
 
@@ -192,7 +192,7 @@ __device__ __forceinline__ void obs_body(const NmParams &prm) {
     // L2 prefetch for a CTA that starts a few microseconds from now (envs are taken highest first): this kernel writes
     // 1.7 GB through L2 while it reads 0.2 GB of tables, so a table fetched on demand waits behind the writes
     const int env_next = env - NM_OBS_PREFETCH_AHEAD;
-    if (env_next >= 0) {
+    if (env_next >= prm.env_lo) {
       if (lane == 0) bulk_prefetch_l2(prm.ent + (size_t)env_next * EA_N * R, (uint32_t)(EA_N_OBS * R * 2));
       else if (lane == 1) bulk_prefetch_l2(prm.ent + (size_t)env_next * EA_N * R + (size_t)EA_STATUS * R, st_bytes);
       else bulk_prefetch_l2(prm.map + (size_t)env_next * map_bytes, map_bytes);

@@ -28,6 +28,7 @@ constexpr int RB = 1024;            // threads per block of the scan-shaped kern
 struct RolloutParams {
   int cap;                 // batch_size + 1 rows
   int n_slots;             // agent slots per step (E * P)
+  int call_lo, call_n;     // store: the slots [call_lo, call_lo + call_n) of this call (row i of its inputs = slot call_lo + i)
   int stride;              // bytes per observation record (multiple of 16)
   // storage (clean_pufferl.py:183-189)
   uint8_t *obs; int32_t *actions; float *logprobs, *rewards, *dones, *values;
@@ -47,9 +48,9 @@ struct RolloutParams {
   int m_off, m_len, t_off, t_len;  // byte ranges of the two sections inside a record (multiples of 16)
   int ids_off;             // byte offset of the int16 AgentId: 0 there = the all-zero record of an agent that just died
   int row_stride;          // bytes per stored row (= stride - m_len - t_len in compact mode)
-  int max_steps;           // Market slots: [max_steps][n_envs][m_len]
+  int max_steps;           // Market blocks: max_steps * n_envs of m_len bytes
   uint8_t *market;
-  int32_t *mslot;          // [cap] row -> step_index * n_envs + env
+  int32_t *mslot;          // [cap] row -> Market block (blocks stored by earlier calls + env of the call)
   int32_t *task;           // [cap] row -> task id
 };
 
@@ -78,7 +79,7 @@ __device__ int block_excl_scan(int v, int *s_warp, int &total) {
 }
 
 __device__ __forceinline__ bool selected(const RolloutParams &p, const uint8_t *mask, const uint8_t *learner, int i) {
-  return i < p.n_slots && mask[i] != 0 && (learner == nullptr || learner[i] != 0);
+  return i < p.call_n && mask[i] != 0 && (learner == nullptr || learner[i] != 0);
 }
 
 // ---- append: pass 1, selected slots per 1024-slot block --------------------------------------
@@ -120,9 +121,10 @@ __global__ void __launch_bounds__(RB) k_store_rows(RolloutParams p, const uint8_
     int4 *o4 = (int4 *)(p.actions + (size_t)pos * 12);
     o4[0] = a4[0]; o4[1] = a4[1]; o4[2] = a4[2];
     p.logprobs[pos] = logprob[i]; p.values[pos] = value[i]; p.rewards[pos] = reward[i]; p.dones[pos] = done[i];
-    p.slot[pos] = i; p.step[pos] = step;
-    p.rank[pos] = p.count[i];                 // steps arrive in order: the running count is the rank
-    p.count[i] += 1;
+    const int g = p.call_lo + i;
+    p.slot[pos] = g; p.step[pos] = step;
+    p.rank[pos] = p.count[g];                 // steps arrive in order: the running count is the rank
+    p.count[g] += 1;
     int k = atomicAdd(&s_n, 1);
     s_src[k] = i; s_dst[k] = pos;
   }
@@ -148,12 +150,13 @@ __global__ void __launch_bounds__(RB) k_store_rows(RolloutParams p, const uint8_
     }
   }
 }
-// compact mode: per kept row the Market slot and the task id; per env the Market block of its first selected agent
+// compact mode: per kept row the Market block and the task id; per env of the call the Market block of its first selected
+// agent, at block mbase + env
 __device__ __forceinline__ bool zero_record(const RolloutParams &p, const uint8_t *obs, int i) {
   return *(const int16_t *)(obs + (size_t)i * p.stride + p.ids_off) == 0;
 }
 __global__ void __launch_bounds__(RB) k_store_compact_keys(RolloutParams p, const uint8_t *obs, const uint8_t *mask, const uint8_t *learner,
-                                                          const int32_t *task_id, int step_index) {
+                                                          const int32_t *task_id, int mbase) {
   __shared__ int s_warp[33];
   const int i = blockIdx.x * RB + threadIdx.x;
   const bool sel = selected(p, mask, learner, i);
@@ -163,14 +166,14 @@ __global__ void __launch_bounds__(RB) k_store_compact_keys(RolloutParams p, cons
   if (sel && pos < p.cap) {
     // an agent that died this tick is stored with the all-zero record: its Market and Task sections are zeros too (-1)
     const bool z = zero_record(p, obs, i);
-    p.mslot[pos] = z ? -1 : step_index * p.n_envs + i / p.agents_per_env;
+    p.mslot[pos] = z ? -1 : mbase + i / p.agents_per_env;
     p.task[pos] = z ? -1 : task_id[i];
   }
 }
 __global__ void __launch_bounds__(256) k_store_market(RolloutParams p, const uint8_t *obs, const uint8_t *mask, const uint8_t *learner,
-                                                     int step_index) {
+                                                     int mbase) {
   const int lane = threadIdx.x & 31, env = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (env >= p.n_envs) return;
+  if (env >= p.call_n / p.agents_per_env) return;
   int first = -1;
   for (int b = 0; b < p.agents_per_env && first < 0; b += 32) {
     const int a = b + lane;
@@ -180,7 +183,7 @@ __global__ void __launch_bounds__(256) k_store_market(RolloutParams p, const uin
   }
   if (first < 0) return;                      // nobody of this env is stored this step
   const uint4 *src = (const uint4 *)(obs + (size_t)(env * p.agents_per_env + first) * p.stride + p.m_off);
-  uint4 *dst = (uint4 *)(p.market + ((size_t)step_index * p.n_envs + env) * p.m_len);
+  uint4 *dst = (uint4 *)(p.market + ((size_t)mbase + env) * p.m_len);
   for (int q = lane; q < (p.m_len >> 4); q += 32) __stcs(dst + q, __ldcs(src + q));
 }
 // re-assemble full records: out[k] = row idxs[k] (or row k when idxs is NULL) with its Market block and Task embedding
@@ -284,7 +287,7 @@ __global__ void k_gae_chains(RolloutParams p) {
 struct nmmo_rollout {
   RolloutParams p;
   int device;
-  int n_steps = 0;         // compact mode: store calls since the last reset (Market slot index)
+  int n_mblocks = 0;       // compact mode: Market blocks stored since the last reset
   std::vector<void *> allocs;
 };
 
@@ -367,49 +370,56 @@ extern "C" int nmmo_rollout_reset(nmmo_rollout *r, void *stream) {
   cudaStream_t st = (cudaStream_t)stream;
   RCU(cudaMemsetAsync(r->p.count, 0, sizeof(int32_t) * r->p.n_slots, st));
   RCU(cudaMemsetAsync(r->p.d_ptr, 0, sizeof(int32_t) * 4, st));
-  r->n_steps = 0;
+  r->n_mblocks = 0;
   return NM_OK;
 }
 
-static int rollout_store(nmmo_rollout *r, const uint8_t *obs, const int32_t *actions, const float *logprob,
-                         const float *value, const float *reward, const float *done, const uint8_t *mask,
-                         const uint8_t *learner_mask, const int32_t *task_id, int step, void *stream);
+extern "C" int nmmo_rollout_store_range(nmmo_rollout *r, int slot_lo, int n, const uint8_t *obs, const int32_t *actions,
+                                        const float *logprob, const float *value, const float *reward, const float *done,
+                                        const uint8_t *mask, const uint8_t *learner_mask, const int32_t *task_id, int step,
+                                        void *stream) {
+  if (!r || !obs || !actions || !logprob || !value || !reward || !done || !mask) return rfail(NM_ERR_ARG, "null argument");
+  if (((uintptr_t)obs | (uintptr_t)actions) & 15) return rfail(NM_ERR_ARG, "obs and actions must be 16-byte aligned");
+  if (slot_lo < 0 || n <= 0 || n > r->p.n_slots - slot_lo) return rfail(NM_ERR_ARG, "slot range must satisfy 0 <= slot_lo < slot_lo + n <= n_slots");
+  RolloutParams p = r->p;
+  p.call_lo = slot_lo; p.call_n = n;
+  int mbase = 0;
+  if (p.compact) {
+    if (!task_id) return rfail(NM_ERR_ARG, "compact store needs the task ids");
+    if (slot_lo % p.agents_per_env || n % p.agents_per_env) return rfail(NM_ERR_ARG, "compact store: the slot range must cover whole envs");
+    if (r->n_mblocks + n / p.agents_per_env > p.max_steps * p.n_envs)
+      return rfail(NM_ERR_LIMIT, "compact rollout: the Market store is full (more than max_steps whole-handle store calls since the last reset)");
+    mbase = r->n_mblocks;
+  } else if (task_id) return rfail(NM_ERR_ARG, "task ids are for compact rollouts only");
+  RCU(cudaSetDevice(r->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  int nb = (n + RB - 1) / RB;
+  k_store_count<<<nb, RB, 0, st>>>(p, mask, learner_mask);
+  k_scan_blocks<<<1, RB, 0, st>>>(p.blocksum, nb, p.d_ptr + 1);
+  if (p.compact) {
+    k_store_compact_keys<<<nb, RB, 0, st>>>(p, obs, mask, learner_mask, task_id, mbase);
+    k_store_market<<<(n / p.agents_per_env * 32 + 255) / 256, 256, 0, st>>>(p, obs, mask, learner_mask, mbase);
+    r->n_mblocks += n / p.agents_per_env;
+  }
+  k_store_rows<<<nb, RB, 0, st>>>(p, obs, actions, logprob, value, reward, done, mask, learner_mask, step);
+  k_advance_ptr<<<1, 32, 0, st>>>(p);
+  RCU(cudaGetLastError());
+  return NM_OK;
+}
 
 extern "C" int nmmo_rollout_store(nmmo_rollout *r, const uint8_t *obs, const int32_t *actions, const float *logprob,
                                   const float *value, const float *reward, const float *done, const uint8_t *mask,
                                   const uint8_t *learner_mask, int step, void *stream) {
   if (r && r->p.compact) return rfail(NM_ERR_STATE, "compact rollout: use nmmo_rollout_store_compact (needs the task ids)");
-  return rollout_store(r, obs, actions, logprob, value, reward, done, mask, learner_mask, nullptr, step, stream);
+  if (!r) return rfail(NM_ERR_ARG, "null argument");
+  return nmmo_rollout_store_range(r, 0, r->p.n_slots, obs, actions, logprob, value, reward, done, mask, learner_mask, nullptr, step, stream);
 }
 
 extern "C" int nmmo_rollout_store_compact(nmmo_rollout *r, const uint8_t *obs, const int32_t *actions, const float *logprob,
                                           const float *value, const float *reward, const float *done, const uint8_t *mask,
                                           const uint8_t *learner_mask, const int32_t *task_id, int step, void *stream) {
   if (!r || !r->p.compact || !task_id) return rfail(NM_ERR_ARG, "compact store needs a compact rollout and the task ids");
-  if (r->n_steps >= r->p.max_steps) return rfail(NM_ERR_LIMIT, "compact rollout: more store calls than max_steps since the last reset");
-  return rollout_store(r, obs, actions, logprob, value, reward, done, mask, learner_mask, task_id, step, stream);
-}
-
-static int rollout_store(nmmo_rollout *r, const uint8_t *obs, const int32_t *actions, const float *logprob,
-                         const float *value, const float *reward, const float *done, const uint8_t *mask,
-                         const uint8_t *learner_mask, const int32_t *task_id, int step, void *stream) {
-  if (!r || !obs || !actions || !logprob || !value || !reward || !done || !mask) return rfail(NM_ERR_ARG, "null argument");
-  if (((uintptr_t)obs | (uintptr_t)actions) & 15) return rfail(NM_ERR_ARG, "obs and actions must be 16-byte aligned");
-  RCU(cudaSetDevice(r->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  const RolloutParams &p = r->p;
-  int nb = (p.n_slots + RB - 1) / RB;
-  k_store_count<<<nb, RB, 0, st>>>(p, mask, learner_mask);
-  k_scan_blocks<<<1, RB, 0, st>>>(p.blocksum, nb, p.d_ptr + 1);
-  if (p.compact) {
-    k_store_compact_keys<<<nb, RB, 0, st>>>(p, obs, mask, learner_mask, task_id, r->n_steps);
-    k_store_market<<<(p.n_envs * 32 + 255) / 256, 256, 0, st>>>(p, obs, mask, learner_mask, r->n_steps);
-    r->n_steps++;
-  }
-  k_store_rows<<<nb, RB, 0, st>>>(p, obs, actions, logprob, value, reward, done, mask, learner_mask, step);
-  k_advance_ptr<<<1, 32, 0, st>>>(p);
-  RCU(cudaGetLastError());
-  return NM_OK;
+  return nmmo_rollout_store_range(r, 0, r->p.n_slots, obs, actions, logprob, value, reward, done, mask, learner_mask, task_id, step, stream);
 }
 
 extern "C" int nmmo_rollout_ptr(nmmo_rollout *r, void *stream, int *ptr_out) {

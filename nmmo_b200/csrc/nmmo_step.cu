@@ -1470,7 +1470,7 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
   int my_prev_price = 0;
   if (tid < P) {
     const int p = tid;
-    const int4 *x4 = (const int4 *)(prm.actions + ((size_t)env * P + p) * AC_N);
+    const int4 *x4 = (const int4 *)(prm.actions + ((size_t)(env - prm.act_env_lo) * P + p) * AC_N);
     const int16_t *gent = prm.ent + (size_t)env * (V::kGlobalTables ? (size_t)NM_BIG_ENT_STRIDE * R : (size_t)EA_N * R);
     const int g_status = gent[V::ent_idx(EA_STATUS, p, R)], g_health = gent[V::ent_idx(EA_HEALTH, p, R)];   // same answer as ent_alive() later
     int4 xa = x4[0], xb = x4[1], xc = x4[2];

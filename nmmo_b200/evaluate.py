@@ -22,7 +22,8 @@ from types import SimpleNamespace
 
 
 def evaluate(pool, policy, rollout, learner_mask=None, max_steps: int = 1 << 30):
-    """Collect ``rollout.batch_size + 1`` samples.  Returns a namespace with the reference's counters:
+    """Collect ``rollout.batch_size + 1`` samples (``rollout`` covers all slots of the pool; each batch of an env pool is
+    stored at its global slots).  Returns a namespace with the reference's counters:
     agent_steps (sum of mask, :306), global_steps (len(mask), :307), steps, infos (list of dicts)."""
     import torch
     rollout.reset()
@@ -34,13 +35,18 @@ def evaluate(pool, policy, rollout, learner_mask=None, max_steps: int = 1 << 30)
         if rollout.ptr >= cap:        # the one host read per step (the reference's `ptr == batch_size + 1` test, :289)
             break
         o, r, d, t, i, env_id, mask = pool.recv()
+        # an env pool (envs_per_batch < num_envs) hands out one batch: its rows are the global slots from slot_base on
+        slot_base = pool.batch_env_range[0] * pool.agents_per_env if hasattr(pool, "batch_env_range") else 0
         n_recv += 1
         infos.extend(i)
         agent_steps += mask.sum()
         padded += mask.numel()
         with torch.no_grad():
             actions, logprob, value = policy(o)
-        rollout.store(o, value, actions, logprob, r, d.float(), mask, step, learner_mask=learner_mask)
+        lm = learner_mask
+        if lm is not None and lm.numel() != mask.numel():      # a mask over all slots: the batch's part
+            lm = lm.reshape(-1)[slot_base:slot_base + mask.numel()]
+        rollout.store(o, value, actions, logprob, r, d.float(), mask, step, learner_mask=lm, slot_base=slot_base)
         # the reference always sends the step's actions and only leaves at the top of the next iteration (:289, :357):
         # the stored (action, logprob, value) of the last row are the ones the envs execute, and the next call's
         # first recv() sees fresh outputs

@@ -17,12 +17,12 @@ _LIB_PATH = Path(__file__).resolve().parent / "_build" / "libnmmo_b200.so"
 _lib = None
 
 EXPORTS = [
-    "nmmo_create", "nmmo_destroy", "nmmo_reset", "nmmo_step", "nmmo_step_host", "nmmo_step_host_i16", "nmmo_step_host_u8", "nmmo_sample_actions", "nmmo_forage_actions",
+    "nmmo_create", "nmmo_destroy", "nmmo_reset", "nmmo_step", "nmmo_step_envs", "nmmo_step_host", "nmmo_step_host_i16", "nmmo_step_host_u8", "nmmo_sample_actions", "nmmo_forage_actions",
     "nmmo_obs_ptr", "nmmo_reward_ptr", "nmmo_terminated_ptr", "nmmo_truncated_ptr", "nmmo_mask_ptr",
     "nmmo_info_ptr", "nmmo_info_valid_ptr", "nmmo_episode_done_ptr", "nmmo_task_id_ptr", "nmmo_task_embed_ptr", "nmmo_obs_stride", "nmmo_num_envs",
     "nmmo_num_agents", "nmmo_step_kernel_name", "nmmo_obs_kernel_name", "nmmo_inject_rng", "nmmo_snapshot", "nmmo_task_state", "nmmo_stats", "nmmo_check", "nmmo_timing", "nmmo_timing_read", "nmmo_profile", "nmmo_set_obs_full", "nmmo_set_autosample",
     "nmmo_last_error",
-    "nmmo_rollout_create", "nmmo_rollout_create_compact", "nmmo_rollout_store_compact", "nmmo_rollout_expand", "nmmo_rollout_destroy", "nmmo_rollout_reset", "nmmo_rollout_store", "nmmo_rollout_ptr",
+    "nmmo_rollout_create", "nmmo_rollout_create_compact", "nmmo_rollout_store_compact", "nmmo_rollout_expand", "nmmo_rollout_destroy", "nmmo_rollout_reset", "nmmo_rollout_store", "nmmo_rollout_store_range", "nmmo_rollout_ptr",
     "nmmo_rollout_gae", "nmmo_rollout_buffer", "nmmo_rollout_last_error",
 ]
 
@@ -55,6 +55,8 @@ def load(build_if_missing: bool = True):
     L.nmmo_reset.argtypes = [vp, vp, vp, vp, vp, vp]
     L.nmmo_step.restype = C.c_int
     L.nmmo_step.argtypes = [vp, vp, vp]
+    L.nmmo_step_envs.restype = C.c_int
+    L.nmmo_step_envs.argtypes = [vp, C.c_int, C.c_int, vp, vp]
     L.nmmo_step_host.restype = C.c_int
     L.nmmo_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
     L.nmmo_step_host_i16.restype = C.c_int
@@ -109,6 +111,8 @@ def load(build_if_missing: bool = True):
     L.nmmo_rollout_reset.argtypes = [vp, vp]
     L.nmmo_rollout_store.restype = C.c_int
     L.nmmo_rollout_store.argtypes = [vp] + [vp] * 8 + [C.c_int, vp]
+    L.nmmo_rollout_store_range.restype = C.c_int
+    L.nmmo_rollout_store_range.argtypes = [vp, C.c_int, C.c_int] + [vp] * 9 + [C.c_int, vp]
     L.nmmo_rollout_ptr.restype = C.c_int
     L.nmmo_rollout_ptr.argtypes = [vp, vp, C.POINTER(C.c_int)]
     L.nmmo_rollout_gae.restype = C.c_int
@@ -240,6 +244,15 @@ class Simulator:
         a = self.actions if actions is None else actions
         assert a.is_cuda and a.dtype == self.torch.int32 and a.is_contiguous() and a.numel() == self.E * self.P * 12
         self._check(self.L.nmmo_step(self.h, C.c_void_p(a.data_ptr()), self._stream()))
+
+    def step_envs(self, lo: int, hi: int, actions):
+        """Step envs [lo, hi) only: actions int32 CUDA tensor [hi - lo, P, 12] (row 0 = env lo). Asynchronous; ranges
+        stepped on different streams may overlap in time when they are disjoint."""
+        a = actions
+        assert a.is_cuda and a.dtype == self.torch.int32 and a.is_contiguous()
+        if a.numel() != max(int(hi) - int(lo), 0) * self.P * 12:
+            raise ValueError(f"actions of envs [{lo}, {hi}) must hold {(hi - lo) * self.P * 12} values, got {a.numel()}")
+        self._check(self.L.nmmo_step_envs(self.h, int(lo), int(hi), C.c_void_p(a.data_ptr()), self._stream()))
 
     def step_host(self, actions: np.ndarray, want_obs: bool = False):
         """Host-buffer call: actions [E,P,12] in host memory (pinned = async copies) as int32, int16 (half the

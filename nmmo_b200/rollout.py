@@ -92,24 +92,35 @@ class DeviceRollout:
         t = t if self.torch.is_tensor(t) else self.torch.as_tensor(t)
         return t.to(device=self.obs.device, dtype=dtype).contiguous()
 
-    def store(self, o, value, actions, logprob, r, d, mask, step: int, learner_mask=None, task_id=None):
+    def store(self, o, value, actions, logprob, r, d, mask, step: int, learner_mask=None, task_id=None, slot_base: int = 0):
         """Append one ``recv()`` (clean_pufferl.py:329-348); every argument is (or becomes) a CUDA tensor.  A compact
-        rollout also needs ``task_id`` (``sim.task_id``: int32 [n_slots] on the device)."""
+        rollout also needs ``task_id`` (``sim.task_id``: int32 [n_slots] on the device).
+
+        The arguments cover ``len(mask)`` slots starting at ``slot_base``: a ``recv()`` of an env pool hands out one batch,
+        whose rows are the global agent slots ``[slot_base, slot_base + len(mask))`` (``slot_base = lo * agents_per_env``
+        for ``pool.batch_env_range == (lo, hi)``); the sort key is the global slot.  ``task_id`` is then the batch's slice."""
         t = self.torch
-        o = self._dev(o, t.uint8); actions = self._dev(actions, t.int32).reshape(self.n_slots, 12)
+        mask = self._dev(mask, t.uint8).reshape(-1)
+        n = mask.numel()
+        o = self._dev(o, t.uint8); actions = self._dev(actions, t.int32).reshape(n, 12)
         value = self._dev(value, t.float32).reshape(-1); logprob = self._dev(logprob, t.float32).reshape(-1)
-        r = self._dev(r, t.float32).reshape(-1); d = self._dev(d, t.float32).reshape(-1); mask = self._dev(mask, t.uint8).reshape(-1)
+        r = self._dev(r, t.float32).reshape(-1); d = self._dev(d, t.float32).reshape(-1)
         lm = None if learner_mask is None else self._dev(learner_mask, t.uint8).reshape(-1)
+        for x in (value, logprob, r, d, lm):
+            if x is not None and x.numel() != n:
+                raise ValueError(f"store(): every per-slot argument must hold len(mask) = {n} entries")
+        if o.shape[0] != n:
+            raise ValueError(f"store(): obs must hold len(mask) = {n} records")
         p = lambda x: None if x is None else C.c_void_p(x.data_ptr())  # noqa: E731
+        tid = None
         if self.compact:
             if task_id is None:
                 raise NmmoError("compact rollout: store() needs task_id (Simulator.task_id)")
             tid = self._dev(task_id, t.int32).reshape(-1)
-            self._check(self.L.nmmo_rollout_store_compact(self.h, p(o), p(actions), p(logprob), p(value), p(r), p(d), p(mask), p(lm),
-                                                          p(tid), int(step), self._stream()))
-            return
-        self._check(self.L.nmmo_rollout_store(self.h, p(o), p(actions), p(logprob), p(value), p(r), p(d), p(mask), p(lm),
-                                              int(step), self._stream()))
+            if tid.numel() != n:
+                raise ValueError(f"store(): task_id must hold len(mask) = {n} entries")
+        self._check(self.L.nmmo_rollout_store_range(self.h, int(slot_base), n, p(o), p(actions), p(logprob), p(value), p(r), p(d),
+                                                    p(mask), p(lm), p(tid), int(step), self._stream()))
 
     def expand(self, idxs=None, n: int = None, out=None):
         """Whole observation records of rows ``idxs`` (int32 CUDA tensor; None = rows 0..n-1): the minibatch gather of

@@ -91,6 +91,31 @@ class DriverEnv:
         self.config = cfg
 
 
+class _BatchedSimulator(Simulator):
+    """Simulator of an env pool: the calls that touch the whole handle first make the current stream wait for every batch
+    stream, so they never run while a batch's step is in flight (nmmo_reset reads and writes back the scalars of every
+    env).  The other whole-handle calls (snapshot, inject_rng, stats, check, task_state) synchronise the device."""
+
+    batch_streams = ()
+
+    def join_batches(self):
+        cur = self.torch.cuda.current_stream(self.device)
+        for st in self.batch_streams:
+            cur.wait_stream(st)
+
+    def reset(self, *args, **kwargs):
+        self.join_batches()
+        return super().reset(*args, **kwargs)
+
+    def step(self, actions=None):
+        self.join_batches()
+        return super().step(actions)
+
+    def step_host(self, *args, **kwargs):
+        self.join_batches()
+        return super().step_host(*args, **kwargs)
+
+
 class B200VecEnv:
     def __init__(self, env_creator=None, env_args=None, env_kwargs: Optional[Dict] = None, num_envs: int = 1,
                  envs_per_worker: int = 1, envs_per_batch: Optional[int] = None, env_pool: bool = False,
@@ -101,9 +126,23 @@ class B200VecEnv:
         """collect_infos: "async" (default) -- finished-agent info records are compacted on the device, copied to
         pinned host memory on a side stream and handed out by the NEXT recv() (no host sync in the loop; call
         drain_infos() after the last step); True -- gathered synchronously inside recv() (exact tick, one host sync
-        per step); False -- never (use stats())."""
-        # env_creator / env_args / envs_per_worker / env_pool are accepted for signature
-        # compatibility; all envs of this backend step in lock-step on one GPU
+        per step); False -- never (use stats()).
+
+        envs_per_batch: b envs per recv()/send() (default num_envs: one lock-step tick per call).  b must divide num_envs;
+        the pool then holds K = num_envs / b batches of contiguous envs, batch k = envs [k*b, (k+1)*b), handed out in
+        the fixed order 0, 1, ..., K-1, 0, ... whatever env_pool says; each batch steps on its own CUDA stream while the
+        caller works on the batch it was handed.  recv() returns the batch's B = b * agents_per_env rows, with env_id
+        the batch's global agent slots (the LSTM-state index of clean_pufferl.py:313-314); batch_env_range is its
+        (lo, hi).  send() takes the actions of those B rows."""
+        # env_creator / env_args / envs_per_worker are accepted for signature compatibility
+        self.num_envs = int(num_envs)
+        b = self.num_envs if envs_per_batch is None else int(envs_per_batch)
+        if self.num_envs < 1 or not 1 <= b <= self.num_envs or self.num_envs % b:
+            raise ValueError(f"envs_per_batch must divide num_envs with 1 <= envs_per_batch <= num_envs (got {b} of {self.num_envs}); "
+                             "batches hold contiguous envs of equal size, e.g. 15 envs in batches of 5, or 18 in batches of 6")
+        self.envs_per_batch = b
+        self.num_batches = self.num_envs // b
+        self.env_pool = bool(env_pool)      # the batch order is round-robin either way (a legal "first ready" order)
         env_kwargs = env_kwargs or {}
         env_ns = env_kwargs.get("env") or default_env_args(resilient_population=0 if agent in ("takeru", "yaofeng", "hybrid") else 0.2)
         wrap_ns = env_kwargs.get("reward_wrapper") or default_wrapper_args(agent)
@@ -130,12 +169,9 @@ class B200VecEnv:
             te = np.ascontiguousarray(task_embed)
             self.task_embed = te.view(np.uint16) if te.dtype == np.float16 else te.astype(np.uint16)
             assert self.task_embed.shape == (self.task_table.shape[0], int(self.cfg[SPEC["NC_TASK_DIM"]]))
-        self.num_envs = int(num_envs)
-        self.envs_per_batch = self.num_envs if envs_per_batch is None else int(envs_per_batch)
-        if self.envs_per_batch != self.num_envs:
-            raise ValueError("B200VecEnv steps every env in lock-step: envs_per_batch must equal num_envs")
-        self.sim = Simulator(self.cfg, self.fcfg, self.num_envs, self.maps, self.task_table, self.task_embed,
-                             device=device, env_base=env_base)
+        sim_cls = Simulator if self.num_batches == 1 else _BatchedSimulator
+        self.sim = sim_cls(self.cfg, self.fcfg, self.num_envs, self.maps, self.task_table, self.task_embed,
+                           device=device, env_base=env_base)
         self.agents_per_env = self.sim.P
         self.stat_prefix = getattr(wrap_ns, "stat_prefix", None)
         self.collect_infos = collect_infos
@@ -151,7 +187,15 @@ class B200VecEnv:
         self._pending = False
         self.last_info_slots = []
         self.env_base = int(env_base)
-        self._info_cap = int(min(info_cap, self.num_envs * self.agents_per_env))
+        self._info_cap = int(min(info_cap, b * self.agents_per_env))
+        self._next_batch = 0
+        self.batch_env_range = (0, self.num_envs)      # envs [lo, hi) of the batch the last recv() returned
+        if self.num_batches > 1:
+            dev = self.sim.obs.device
+            self._streams = [torch.cuda.Stream(device=dev) for _ in range(self.num_batches)]
+            self._sent = [torch.cuda.Event() for _ in range(self.num_batches)]       # actions of batch k are ready
+            self._stepped = [torch.cuda.Event() for _ in range(self.num_batches)]    # batch k's outputs are ready
+            self.sim.batch_streams = self._streams
         self._info_q = None              # in-flight async gather: (event, n, idx, rows, done)
         self._info_stream = None
 
@@ -163,6 +207,7 @@ class B200VecEnv:
         self.sim.reset(global_seeds(int(seed), self.env_base, self.num_envs))
         self._info_q = None
         self._pending = True
+        self._next_batch = 0
 
     def reset_envs(self, env_indices, seeds, new_tasks=None):
         """Reset some envs, optionally assigning each a task (one table row for all of its agents): the
@@ -191,9 +236,9 @@ class B200VecEnv:
                                              task_names=self.task_names))
         return infos
 
-    def _enqueue_infos(self):
-        """Compact this tick's finished-agent records on the device (fixed capacity, no size read-back) and start their
-        copy to pinned host memory on a side stream."""
+    def _enqueue_infos(self, s0: int, s1: int):
+        """Compact the finished-agent records of slots [s0, s1) (this tick's, or the batch's) on the device (fixed
+        capacity, no size read-back) and start their copy to pinned host memory on a side stream."""
         t, s = self._torch, self.sim
         cap = self._info_cap
         if self._info_stream is None:
@@ -202,8 +247,11 @@ class B200VecEnv:
                                 t.empty((cap, s.info.shape[1]), dtype=t.float32).pin_memory(),
                                 t.empty(self.num_envs, dtype=t.uint8).pin_memory()) for _ in range(2)]
             self._info_flip = 0
-        n_d = s.info_valid.sum(dtype=t.int64).reshape(1)
-        idx_d = t.nonzero_static(s.info_valid, size=cap, fill_value=0).flatten()
+        valid = s.info_valid[s0:s1]
+        n_d = valid.sum(dtype=t.int64).reshape(1)
+        idx_d = t.nonzero_static(valid, size=cap, fill_value=0).flatten()
+        if s0:
+            idx_d += s0
         rows_d = s.info[idx_d]
         done_d = s.episode_done.clone()
         ev = t.cuda.Event()
@@ -216,7 +264,7 @@ class B200VecEnv:
             for x in (n_d, idx_d, rows_d, done_d):
                 x.record_stream(self._info_stream)
             ev.record(self._info_stream)
-        self._info_q = (ev, h, s.info_valid.clone())
+        self._info_q = (ev, h, valid.clone(), s0)
 
     def drain_infos(self):
         """Infos of the in-flight asynchronous gather (the last step's), if any."""
@@ -224,14 +272,16 @@ class B200VecEnv:
         self.last_info_slots = []
         if q is None:
             return []
-        ev, h, valid_d = q
+        ev, h, valid_d, s0 = q
         ev.synchronize()           # recorded a whole tick ago on a side stream: normally already complete
         n = int(h[0][0])
         if n > self._info_cap:
             # more agents finished in one tick than the staging holds (every env truncating at the horizon together):
             # gather them synchronously.  Their records are still intact: a slot cannot finish again in the tick
-            # that resets its env.
-            idx_d = valid_d.nonzero().flatten()
+            # that resets its env.  (An env pool's batch may be stepping again: wait for it first.)
+            if self.num_batches > 1:
+                self.sim.join_batches()
+            idx_d = valid_d.nonzero().flatten() + s0
             idx, rows = idx_d.cpu().numpy(), self.sim.info[idx_d].cpu().numpy()
         else:
             idx, rows = h[1][:n].numpy().copy(), h[2][:n].numpy()
@@ -249,25 +299,51 @@ class B200VecEnv:
         s = self.sim
         if not self._pending:
             raise RuntimeError("recv() without a preceding async_reset()/send(): the outputs on the device were already handed out")
+        P, b, k = self.agents_per_env, self.envs_per_batch, self._next_batch
+        lo, hi = k * b, (k + 1) * b
+        self.batch_env_range = (lo, hi)
+        s0, s1 = lo * P, hi * P
+        if self.num_batches > 1:
+            # the caller's stream waits for the batch's last step; the host does not
+            self._torch.cuda.current_stream(s.obs.device).wait_event(self._stepped[k])
         infos: List[Dict] = []
         self.last_info_slots = []        # flat agent slot (env * agents_per_env + agent) of each entry of `infos`
         if self.collect_infos == "async":
-            infos = self.drain_infos()   # the previous step's records (their copy ran underneath that step)
-            self._enqueue_infos()
+            infos = self.drain_infos()   # the previous recv()'s records (their copy ran underneath that step)
+            self._enqueue_infos(s0, s1)
         elif self.collect_infos:
-            valid = s.info_valid.nonzero().flatten()
+            # only this batch's flags: the other batches' still hold their last step, whose infos were handed out then
+            valid = s.info_valid[s0:s1].nonzero().flatten()
             if valid.numel():
+                if s0:
+                    valid += s0
                 idx = valid.cpu().numpy()
                 self.last_info_slots = idx
                 infos = self._infos_from(idx, s.info[valid].cpu().numpy(), s.episode_done.cpu().numpy())
         self._pending = False
-        return s.obs, s.rewards, s.terminated, s.truncated, infos, self.env_id, s.mask
+        if self.num_batches == 1:
+            return s.obs, s.rewards, s.terminated, s.truncated, infos, self.env_id, s.mask
+        return (s.obs[s0:s1], s.rewards[s0:s1], s.terminated[s0:s1], s.truncated[s0:s1], infos, self.env_id[s0:s1],
+                s.mask[s0:s1])
 
     def send(self, actions):
+        """actions: [B, 12] for the B = envs_per_batch * agents_per_env slots the last recv() returned."""
         t = self._torch
         a = actions if t.is_tensor(actions) else t.as_tensor(np.asarray(actions))
-        a = a.to(device=self.sim.obs.device, dtype=t.int32).reshape(self.num_envs, self.agents_per_env, 12).contiguous()
-        self.sim.step(a)
+        a = a.to(device=self.sim.obs.device, dtype=t.int32).reshape(self.envs_per_batch, self.agents_per_env, 12).contiguous()
+        if self.num_batches == 1:
+            self.sim.step(a)
+        else:
+            k = self._next_batch
+            lo, hi = self.batch_env_range
+            st = self._streams[k]
+            self._sent[k].record(t.cuda.current_stream(self.sim.obs.device))
+            st.wait_event(self._sent[k])
+            with t.cuda.stream(st):
+                self.sim.step_envs(lo, hi, a)
+                self._stepped[k].record(st)
+            a.record_stream(st)      # the caching allocator must not hand `a` out again before the step has read it
+            self._next_batch = (k + 1) % self.num_batches
         self._pending = True
 
     def close(self):
@@ -276,6 +352,8 @@ class B200VecEnv:
     # ---- extras --------------------------------------------------------------------------
     def stats(self, clear: bool = False) -> Dict[str, float]:
         """Means of the finished-agent infos since the last clear (clean_pufferl.py:381-390)."""
+        if self.num_batches > 1:
+            self.sim.join_batches()
         self.sim.check()             # a dropped event makes these means wrong: fail instead of reporting them
         sums, counts, counters = self.sim.stats(clear)
         out = {}
