@@ -86,13 +86,21 @@ def test_big_family_shapes(P, N, center, E, over):
     sim.close()
 
 
+def config5_stress_world():
+    """The configs[4] table shape with a 64-d task block and a folded engine default changed (NC_RES_DEPLETION): neither
+    is the std record layout / engine table, so a handle of this world runs the generic big kernels."""
+    return build_world(task_dim=64, n_maps=2, NC_N_PLAYERS=1024, NC_N_NPCS=2048, NC_MAP_CENTER=512, NC_HORIZON=48,
+                       NC_SPAWN_PATCH=32, NC_SAMPLE_MOVE_PCT=90, NC_SPAWN_IMMUNITY=5, NC_RES_DEPLETION=4)
+
+
 def test_config5_stress_shape():
-    """The configs[4] shape itself: 1024 players, 2048 NPCs, 544^2 map (centre 512 + 2 x 16 border), all players spawned
-    in a 32x32 patch, Move chosen with p = 0.9 by the built-in sampler, spawn immunity short enough that the crowd
-    fights.  Every observation, mask, reward, flag and (every 10 ticks) the full state against the oracle."""
-    world = build_world(task_dim=64, n_maps=2, NC_N_PLAYERS=1024, NC_N_NPCS=2048, NC_MAP_CENTER=512, NC_HORIZON=48,
-                        NC_SPAWN_PATCH=32, NC_SAMPLE_MOVE_PCT=90, NC_SPAWN_IMMUNITY=5, NC_RES_DEPLETION=4)
-    sim, oracles = _make(world, 2)
+    """The generic big kernels (nmmo_step_big_kernel / nmmo_obs_big_kernel) at the configs[4] table shape: 1024 players,
+    2048 NPCs, 544^2 map (centre 512 + 2 x 16 border), all players spawned in a 32x32 patch, Move chosen with p = 0.9 by
+    the built-in sampler, spawn immunity short enough that the crowd fights.  Every observation, mask, reward, flag and
+    (every 10 ticks) the full state against the oracle.  The 64-d task block and NC_RES_DEPLETION = 4 keep this world off
+    the compile-time-shape kernels that `bench.py --workload config5` runs; tests/test_config5_std_gpu.py checks those."""
+    sim, oracles = _make(config5_stress_world(), 2)
+    assert sim.kernel_names() == ("nmmo_step_big_kernel", "nmmo_obs_big_kernel")
     moved = []
 
     def watch(t, sim_, oracles_):

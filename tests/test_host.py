@@ -154,14 +154,8 @@ def test_pack_actions_u8_layout():
 def test_std_cfg_table_matches_the_python_defaults():
     """nm_cfg_std_value (csrc/nmmo_device.cuh): the engine defaults the *_std kernel instantiations fold to immediates must be
     the values nmmo_b200/config.py produces; entries the reference's Config or wrappers set stay run-time."""
-    import re
-    from pathlib import Path
-    from nmmo_b200.config import SPEC, make_config
-    text = (Path(__file__).resolve().parent.parent / "nmmo_b200" / "csrc" / "nmmo_device.cuh").read_text()
-    body = text[text.index("constexpr int nm_cfg_std_value"):text.index("default: return NM_CFG_RUNTIME")]
-    table = {}
-    for name, off, val in re.findall(r"case (NC_\w+)(?: \+ (\d+))?: return (-?\d+);", body):
-        table[SPEC[name] + int(off or 0)] = int(val)
+    from util import std_cfg_table
+    table = std_cfg_table()
     assert len(table) > 60
     for agent in ("takeru", "neurips23_start_kit", "yaofeng"):
         cfg, _ = make_config(agent=agent)

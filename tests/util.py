@@ -11,6 +11,16 @@ from nmmo_b200.mapgen import generate_maps
 from nmmo_b200.tasks import default_curriculum, make_task_table
 
 SMALL = dict(NC_N_PLAYERS=16, NC_N_NPCS=32, NC_MAP_CENTER=32)
+DEVICE_HEADER = Path(__file__).resolve().parent.parent / "nmmo_b200" / "csrc" / "nmmo_device.cuh"
+
+
+def std_cfg_table():
+    """nm_cfg_std_value (csrc/nmmo_device.cuh) as {config index: value}: the engine defaults that the *_std kernel
+    instantiations fold into immediates."""
+    import re
+    text = DEVICE_HEADER.read_text()
+    body = text[text.index("constexpr int nm_cfg_std_value"):text.index("default: return NM_CFG_RUNTIME")]
+    return {SPEC[name] + int(off or 0): int(val) for name, off, val in re.findall(r"case (NC_\w+)(?: \+ (\d+))?: return (-?\d+);", body)}
 
 
 def reference_file(*parts):
