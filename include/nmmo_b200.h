@@ -153,6 +153,27 @@ int nmmo_stats(nmmo_handle *h, double *sums, double *counts, uint64_t *counters,
  * counters were last cleared.  nmmo_step is asynchronous and cannot report it; the host-buffer calls do. */
 int nmmo_check(nmmo_handle *h);
 
+/* Environment state (DESIGN.md 2.3): one fixed-size blob per env, `bytes` long (header included, a multiple of 128), that
+ * holds everything a step reads and an earlier step or reset wrote: the tables, the agents' wrapper and task state, and
+ * the outputs recv() returns.  A blob loads into any slot of any handle created from the same config, maps, task table
+ * and task embeddings (a digest of them is in the header) and of the same kernel family; E, env_base, envs per CTA and
+ * the std / generic kernel choice do not matter.  The loaded env continues exactly as the saved one would have: every
+ * engine draw is keyed by the env's own seed.  The built-in random policy (nmmo_set_autosample, nmmo_sample_actions) is
+ * keyed by the global slot, so its draws after a load are those of the destination slot. */
+int nmmo_state_bytes(nmmo_handle *h, size_t *bytes);
+/* Writes the blobs of envs env_ids[0..n) (HOST int32, duplicates allowed) to DEVICE uint8 [n][bytes] (16-byte aligned).
+ * Asynchronous on `stream`.  NM_ERR_ARG for n < 1, an id out of range or misaligned states. */
+int nmmo_save_envs(nmmo_handle *h, const int32_t *env_ids, int n, uint8_t *states_dev, void *stream);
+/* Loads blob i of DEVICE uint8 [n][bytes] into env env_ids[i] (HOST int32, no duplicates; one blob may be repeated to
+ * load it into several slots), then rewrites the observation records, ActionTargets masks and built-in-policy rows of
+ * envs [min id, max id + 1) with the observation kernel, as nmmo_reset does: the loaded envs' become exactly those of
+ * the tick they were saved at.  Synchronises `stream` and reads the headers back before it touches any device state;
+ * the load and observation kernels then run on `stream`.  Like nmmo_reset it must be ordered after every range step in
+ * flight.  Leaves the nmmo_stats sums and counters 0-2 alone.  NM_ERR_ARG (the handle is unchanged) for n < 1, an id
+ * out of range, a duplicate id, misaligned states, a bad magic or format version, a blob of the other family, or a
+ * digest mismatch; NM_ERR_STATE while per-kernel timing or the phase profiler is on. */
+int nmmo_load_envs(nmmo_handle *h, const int32_t *env_ids, int n, const uint8_t *states_dev, void *stream);
+
 /* Per-kernel device timing (CUDA events recorded on the launching stream around the step kernel
  * and the observation kernel): enable, run steps, read the mean milliseconds per launch. */
 int nmmo_timing(nmmo_handle *h, int enable);

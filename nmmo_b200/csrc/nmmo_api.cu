@@ -13,6 +13,7 @@
 #include "nmmo_step.cu"
 #include "nmmo_obs.cu"
 #include "nmmo_rollout.cu"
+#include "nmmo_state.cu"
 
 static thread_local std::string g_err;
 static int fail(int code, const std::string &msg) { g_err = msg; return code; }
@@ -46,6 +47,8 @@ struct nmmo_handle {
   bool timing = false;
   std::vector<cudaEvent_t> ev;    // triples: before step kernel, between, after obs kernel
   size_t ev_used = 0;
+  // environment state blobs (nmmo_state.cu): the section table of this handle's family and shape, with the header
+  NmStateArgs state;
 };
 
 static size_t a16(size_t x) { return (x + 15) & ~(size_t)15; }
@@ -144,6 +147,59 @@ static int dalloc(nmmo_handle *h, T **ptr, size_t count, bool zero = true) {
 #define DA(ptr, count) do { int rc_ = dalloc(h, &(ptr), (count)); if (rc_) return rc_; } while (0)
 
 extern "C" const char *nmmo_last_error(void) { return g_err.c_str(); }
+
+// 64-bit digest of what a handle was created from (everything but n_envs, device and env_base): a state blob means
+// nothing under other maps (respawn reads the source map), another task table (task ids index it) or another config
+static uint64_t digest_bytes(uint64_t d, const void *data, size_t n) {
+  const uint8_t *b = (const uint8_t *)data;
+  d = nm_mix64(d ^ (uint64_t)n);
+  size_t i = 0;
+  for (; i + 8 <= n; i += 8) { uint64_t w; memcpy(&w, b + i, 8); d = nm_mix64(d ^ w); }
+  uint64_t w = 0;
+  memcpy(&w, b + i, n - i);
+  return nm_mix64(d ^ w);
+}
+
+// The blob layout (DESIGN.md 2.3): a header, then every per-env buffer that is state, each at a 16-byte-aligned offset.
+// It depends on the family and the shape only, not on E, env_base, envs per CTA or the std / generic kernel choice.
+static void state_layout(nmmo_handle *h, uint64_t digest) {
+  NmParams &p = h->prm;
+  NmStateArgs &a = h->state;
+  memset(&a, 0, sizeof(a));
+  uint32_t off = NM_STATE_HEADER;
+  auto add = [&](void *base, size_t h_env, size_t bytes, int live_sc = -1, int unit = 1) {
+    NmStateSec &q = a.sec[a.n_sec++];
+    q.h = (uint8_t *)base; q.h_env = (uint32_t)h_env; q.b_off = off; q.bytes = (uint32_t)bytes;
+    q.live_sc = (int16_t)live_sc; q.unit = (int16_t)unit;
+    off = (uint32_t)a16(off + bytes);
+  };
+  const size_t P = p.P, ent_bytes = (p.big ? (size_t)NM_BIG_ENT_STRIDE : (size_t)EA_N) * p.R * 2;
+  const size_t tile = p.big ? sizeof(VBig::tile_t) : sizeof(VSmall::tile_t), depl_cap = p.big ? VBig::kDeplCap : VSmall::kDeplCap;
+  a.sc_off = off;
+  add(p.scalars, NM_SC_N * 4, NM_SC_N * 4);
+  add(p.seed, 8, 8);
+  add(p.episode_done, 1, 1);
+  add(p.ent, ent_bytes, ent_bytes);
+  for (int k = 0; k < IS_N; k++) add(p.item + (size_t)k * p.CAP, (size_t)IS_N * p.CAP * 2, (size_t)p.CAP * 2, SC_ITEM_HI, 2);
+  add(p.map, (size_t)p.S * p.S / 2, (size_t)p.S * p.S / 2);
+  add(p.depl, depl_cap * tile, depl_cap * tile, SC_N_DEPL, (int)tile);
+  add(p.danger, (size_t)p.N * 2, (size_t)p.N * 2, SC_N_DANGER, 2);
+  add(p.stats, P * ST_N * 4, P * ST_N * 4);
+  add(p.dstats, P * DS_N * 8, P * DS_N * 8);
+  add(p.uniq, P * NM_UNIQ_WORDS * 4, P * NM_UNIQ_WORDS * 4);
+  add(p.task_id, P * 4, P * 4);
+  add(p.rew, P * 4, P * 4);
+  add(p.term, P, P); add(p.trunc, P, P); add(p.mask, P, P); add(p.info_valid, P, P);
+  add(p.info, P * IN_N * 4, P * IN_N * 4);
+  a.state_bytes = (off + 127) & ~127u;
+  for (int s = 0; s < a.n_sec; s++) a.sec[s].span = (s + 1 < a.n_sec ? a.sec[s + 1].b_off : a.state_bytes) - a.sec[s].b_off;
+  a.n_chunks = (a.state_bytes + NM_STATE_CHUNK - 1) / NM_STATE_CHUNK;
+  a.scalars = p.scalars; a.obs_meta = p.obs_meta; a.P = p.P;
+  a.hdr.magic = NM_STATE_MAGIC; a.hdr.version = NM_STATE_VERSION; a.hdr.family = (uint32_t)p.big;
+  a.hdr.state_bytes = a.state_bytes; a.hdr.digest = digest;
+}
+static_assert(IS_N + 17 <= NM_STATE_MAX_SECS, "state sections");
+static_assert(sizeof(NmStateArgs) <= 4096, "the section table and the env ids travel as kernel parameters");
 
 extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, int n_fcfg, int n_envs, int device,
                            int env_base, const uint8_t *maps, int n_maps, const int32_t *tasks,
@@ -288,6 +344,15 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   for (size_t e = 0; e < E; e++) sc[e * NM_SC_N + SC_DONE] = 1;
   CU(cudaMemcpy(p.scalars, sc.data(), sizeof(int32_t) * sc.size(), cudaMemcpyHostToDevice));
   if (const char *ov = getenv("NMMO_B200_H2D_SPLIT_MIN")) { int v = atoi(ov); if (v >= 1) h->h2d_split_min = v; }      // test hook
+  {
+    uint64_t d = 0x6E6D6D6F53544154ULL;
+    d = digest_bytes(d, cfg, sizeof(int32_t) * NC_COUNT);
+    d = digest_bytes(d, fcfg, sizeof(double) * NF_COUNT);
+    d = digest_bytes(d, maps, (size_t)n_maps * p.S * p.S);
+    d = digest_bytes(d, tasks, sizeof(int32_t) * n_tasks * NM_TASK_COLS);
+    d = digest_bytes(d, task_embed, sizeof(uint16_t) * n_tasks * p.L.task_dim);
+    state_layout(h, d);
+  }
   guard.armed = false;
   *out = h;
   return NM_OK;
@@ -781,4 +846,85 @@ extern "C" int nmmo_set_autosample(nmmo_handle *h, uint64_t seed, int32_t *actio
   h->prm.sample_out = actions_dev_out;
   h->prm.sample_seed = seed;
   return NM_OK;
+}
+
+// ------------------------------------------------------------------------------------------ environment state ----
+extern "C" int nmmo_state_bytes(nmmo_handle *h, size_t *bytes) {
+  if (!h || !bytes) return fail(NM_ERR_ARG, "null argument");
+  *bytes = h->state.state_bytes;
+  return NM_OK;
+}
+
+static int state_check_ids(nmmo_handle *h, const int32_t *env_ids, int n, const void *states, bool unique) {
+  if (!h) return fail(NM_ERR_ARG, "null handle");
+  if (n < 1) return fail(NM_ERR_ARG, "n must be at least 1");
+  if (!env_ids || !states) return fail(NM_ERR_ARG, "null argument");
+  std::vector<uint8_t> seen(unique ? h->prm.E : 0, 0);
+  for (int i = 0; i < n; i++) {
+    const int e = env_ids[i];
+    if (e < 0 || e >= h->prm.E) return fail(NM_ERR_ARG, "env id " + std::to_string(e) + " out of range [0, " + std::to_string(h->prm.E) + ")");
+    if (unique && seen[e]++) return fail(NM_ERR_ARG, "env id " + std::to_string(e) + " appears twice in a load");
+  }
+  if ((uintptr_t)states & 15) return fail(NM_ERR_ARG, "states must be 16-byte aligned");
+  return NM_OK;
+}
+
+// save / load kernels over env_ids, NM_STATE_IDS envs per launch; blob j of the call is states + j * state_bytes
+static int launch_state(nmmo_handle *h, bool save, const int32_t *env_ids, int n, uint8_t *states, cudaStream_t st) {
+  NmStateArgs a = h->state;
+  for (int k = 0; k < n; k += NM_STATE_IDS) {
+    a.n = std::min(NM_STATE_IDS, n - k);
+    memcpy(a.ids, env_ids + k, sizeof(int32_t) * a.n);
+    const unsigned grid = (unsigned)a.n * a.n_chunks;
+    uint8_t *blobs = states + (size_t)k * a.state_bytes;
+    if (save) nmmo_state_save_kernel<<<grid, NM_STATE_THREADS, 0, st>>>(a, blobs);
+    else nmmo_state_load_kernel<<<grid, NM_STATE_THREADS, 0, st>>>(a, blobs);
+    CU(cudaGetLastError());
+  }
+  return NM_OK;
+}
+
+extern "C" int nmmo_save_envs(nmmo_handle *h, const int32_t *env_ids, int n, uint8_t *states_dev, void *stream) {
+  int rc = state_check_ids(h, env_ids, n, states_dev, false);
+  if (rc) return rc;
+  CU(cudaSetDevice(h->device));
+  return launch_state(h, true, env_ids, n, states_dev, (cudaStream_t)stream);
+}
+
+extern "C" int nmmo_load_envs(nmmo_handle *h, const int32_t *env_ids, int n, const uint8_t *states_dev, void *stream) {
+  int rc = state_check_ids(h, env_ids, n, states_dev, true);
+  if (rc) return rc;
+  if (h->timing || h->prm.prof)
+    return fail(NM_ERR_STATE, "per-kernel timing and the phase profiler describe whole-handle launches: switch them off to load envs");
+  CU(cudaSetDevice(h->device));
+  const cudaStream_t st = (cudaStream_t)stream;
+  const NmStateArgs &a = h->state;
+  // every header is checked before any device state is touched: an NM_ERR_ARG return leaves the handle as it was
+  CU(cudaStreamSynchronize(st));
+  std::vector<NmStateHeader> hd(n);
+  CU(cudaMemcpy2DAsync(hd.data(), sizeof(NmStateHeader), states_dev, a.state_bytes, sizeof(NmStateHeader), n,
+                       cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  static const char *fam[2] = {"small", "big"};
+  for (int i = 0; i < n; i++) {
+    const NmStateHeader &x = hd[i];
+    const std::string which = "state " + std::to_string(i) + ": ";
+    if (x.magic != NM_STATE_MAGIC) return fail(NM_ERR_ARG, which + "not an environment state blob (bad magic)");
+    if (x.version != NM_STATE_VERSION)
+      return fail(NM_ERR_ARG, which + "format version " + std::to_string(x.version) + "; this build reads version " + std::to_string(NM_STATE_VERSION));
+    if (x.family != a.hdr.family)
+      return fail(NM_ERR_ARG, which + "saved by a " + std::string(x.family <= 1 ? fam[x.family] : "unknown") + "-family handle; this handle runs the " +
+                              fam[a.hdr.family] + " family");
+    if (x.state_bytes != a.state_bytes)
+      return fail(NM_ERR_ARG, which + "a blob of " + std::to_string(x.state_bytes) + " bytes; this handle's are " + std::to_string(a.state_bytes));
+    if (x.digest != a.hdr.digest)
+      return fail(NM_ERR_ARG, which + "digest mismatch: saved by a handle created with another config, maps, task table or task embeddings");
+  }
+  rc = launch_state(h, false, env_ids, n, (uint8_t *)states_dev, st);
+  if (rc) return rc;
+  // the loaded envs' records, ActionTargets masks and built-in-policy rows, rebuilt by the observation kernel as after a
+  // reset; the other envs of the span get the bytes they already hold
+  const int lo = *std::min_element(env_ids, env_ids + n), hi = *std::max_element(env_ids, env_ids + n) + 1;
+  NmParams prm = h->prm;
+  return launch_obs_kernel(h, prm, st, lo, hi);
 }

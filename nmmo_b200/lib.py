@@ -21,7 +21,7 @@ EXPORTS = [
     "nmmo_obs_ptr", "nmmo_reward_ptr", "nmmo_terminated_ptr", "nmmo_truncated_ptr", "nmmo_mask_ptr",
     "nmmo_info_ptr", "nmmo_info_valid_ptr", "nmmo_episode_done_ptr", "nmmo_task_id_ptr", "nmmo_task_embed_ptr", "nmmo_obs_stride", "nmmo_num_envs",
     "nmmo_num_agents", "nmmo_step_kernel_name", "nmmo_obs_kernel_name", "nmmo_inject_rng", "nmmo_snapshot", "nmmo_task_state", "nmmo_stats", "nmmo_check", "nmmo_timing", "nmmo_timing_read", "nmmo_profile", "nmmo_set_obs_full", "nmmo_set_autosample",
-    "nmmo_last_error",
+    "nmmo_state_bytes", "nmmo_save_envs", "nmmo_load_envs", "nmmo_last_error",
     "nmmo_rollout_create", "nmmo_rollout_create_compact", "nmmo_rollout_store_compact", "nmmo_rollout_expand", "nmmo_rollout_destroy", "nmmo_rollout_reset", "nmmo_rollout_store", "nmmo_rollout_store_range", "nmmo_rollout_ptr",
     "nmmo_rollout_gae", "nmmo_rollout_buffer", "nmmo_rollout_last_error",
 ]
@@ -97,6 +97,12 @@ def load(build_if_missing: bool = True):
     L.nmmo_set_autosample.argtypes = [vp, C.c_uint64, vp]
     L.nmmo_profile.restype = C.c_int
     L.nmmo_profile.argtypes = [vp, C.c_int, vp]
+    L.nmmo_state_bytes.restype = C.c_int
+    L.nmmo_state_bytes.argtypes = [vp, C.POINTER(C.c_size_t)]
+    L.nmmo_save_envs.restype = C.c_int
+    L.nmmo_save_envs.argtypes = [vp, vp, C.c_int, vp, vp]
+    L.nmmo_load_envs.restype = C.c_int
+    L.nmmo_load_envs.argtypes = [vp, vp, C.c_int, vp, vp]
     L.nmmo_last_error.restype = C.c_char_p
     L.nmmo_rollout_create.restype = C.c_int
     L.nmmo_rollout_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
@@ -213,6 +219,9 @@ class Simulator:
             self.task_id = view("nmmo_task_id_ptr", (n,), "<i4")
             self.task_embed_ptr = self.L.nmmo_task_embed_ptr(self.h)
             self.actions = torch.zeros((self.E, self.P, 12), dtype=torch.int32, device=dev)
+        nb = C.c_size_t()
+        self._check(self.L.nmmo_state_bytes(self.h, C.byref(nb)))
+        self.state_bytes = int(nb.value)      # bytes of one environment's saved state (save_envs / load_envs)
 
     def _check(self, rc: int):
         if rc != 0:
@@ -253,6 +262,33 @@ class Simulator:
         if a.numel() != max(int(hi) - int(lo), 0) * self.P * 12:
             raise ValueError(f"actions of envs [{lo}, {hi}) must hold {(hi - lo) * self.P * 12} values, got {a.numel()}")
         self._check(self.L.nmmo_step_envs(self.h, int(lo), int(hi), C.c_void_p(a.data_ptr()), self._stream()))
+
+    def save_envs(self, env_ids, out=None):
+        """Saved state of envs `env_ids` (duplicates allowed) -> uint8 CUDA tensor [n, state_bytes] on this handle's device
+        (or `out`, a contiguous uint8 tensor of that shape there).  Asynchronous on the current stream.  torch.save of the
+        tensor is a checkpoint of those envs (DESIGN.md 2.3)."""
+        ids = np.ascontiguousarray(np.asarray(env_ids, np.int64).reshape(-1), np.int32)
+        t = self.torch
+        if out is None:
+            out = t.empty((len(ids), self.state_bytes), dtype=t.uint8, device=t.device("cuda", self.device))
+        if not (out.is_cuda and out.device.index == self.device and out.dtype == t.uint8 and out.is_contiguous()
+                and tuple(out.shape) == (len(ids), self.state_bytes)):
+            raise ValueError(f"out must be a contiguous uint8 tensor [{len(ids)}, {self.state_bytes}] on cuda:{self.device}")
+        self._check(self.L.nmmo_save_envs(self.h, _p(ids), len(ids), C.c_void_p(out.data_ptr()), self._stream()))
+        return out
+
+    def load_envs(self, env_ids, states):
+        """Load states[i] (a row of save_envs, from this or another handle of the same world and family) into env
+        env_ids[i]; a CPU tensor, e.g. one read back with torch.load, is copied to the device first.  The loaded envs'
+        observations, masks, outputs and built-in-policy rows become those of the tick they were saved at; their next
+        step continues the saved episode."""
+        ids = np.ascontiguousarray(np.asarray(env_ids, np.int64).reshape(-1), np.int32)
+        t = self.torch
+        s = states if t.is_tensor(states) else t.as_tensor(np.asarray(states))
+        if s.dtype != t.uint8 or tuple(s.shape) != (len(ids), self.state_bytes):
+            raise ValueError(f"states must be uint8 [{len(ids)}, {self.state_bytes}], got {s.dtype} {tuple(s.shape)}")
+        s = s.to(device=t.device("cuda", self.device), non_blocking=False).contiguous()
+        self._check(self.L.nmmo_load_envs(self.h, _p(ids), len(ids), C.c_void_p(s.data_ptr()), self._stream()))
 
     def step_host(self, actions: np.ndarray, want_obs: bool = False):
         """Host-buffer call: actions [E,P,12] in host memory (pinned = async copies) as int32, int16 (half the

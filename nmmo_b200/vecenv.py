@@ -115,6 +115,14 @@ class _BatchedSimulator(Simulator):
         self.join_batches()
         return super().step_host(*args, **kwargs)
 
+    def save_envs(self, *args, **kwargs):
+        self.join_batches()
+        return super().save_envs(*args, **kwargs)
+
+    def load_envs(self, *args, **kwargs):
+        self.join_batches()
+        return super().load_envs(*args, **kwargs)
+
 
 class B200VecEnv:
     def __init__(self, env_creator=None, env_args=None, env_kwargs: Optional[Dict] = None, num_envs: int = 1,
@@ -220,6 +228,20 @@ class B200VecEnv:
             task_ids = np.zeros((E, P), np.int32)
             task_ids[np.asarray(env_indices)] = np.asarray(new_tasks, np.int32).reshape(-1, 1)
         self.sim.reset(sd, task_ids=task_ids, env_mask=mask)
+        self._pending = True
+
+    def save_envs(self, env_indices):
+        """Saved state of envs `env_indices` -> uint8 CUDA tensor [n, sim.state_bytes] (DESIGN.md 2.3).  Call it where
+        reset_envs may be called; a batch in flight finishes first.  A checkpoint of the whole pool is
+        ``torch.save(pool.save_envs(range(pool.num_envs)), path)`` next to the trainer's own checkpoint."""
+        return self.sim.save_envs(env_indices)
+
+    def load_envs(self, env_indices, states):
+        """Put saved states (rows of save_envs, from this pool or another one of the same world) into envs
+        `env_indices`, where reset_envs may be called.  Like reset_envs it leaves the outputs pending: the restored envs'
+        observations, rewards, flags and masks appear in their batch's next recv(), and so do the infos of the tick
+        they were saved at, which are handed out again."""
+        self.sim.load_envs(env_indices, states)
         self._pending = True
 
     def sim_env_base(self) -> int:
