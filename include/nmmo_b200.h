@@ -174,6 +174,25 @@ int nmmo_save_envs(nmmo_handle *h, const int32_t *env_ids, int n, uint8_t *state
  * digest mismatch; NM_ERR_STATE while per-kernel timing or the phase profiler is on. */
 int nmmo_load_envs(nmmo_handle *h, const int32_t *env_ids, int n, const uint8_t *states_dev, void *stream);
 
+/* Event log (DESIGN.md 2.4): the player events each env emitted in its last step, as the reference's event log holds
+ * them.  enable = 1 allocates the staging (E * ring size * 8 bytes: 32 MB for 4096 envs of the default shape) and zeroes
+ * every env's count (also when already on); 0 frees it.  From then on every step call (nmmo_step, nmmo_step_envs, the
+ * step_host calls) keeps each stepped env's events; an env the call resets has none, and so has an env that nmmo_reset
+ * resets or nmmo_load_envs loads (the events are not part of a state blob).  Synchronises the device, so it is ordered
+ * after every range step in flight.  With the log off, the step kernels do what they did without it. */
+int nmmo_set_event_log(nmmo_handle *h, int enable);
+/* Rows of the events of envs [env_lo, env_hi) -> DEVICE int32 rows_dev[cap][9], each
+ * [env, ent_id, tick, event, type, level, number, gold, target]: env is the handle's env index, ent_id the agent row + 1,
+ * tick the env's tick after the step, event the reference's EventCode; number and gold are sign-extended, target is the
+ * target's entity id (players > 0, NPCs < 0) for SCORE_HIT, PLAYER_KILL, LOOT_ITEM and LOOT_GOLD and 0 otherwise.
+ * Columns 1..8 are those of the reference's EventLogger rows.  Order: env, then agent, then the order the agent's events
+ * happened in.  DEVICE int32 count_dev[0] receives the number of rows of the range, which may exceed cap; rows beyond
+ * cap are not written.  An env whose event ring overflowed has the events the ring kept (nmmo_check reports the
+ * overflow).  Asynchronous on `stream`, no host synchronisation.  NM_ERR_STATE while the log is off; NM_ERR_ARG for an
+ * empty, reversed or out-of-bounds range, cap < 0, or a NULL or not 4-byte-aligned pointer (rows_dev may be NULL when
+ * cap = 0). */
+int nmmo_events(nmmo_handle *h, int env_lo, int env_hi, int32_t *rows_dev, int cap, int32_t *count_dev, void *stream);
+
 /* Per-kernel device timing (CUDA events recorded on the launching stream around the step kernel
  * and the observation kernel): enable, run steps, read the mean milliseconds per launch. */
 int nmmo_timing(nmmo_handle *h, int enable);

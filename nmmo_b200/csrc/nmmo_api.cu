@@ -14,6 +14,7 @@
 #include "nmmo_obs.cu"
 #include "nmmo_rollout.cu"
 #include "nmmo_state.cu"
+#include "nmmo_events.cu"
 
 static thread_local std::string g_err;
 static int fail(int code, const std::string &msg) { g_err = msg; return code; }
@@ -49,6 +50,9 @@ struct nmmo_handle {
   size_t ev_used = 0;
   // environment state blobs (nmmo_state.cu): the section table of this handle's family and shape, with the header
   NmStateArgs state;
+  // event log (nmmo_events.cu): first row of each env in its nmmo_events call ([E]; calls over disjoint ranges touch
+  // disjoint entries); allocated with the staging
+  int32_t *ev_off = nullptr;
 };
 
 static size_t a16(size_t x) { return (x + 15) & ~(size_t)15; }
@@ -368,6 +372,7 @@ extern "C" int nmmo_destroy(nmmo_handle *h) {
   for (cudaEvent_t e : h->ev) cudaEventDestroy(e);
   if (h->h2d_stream) { cudaStreamDestroy(h->h2d_stream); cudaEventDestroy(h->ev_entry); cudaEventDestroy(h->ev_h2d[0]); cudaEventDestroy(h->ev_h2d[1]); }
   if (h->copy_stream) { cudaStreamDestroy(h->copy_stream); cudaEventDestroy(h->ev_step_done); cudaEventDestroy(h->ev_copy_done); cudaFreeHost(h->h_overflow); }
+  if (h->prm.ev_log) { cudaFree(h->prm.ev_log); cudaFree(h->prm.ev_n); cudaFree(h->ev_off); }
   delete h;
   return NM_OK;
 }
@@ -877,6 +882,7 @@ static int launch_state(nmmo_handle *h, bool save, const int32_t *env_ids, int n
     memcpy(a.ids, env_ids + k, sizeof(int32_t) * a.n);
     const unsigned grid = (unsigned)a.n * a.n_chunks;
     uint8_t *blobs = states + (size_t)k * a.state_bytes;
+    a.ev_n = h->prm.ev_n;
     if (save) nmmo_state_save_kernel<<<grid, NM_STATE_THREADS, 0, st>>>(a, blobs);
     else nmmo_state_load_kernel<<<grid, NM_STATE_THREADS, 0, st>>>(a, blobs);
     CU(cudaGetLastError());
@@ -927,4 +933,51 @@ extern "C" int nmmo_load_envs(nmmo_handle *h, const int32_t *env_ids, int n, con
   const int lo = *std::min_element(env_ids, env_ids + n), hi = *std::max_element(env_ids, env_ids + n) + 1;
   NmParams prm = h->prm;
   return launch_obs_kernel(h, prm, st, lo, hi);
+}
+
+// ------------------------------------------------------------------------------------------------ event log ----
+extern "C" int nmmo_set_event_log(nmmo_handle *h, int enable) {
+  if (!h) return fail(NM_ERR_ARG, "null handle");
+  CU(cudaSetDevice(h->device));
+  CU(cudaDeviceSynchronize());      // no step in flight may write the staging while it changes
+  NmParams &p = h->prm;
+  if (!enable) {
+    if (p.ev_log) { CU(cudaFree(p.ev_log)); CU(cudaFree(p.ev_n)); CU(cudaFree(h->ev_off)); }
+    p.ev_log = nullptr; p.ev_n = nullptr; h->ev_off = nullptr;
+    return NM_OK;
+  }
+  if (!p.ev_log) {
+    uint2 *log = nullptr; int32_t *n = nullptr, *off = nullptr;
+    cudaError_t e = cudaMalloc((void **)&log, (size_t)p.E * p.ev_cap * sizeof(uint2));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&n, (size_t)p.E * sizeof(int32_t));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&off, (size_t)p.E * sizeof(int32_t));
+    if (e != cudaSuccess) {
+      cudaFree(log); cudaFree(n); cudaFree(off);
+      return fail(NM_ERR_CUDA, std::string("event log staging: ") + cudaGetErrorString(e));
+    }
+    p.ev_log = log; p.ev_n = n; h->ev_off = off;
+  }
+  CU(cudaMemset(p.ev_n, 0, (size_t)p.E * sizeof(int32_t)));
+  return NM_OK;
+}
+
+extern "C" int nmmo_events(nmmo_handle *h, int env_lo, int env_hi, int32_t *rows_dev, int cap, int32_t *count_dev, void *stream) {
+  if (!h) return fail(NM_ERR_ARG, "null handle");
+  const NmParams &p = h->prm;
+  if (!p.ev_log) return fail(NM_ERR_STATE, "the event log is off: nmmo_set_event_log(h, 1) first");
+  if (env_lo < 0 || env_hi > p.E || env_lo >= env_hi) return fail(NM_ERR_ARG, "env range must satisfy 0 <= env_lo < env_hi <= E");
+  if (cap < 0) return fail(NM_ERR_ARG, "cap must be >= 0");
+  if (!count_dev || (cap > 0 && !rows_dev)) return fail(NM_ERR_ARG, "null argument");
+  if (((uintptr_t)rows_dev | (uintptr_t)count_dev) & 3) return fail(NM_ERR_ARG, "rows and count must be 4-byte aligned");
+  CU(cudaSetDevice(h->device));
+  const cudaStream_t st = (cudaStream_t)stream;
+  nmmo_events_scan_kernel<<<1, NM_EV_SCAN_THREADS, 0, st>>>(p.ev_n, env_lo, env_hi, h->ev_off, count_dev);
+  CU(cudaGetLastError());
+  if (cap == 0) return NM_OK;
+  NmEventsArgs a;
+  a.ev_log = p.ev_log; a.ev_n = p.ev_n; a.off = h->ev_off; a.scalars = p.scalars;
+  a.ev_cap = p.ev_cap; a.P = p.P; a.lo = env_lo; a.rows = rows_dev; a.cap = cap;
+  nmmo_events_kernel<<<env_hi - env_lo, NM_EV_THREADS, (size_t)(p.P + p.ev_cap) * sizeof(int), st>>>(a);
+  CU(cudaGetLastError());
+  return NM_OK;
 }

@@ -102,6 +102,10 @@ struct NmParams {
   int env_lo, env_hi;          // step and observation kernels: the environments this launch covers
   int act_env_lo;              // env whose actions are row 0 of `actions` (0 = a whole-handle buffer; nmmo_step_envs: its env_lo)
   int env_base;                // global env index of env 0 (multi-GPU sharding; seeds derive from it)
+  // event log (nmmo_set_event_log; NULL = off): the step kernel keeps each env's events of the call here, the ring as
+  // emitted, and their count (0 for an env the call resets); nmmo_events turns them into rows (nmmo_events.cu)
+  uint2 *ev_log;               // [E][ev_cap]
+  int32_t *ev_n;               // [E]
 };
 
 // The reference's default shape (config 2: 128 players, 256 NPCs, 160^2 map, N_ent 100, N_mkt 384, 12 inventory rows,

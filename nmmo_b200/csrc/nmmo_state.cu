@@ -37,6 +37,7 @@ struct NmStateArgs {
   uint32_t state_bytes, n_chunks, sc_off;      // sc_off: blob offset of the scalars section
   const int32_t *scalars;                      // save: the handle's scalars (live prefixes)
   uint32_t *obs_meta;                          // load: OM_TASK is cleared for the loaded envs' agents
+  int32_t *ev_n;                               // load, event log on: the loaded envs have no events
   int P;
   NmStateHeader hdr;
   int n;
@@ -94,6 +95,7 @@ __device__ __forceinline__ void state_body(const NmStateArgs &a, uint8_t *blobs)
     } else {
       // the Task block of the slot's records may hold another task: the observation pass after the load rewrites it
       for (int i = threadIdx.x; i < a.P; i += blockDim.x) a.obs_meta[(size_t)env * a.P + i] &= ~OM_TASK;
+      if (a.ev_n && threadIdx.x == 0) a.ev_n[env] = 0;
     }
   }
   for (int s = 0; s < a.n_sec; s++) {

@@ -155,6 +155,10 @@ template <class V>
 __device__ void emit(const Ctx<V> &ctx, int prow, int code, int type, int level, int number, int gold, int target) {
   int i = atomicAdd(&ctx.sc[0], 1);
   if (i >= ctx.p->ev_cap) { ctx.sc[1] = 1; return; }      // ev_cap = V::kEvCap (a test hook can lower it)
+  // the target's id (players > 0, NPCs < 0) goes into the half of w1 its event leaves zero: number for LOOT_GOLD, gold
+  // for SCORE_HIT, PLAYER_KILL and LOOT_ITEM.  fold_event reads neither there, and `code` is a constant at every call.
+  if (code == EV_LOOT_GOLD) number = target;
+  else if (target != 0) gold = target;
   // agent 16 bits | dense event 5 | item type / skill 5 | level 4 | target sign 2
   uint32_t w0 = (uint32_t)prow | ((uint32_t)nm_dense_event(code) << 16) | ((uint32_t)type << 21) |
                 ((uint32_t)(level & 15) << 26) | (target > 0 ? (1u << 30) : 0u) | (target < 0 ? (1u << 31) : 0u);
@@ -1267,6 +1271,7 @@ __device__ NM_RESET_INLINE void reset_env(const NmParams &P_, int env, uint64_t 
     sc[SC_TICK] = 0; sc[SC_DONE] = 0; sc[SC_NEXT_NPC_ID] = -1; sc[SC_N_DANGER] = 0; sc[SC_MAP_ID] = map_id;
     sc[SC_FRESH] = 1; sc[SC_ITEM_HI] = 0; sc[SC_N_DEPL] = 0; sc[SC_NEED_RESET] = 0; sc[SC_EXPLICIT_MAP] = 0; sc[SC_EXPLICIT_TASKS] = 0;
     P_.episode_done[env] = 0;
+    if (P_.ev_n) P_.ev_n[env] = 0;      // a reset env has no events in the event log
   }
 }
 
@@ -2125,8 +2130,14 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
     {
       const int nev = min(ctx.sc[0], prm.ev_cap);
       PCOUNT(26, nev);
+      uint2 *const ev_log = prm.ev_log ? prm.ev_log + (size_t)env * prm.ev_cap : nullptr;      // event log on: keep the ring
+      if (ev_log && tid == 0) prm.ev_n[env] = nev;
       #pragma unroll 1
-      for (int i = T - 1 - tid; i < nev; i += T) fold_event(ctx, ctx.ev[i]);
+      for (int i = T - 1 - tid; i < nev; i += T) {
+        const uint2 e = ctx.ev[i];
+        if (ev_log) ev_log[i] = e;
+        fold_event(ctx, e);
+      }
     }
     // one draw per depleted tile; the tiles that stay depleted form next tick's list
     #pragma unroll 1

@@ -56,6 +56,30 @@ class TaskView:
         self.progress_info = {"max_progress": float(max_progress), "completed_tick": int(completed) if completed else None}
 
 
+class EventLogView:
+    """``realm.event_log`` of the reference (nmmo/lib/event_log.py EventLogger) over the episode's rows: int32
+    [n, 9] = [id, ent_id, tick, event, type, level, number, gold, target_ent], id the running row number.  Each tick's
+    rows are ordered by agent, then by the order the agent's events happened in."""
+
+    attr_to_col = {"event": 3, "type": 4, "item_type": 4, "combat_style": 4, "skill": 4, "level": 5, "number": 6,
+                   "distance": 6, "damage": 6, "quantity": 6, "gold": 7, "price": 7, "target_ent": 8}
+
+    def __init__(self, rows: np.ndarray, tick: int):
+        self._rows, self._tick = rows, int(tick)
+
+    def get_data(self, event_code=None, agents=None, tick=None) -> np.ndarray:
+        """Rows of event `event_code` (an EventCode), of the agents (ent ids) in `agents`, at tick `tick` (-1: the
+        current tick); None keeps every row on that axis."""
+        log = self._rows
+        if event_code is not None:
+            log = log[log[:, 3] == int(event_code)]
+        if agents is not None:
+            log = log[np.isin(log[:, 1], np.asarray(list(agents), np.int64))]
+        if tick is not None:
+            log = log[log[:, 2] == (self._tick if int(tick) == -1 else int(tick))]
+        return log
+
+
 ACTION_KEYS = [("Attack", "Style"), ("Attack", "Target"), ("Buy", "MarketItem"), ("Destroy", "InventoryItem"),
                ("Give", "InventoryItem"), ("Give", "Target"), ("GiveGold", "Price"), ("GiveGold", "Target"),
                ("Move", "Direction"), ("Sell", "InventoryItem"), ("Sell", "Price"), ("Use", "InventoryItem")]
@@ -71,6 +95,10 @@ class EnvView:
         self.max_num_agents = self.P
         self.config = SimpleNamespace(COMBAT_SPAWN_IMMUNITY=int(sim.cfg[SPEC["NC_SPAWN_IMMUNITY"]]), PLAYER_N=self.P,
                                       HORIZON=int(sim.cfg[SPEC["NC_HORIZON"]]))      # yaofeng/reward_wrapper.py:33
+        # the episode's event log, accumulated on the host from the device rows of every step (realm.event_log)
+        sim.set_event_log(True)
+        self._log = np.zeros((0, 9), np.int32)
+        self._log_done = False      # the env finished its episode: the next step resets it and starts a new log
 
     def _slice(self, t):
         return t[self.k * self.P:(self.k + 1) * self.P].cpu().numpy()
@@ -94,6 +122,8 @@ class EnvView:
         if new_task is not None:
             task_ids = np.zeros((self.sim.E, self.P), np.int32); task_ids[self.k] = int(new_task)
         self.sim.reset(seeds, task_ids=task_ids, env_mask=mask)
+        self._log = np.zeros((0, 9), np.int32)
+        self._log_done = False
         present = self._slice(self.sim.mask).astype(bool)
         self.agents = [p + 1 for p in range(self.P) if present[p]]
         return self._obs(present), {a: {} for a in self.agents}
@@ -112,6 +142,8 @@ class EnvView:
         rew, term, trunc = self._slice(self.sim.rewards), self._slice(self.sim.terminated), self._slice(self.sim.truncated)
         iv, info = self._slice(self.sim.info_valid), self._slice(self.sim.info)
         done = bool(self.sim.episode_done[self.k].item())
+        self._append_events()
+        self._log_done = done
         ids = [p + 1 for p in range(self.P) if present[p]]
         infos = {a: (info_record_to_dict(info[a - 1]) if iv[a - 1] else {}) for a in ids}
         if done and ids:
@@ -120,6 +152,15 @@ class EnvView:
         return (self._obs(present), {a: float(rew[a - 1]) for a in ids}, {a: bool(term[a - 1]) for a in ids},
                 {a: bool(trunc[a - 1]) for a in ids}, infos)
 
+    def _append_events(self):
+        rows, cnt = self.sim.events(self.k, self.k + 1)
+        n = int(cnt.item())
+        if n > rows.shape[0]:
+            rows, _ = self.sim.events(self.k, self.k + 1, out=rows.new_empty((n, 9)))
+        new = rows[:n].cpu().numpy()
+        new[:, 0] = np.arange(1, n + 1) + (0 if self._log_done else len(self._log))
+        self._log = new if self._log_done else np.concatenate([self._log, new])
+
     @property
     def tick(self):
         return int(self.sim.snapshot(self.k)[3][0])
@@ -127,8 +168,8 @@ class EnvView:
     @property
     def realm(self):
         """``env.realm`` as the wrappers use it: ``tick``, ``players[id]``, ``players.dead_this_tick``
-        (stat_wrapper.py:136,140).  The per-tick event log is folded on the device and not kept
-        (``event_log.get_data`` is unavailable; its consumers' results are in the episode info)."""
+        (stat_wrapper.py:136,140) and ``event_log.get_data`` (stat_wrapper.py:123): the episode's player events,
+        exported from the device after every step (Simulator.events) and kept on the host until the next reset."""
         ent, items, _, sc = self.sim.snapshot(self.k)
         cfg = self.sim.cfg
 
@@ -147,7 +188,7 @@ class EnvView:
         st = ent[:self.P, SPEC["EA_STATUS"]]
         players = _Players({p + 1: PlayerView(ent[p], defense(ent[p])) for p in range(self.P) if st[p] == SPEC["ES_ALIVE"]})
         players.dead_this_tick = {p + 1: PlayerView(ent[p], 0) for p in range(self.P) if st[p] == SPEC["ES_DEAD_THIS_TICK"]}
-        return SimpleNamespace(tick=int(sc[0]), players=players)
+        return SimpleNamespace(tick=int(sc[0]), players=players, event_log=EventLogView(self._log, int(sc[0])))
 
     @property
     def agent_task_map(self):

@@ -21,7 +21,7 @@ EXPORTS = [
     "nmmo_obs_ptr", "nmmo_reward_ptr", "nmmo_terminated_ptr", "nmmo_truncated_ptr", "nmmo_mask_ptr",
     "nmmo_info_ptr", "nmmo_info_valid_ptr", "nmmo_episode_done_ptr", "nmmo_task_id_ptr", "nmmo_task_embed_ptr", "nmmo_obs_stride", "nmmo_num_envs",
     "nmmo_num_agents", "nmmo_step_kernel_name", "nmmo_obs_kernel_name", "nmmo_inject_rng", "nmmo_snapshot", "nmmo_task_state", "nmmo_stats", "nmmo_check", "nmmo_timing", "nmmo_timing_read", "nmmo_profile", "nmmo_set_obs_full", "nmmo_set_autosample",
-    "nmmo_state_bytes", "nmmo_save_envs", "nmmo_load_envs", "nmmo_last_error",
+    "nmmo_state_bytes", "nmmo_save_envs", "nmmo_load_envs", "nmmo_set_event_log", "nmmo_events", "nmmo_last_error",
     "nmmo_rollout_create", "nmmo_rollout_create_compact", "nmmo_rollout_store_compact", "nmmo_rollout_expand", "nmmo_rollout_destroy", "nmmo_rollout_reset", "nmmo_rollout_store", "nmmo_rollout_store_range", "nmmo_rollout_ptr",
     "nmmo_rollout_gae", "nmmo_rollout_buffer", "nmmo_rollout_last_error",
 ]
@@ -103,6 +103,10 @@ def load(build_if_missing: bool = True):
     L.nmmo_save_envs.argtypes = [vp, vp, C.c_int, vp, vp]
     L.nmmo_load_envs.restype = C.c_int
     L.nmmo_load_envs.argtypes = [vp, vp, C.c_int, vp, vp]
+    L.nmmo_set_event_log.restype = C.c_int
+    L.nmmo_set_event_log.argtypes = [vp, C.c_int]
+    L.nmmo_events.restype = C.c_int
+    L.nmmo_events.argtypes = [vp, C.c_int, C.c_int, vp, C.c_int, vp, vp]
     L.nmmo_last_error.restype = C.c_char_p
     L.nmmo_rollout_create.restype = C.c_int
     L.nmmo_rollout_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
@@ -289,6 +293,31 @@ class Simulator:
             raise ValueError(f"states must be uint8 [{len(ids)}, {self.state_bytes}], got {s.dtype} {tuple(s.shape)}")
         s = s.to(device=t.device("cuda", self.device), non_blocking=False).contiguous()
         self._check(self.L.nmmo_load_envs(self.h, _p(ids), len(ids), C.c_void_p(s.data_ptr()), self._stream()))
+
+    def set_event_log(self, enable: bool = True):
+        """Event log on (allocates E * ring size * 8 bytes of device staging, zeroes every env's events) or off (frees
+        it).  While it is on, every step keeps the player events each stepped env emitted; events() hands them out."""
+        self._check(self.L.nmmo_set_event_log(self.h, int(bool(enable))))
+
+    def events(self, lo: int = 0, hi: Optional[int] = None, out=None, count=None):
+        """The last step's events of envs [lo, hi) (default all) -> (rows int32 CUDA [cap, 9], count int32 CUDA [1]).
+        A row is [env, ent_id, tick, event, type, level, number, gold, target] (columns 1..8 as in the reference's event
+        log; env is the handle's env index), ordered by env, agent, then the order the agent's events happened in.
+        count[0] is the number of rows of the range; only the first cap = len(out) of them are written (without `out`,
+        cap = (hi - lo) * max(8 * P, 1024)).  Asynchronous on the current stream: nothing is read back to the host."""
+        t = self.torch
+        hi = self.E if hi is None else int(hi)
+        dev = t.device("cuda", self.device)
+        if out is None:
+            out = t.empty((max(hi - int(lo), 0) * max(8 * self.P, 1024), 9), dtype=t.int32, device=dev)
+        if count is None:
+            count = t.empty(1, dtype=t.int32, device=dev)
+        for name, x, shape in (("out", out, (out.shape[0], 9)), ("count", count, (1,))):
+            if not (x.is_cuda and x.device.index == self.device and x.dtype == t.int32 and x.is_contiguous() and tuple(x.shape) == shape):
+                raise ValueError(f"{name} must be a contiguous int32 tensor {list(shape)} on cuda:{self.device}")
+        self._check(self.L.nmmo_events(self.h, int(lo), hi, C.c_void_p(out.data_ptr()), int(out.shape[0]),
+                                       C.c_void_p(count.data_ptr()), self._stream()))
+        return out, count
 
     def step_host(self, actions: np.ndarray, want_obs: bool = False):
         """Host-buffer call: actions [E,P,12] in host memory (pinned = async copies) as int32, int16 (half the

@@ -123,6 +123,10 @@ class _BatchedSimulator(Simulator):
         self.join_batches()
         return super().load_envs(*args, **kwargs)
 
+    def set_event_log(self, *args, **kwargs):
+        self.join_batches()
+        return super().set_event_log(*args, **kwargs)
+
 
 class B200VecEnv:
     def __init__(self, env_creator=None, env_args=None, env_kwargs: Optional[Dict] = None, num_envs: int = 1,
@@ -130,7 +134,7 @@ class B200VecEnv:
                  mask_agents: bool = True, agent: str = "takeru", device: int = 0, env_base: int = 0,
                  maps: Optional[np.ndarray] = None, task_rows=None, map_seed: int = 2023, collect_infos="async",
                  task_embed: Optional[np.ndarray] = None, info_cap: int = 16384, curriculum: Optional[str] = None,
-                 task_names: Optional[List[str]] = None):
+                 task_names: Optional[List[str]] = None, event_log_cap: int = 0):
         """collect_infos: "async" (default) -- finished-agent info records are compacted on the device, copied to
         pinned host memory on a side stream and handed out by the NEXT recv() (no host sync in the loop; call
         drain_infos() after the last step); True -- gathered synchronously inside recv() (exact tick, one host sync
@@ -141,7 +145,13 @@ class B200VecEnv:
         the fixed order 0, 1, ..., K-1, 0, ... whatever env_pool says; each batch steps on its own CUDA stream while the
         caller works on the batch it was handed.  recv() returns the batch's B = b * agents_per_env rows, with env_id
         the batch's global agent slots (the LSTM-state index of clean_pufferl.py:313-314); batch_env_range is its
-        (lo, hi).  send() takes the actions of those B rows."""
+        (lo, hi).  send() takes the actions of those B rows.
+
+        event_log_cap: 0 (default) leaves the event log off.  n > 0 switches it on: every send() also exports the
+        stepped batch's player events, as rows of the reference's event log, into a device buffer of n rows per batch,
+        and events() hands out the rows of the batch the last recv() returned (DESIGN.md 2.4)."""
+        if int(event_log_cap) < 0:
+            raise ValueError(f"event_log_cap must be >= 0 (0 = event log off), got {event_log_cap}")
         # env_creator / env_args / envs_per_worker are accepted for signature compatibility
         self.num_envs = int(num_envs)
         b = self.num_envs if envs_per_batch is None else int(envs_per_batch)
@@ -206,6 +216,13 @@ class B200VecEnv:
             self.sim.batch_streams = self._streams
         self._info_q = None              # in-flight async gather: (event, n, idx, rows, done)
         self._info_stream = None
+        self._recv_batch = 0
+        self._ev = None                  # event log on: per batch (rows int32 [event_log_cap, 9], count int32 [1])
+        if event_log_cap:
+            self.sim.set_event_log(True)
+            dev = self.sim.obs.device
+            self._ev = [(torch.empty((int(event_log_cap), 9), dtype=torch.int32, device=dev),
+                         torch.zeros(1, dtype=torch.int32, device=dev)) for _ in range(self.num_batches)]
 
     # ---- pufferlib pool contract -------------------------------------------------------
     def async_reset(self, seed: int = 0):
@@ -213,6 +230,7 @@ class B200VecEnv:
         # trajectories of one handle holding all the envs
         from .dist import global_seeds
         self.sim.reset(global_seeds(int(seed), self.env_base, self.num_envs))
+        self._export_all_events()
         self._info_q = None
         self._pending = True
         self._next_batch = 0
@@ -228,6 +246,7 @@ class B200VecEnv:
             task_ids = np.zeros((E, P), np.int32)
             task_ids[np.asarray(env_indices)] = np.asarray(new_tasks, np.int32).reshape(-1, 1)
         self.sim.reset(sd, task_ids=task_ids, env_mask=mask)
+        self._export_all_events()
         self._pending = True
 
     def save_envs(self, env_indices):
@@ -242,7 +261,26 @@ class B200VecEnv:
         observations, rewards, flags and masks appear in their batch's next recv(), and so do the infos of the tick
         they were saved at, which are handed out again."""
         self.sim.load_envs(env_indices, states)
+        self._export_all_events()
         self._pending = True
+
+    def events(self):
+        """(rows int32 CUDA [event_log_cap, 9], count int32 CUDA [1]): the player events of the step whose outputs the
+        last recv() returned, for that batch's envs (none for envs reset or loaded since), as Simulator.events lays them
+        out: rows [env, ent_id, tick, event, type, level, number, gold, target] by env, agent and order of occurrence,
+        count[0] the number of rows (only the first event_log_cap are kept).  Views of the batch's buffer, ready on the
+        caller's stream with no host sync, and rewritten by the batch's next send()."""
+        if self._ev is None:
+            raise RuntimeError("the event log is off: create the pool with event_log_cap > 0")
+        return self._ev[self._recv_batch]
+
+    def _export_all_events(self):
+        """After a reset or load: every batch's rows again describe the envs as they now stand (reset and loaded envs
+        have no events).  Runs on the current stream, which the sim call has made wait for every batch stream."""
+        if self._ev is not None:
+            b = self.envs_per_batch
+            for k, (rows, cnt) in enumerate(self._ev):
+                self.sim.events(k * b, (k + 1) * b, out=rows, count=cnt)
 
     def sim_env_base(self) -> int:
         return self.env_base
@@ -324,6 +362,7 @@ class B200VecEnv:
         P, b, k = self.agents_per_env, self.envs_per_batch, self._next_batch
         lo, hi = k * b, (k + 1) * b
         self.batch_env_range = (lo, hi)
+        self._recv_batch = k
         s0, s1 = lo * P, hi * P
         if self.num_batches > 1:
             # the caller's stream waits for the batch's last step; the host does not
@@ -355,6 +394,8 @@ class B200VecEnv:
         a = a.to(device=self.sim.obs.device, dtype=t.int32).reshape(self.envs_per_batch, self.agents_per_env, 12).contiguous()
         if self.num_batches == 1:
             self.sim.step(a)
+            if self._ev is not None:
+                self.sim.events(0, self.num_envs, out=self._ev[0][0], count=self._ev[0][1])
         else:
             k = self._next_batch
             lo, hi = self.batch_env_range
@@ -363,6 +404,8 @@ class B200VecEnv:
             st.wait_event(self._sent[k])
             with t.cuda.stream(st):
                 self.sim.step_envs(lo, hi, a)
+                if self._ev is not None:
+                    self.sim.events(lo, hi, out=self._ev[k][0], count=self._ev[k][1])
                 self._stepped[k].record(st)
             a.record_stream(st)      # the caching allocator must not hand `a` out again before the step has read it
             self._next_batch = (k + 1) % self.num_batches
