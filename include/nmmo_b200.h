@@ -120,8 +120,9 @@ void *nmmo_episode_done_ptr(nmmo_handle *h); /* uint8 [E]    infos[..]["episode_
 void *nmmo_task_id_ptr(nmmo_handle *h);      /* int32 [E*P]  task-table row of every agent slot (this episode) */
 void *nmmo_task_embed_ptr(nmmo_handle *h);   /* fp16  [n_tasks][task_dim]  the task embeddings (the Task block of a record) */
 int nmmo_obs_stride(nmmo_handle *h);
-/* Names of the kernel instantiations this handle launches per step (family and compile-time shape are chosen by
- * nmmo_create from the configuration), as a profiler lists them. */
+/* Names of the step and observation kernel instantiations the handle's next launch uses, as a profiler lists them.
+ * nmmo_create chooses the family, the envs per CTA and the compile-time shape from the configuration; the name is the
+ * generic instantiation while the phase profiler is on, or, for the step kernel, while draws are injected. */
 const char *nmmo_step_kernel_name(nmmo_handle *h);
 const char *nmmo_obs_kernel_name(nmmo_handle *h);
 int nmmo_num_envs(nmmo_handle *h);

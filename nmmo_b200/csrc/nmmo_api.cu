@@ -2,6 +2,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <string>
 #include <vector>
 #include <algorithm>
@@ -24,6 +25,165 @@ static int fail(int code, const std::string &msg) { g_err = msg; return code; }
     if (e_ != cudaSuccess) return fail(NM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); \
   } while (0)
 
+static size_t a16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// ---------------------------------------------------------------------------------------------- launch plan ----
+// One environment of step_body<V>: its dynamic shared memory and its HBM workspace, array by array in the order of the
+// carve there (carve / carve_ws, each array rounded to 16 bytes)
+struct NmStepBytes { size_t smem, ws; };
+template <class V>
+static NmStepBytes step_bytes(const NmParams &p) {
+  constexpr size_t kSlack = 128;
+  typedef typename V::tile_t tile_t;
+  const size_t P = p.P, N = p.N, R = p.R, S = p.S, CAP = p.CAP, NINV = p.cfg[NC_N_INV];
+  NmStepBytes b{0, 0};
+  auto carve = [&](size_t bytes) { b.smem += a16(bytes); };
+  auto carve_ws = [&](size_t bytes, bool in_ws = V::kGlobalTables || V::kScratchInWs) { (in_ws ? b.ws : b.smem) += a16(bytes); };
+  if (!V::kGlobalTables) { carve(EA_N * R * 2); if (!V::kItemsInPlace) carve(IS_N * CAP * 2); carve(S * S / 2); }      // ent, item, map
+  carve((S * S + 31) / 32 * 4);                                       // occ
+  carve((CAP + 31) / 32 * 4); carve((CAP + 31) / 32 * 4);             // used, fresh
+  carve_ws(P * NINV * 2, V::kScratchInWs);                            // inv
+  carve(P);                                                           // invn
+  carve_ws(A_N * P * 2);                                              // act
+  carve(N); carve(N * 2);                                             // npc_move, npc_att
+  carve_ws((size_t)V::kEvCap * 8, V::kItemsInPlace || V::kGlobalTables || V::kScratchInWs);      // ev
+  carve_ws(P * 4, V::kScratchInWs);                                   // duniq
+  if (!V::kScratchInWs) carve(P * 4);                                 // s_list
+  carve((size_t)V::kNpcHash * 2);                                     // npc_hash
+  carve_ws(P * 16); carve_ws(P * 8);                                  // task, acc
+  carve(std::max<size_t>(4096, R * 8) + (V::kScratchInWs ? 0 : 32 * V::kChunkIters * 4));      // s_scratch
+  carve(R * (sizeof(tile_t) + 2));                                    // s_mv
+  if (!V::kGlobalTables && !V::kScratchInWs) carve((size_t)V::kDeplCap * sizeof(tile_t));      // dlist
+  if (!V::kScratchInWs) carve((size_t)V::kTblSlots * 4);              // s_tbl
+  carve_ws(P, V::kScratchInWs);                                       // slow
+  if (!V::kScratchInWs) carve(P * 4);                                 // s_plist
+  carve(32 * 4); carve(16);                                           // sc, bar
+  b.smem += kSlack;
+  if (V::kGlobalTables) b.ws += kSlack;      // (the big family's workspace has the same slack, the small layouts' none)
+  return b;
+}
+
+// The dynamic shared memory of one obs_body<V> CTA, array by array in the order of the carve there
+template <class V>
+static size_t obs_bytes(const NmParams &p) {
+  constexpr size_t kSlack = V::kStage ? 64 : 128;
+  constexpr size_t NW = NM_OBS_THREADS / 32;
+  const int AP = V::kStage ? p.P : std::min(p.P, NM_BIG_OBS_AGENTS);
+  const size_t R = p.R, S = p.S, A = AP, R32 = (R + 31) & ~(size_t)31, ncx = (S + NM_OBS_CELL - 1) / NM_OBS_CELL;
+  size_t s = 0;
+  auto carve = [&](size_t bytes) { s += a16(bytes); };
+  if (V::kStage) {
+    carve(EA_N_OBS * (R + NM_OBS_ENT_SKEW) * 2); carve(R * 2);          // s_ent, s_status
+    carve(IS_N * (size_t)p.ICAP * 2); carve(S * S / 2);                 // s_item, s_map
+  }
+  carve((size_t)p.L.n_mkt * IA_N_OBS * 2); carve((size_t)p.L.n_mkt * 2);      // s_mkt, s_mkt_rows
+  carve(A * p.cfg[NC_N_INV] * 2); carve(A * 4); carve(128 * 4);               // s_inv, s_invn, s_scan
+  carve(NW * a16((size_t)p.L.n_ent * 2));                                     // s_vis_all
+  carve(NW * NM_OBS_BATCH * 33 * 4); carve(NW * NM_OBS_BATCH * 2); carve(NW * NM_OBS_BATCH * AC_N * 2);      // s_bb_all, s_ba_all, s_pick_all
+  if (V::kStage) carve(NW * NM_OBS_EROWS * 64);                               // s_ebuf_all
+  carve(R32 * 4);                                                             // s_pos
+  carve((ncx * ncx + 1) * 4); carve(R32 * 2); carve(NW * (R32 / 32) * 4);     // s_cend, s_crow, s_vbm_all
+  carve((3 * AC_N + 2) * 4); carve(A * 8); carve(A * 4); carve(A * 8);        // s_head, s_hash, s_meta, s_work
+  if (nm_obs_pre_ok(p.R, AP)) { carve(A * 33 * 2); carve(A * 3 * 4); }        // s_va, s_tg
+  carve(16);                                                                  // bar
+  return s + kSlack;
+}
+
+// Test hooks: environment variables that steer nmmo_create's choices, read when an NmHooks is constructed
+struct NmHooks {
+  static int num(const char *name, int unset) { const char *v = getenv(name); return v ? atoi(v) : unset; }
+  bool force_big = num("NMMO_B200_FORCE_BIG", 0) == 1;       // the big family on a small shape
+  int envs_per_cta = num("NMMO_B200_ENVS_PER_CTA", 4);       // 4: four per CTA, else three; >= 3: three; 1: one; else two if they fit
+  bool no_std_step = num("NMMO_B200_NO_STD_STEP", 0) == 1;   // the generic step kernel (big family: observation kernel too) ...
+  bool no_std_obs = num("NMMO_B200_NO_STD_OBS", 0) == 1;     // ... the generic small observation kernel, on a compile-time shape
+  bool no_depl_list = getenv("NMMO_B200_NO_DEPL_LIST") != nullptr;      // never trust the depleted-tile list
+  int ev_cap = num("NMMO_B200_EV_CAP", 0);                   // a smaller event ring, to provoke overflow
+  int icap = num("NMMO_B200_ICAP", 0);                       // a tiny staged item prefix: the observation kernel's HBM tail path
+  int h2d_split_min = num("NMMO_B200_H2D_SPLIT_MIN", 0);     // the smallest handle whose byte-packed actions arrive in two ranges
+};
+
+// A kernel instantiation and its name as a profiler lists it
+struct NmKernel { void (*fn)(NmParams); const char *name; };
+#define NM_KERNEL(k) NmKernel{k, #k}
+
+// How a handle launches its step and observation kernels (plan_launches)
+struct NmPlan {
+  int big;                       // family (NmParams.big)
+  int envs_per_cta, threads_per_env;
+  int half_smem;                 // step kernel, per environment: dynamic shared memory (NmParams.half_smem) ...
+  size_t ws_bytes;               // ... and HBM workspace (NmParams.ws_bytes; 0 = none)
+  size_t obs_smem;               // observation kernel: dynamic shared memory per CTA ...
+  int obs_parts;                 // ... and CTAs per environment
+  // lean: the *_std instantiation where the handle has its compile-time shape, else the generic one; full: the generic
+  // one, the only one with the phase profiler and (step kernels) the injected-draw lookup
+  NmKernel step_lean, step_full, obs_lean, obs_full;
+};
+
+// The handle's shape is the compile-time shape SH (StdShape, StdShape5): its table shape, the record layout and the
+// engine defaults the *_std kernels fold in (nm_cfg_std_value)
+template <class SH>
+static bool has_std_shape(const NmParams &p) {
+  constexpr nm_obs_layout sl = nm_std_layout();
+  for (int i = 0; i < NC_COUNT; i++)
+    if (nm_cfg_std_value(i) != NM_CFG_RUNTIME && p.cfg[i] != nm_cfg_std_value(i)) return false;
+  return memcmp(&p.L, &sl, sizeof(sl)) == 0 && p.P == SH::P && p.N == SH::N && p.R == SH::R && p.S == SH::S && p.CAP == SH::CAP &&
+         p.cfg[NC_N_INV] == SH::NINV;
+}
+
+// The family, the envs per CTA, the sizes and the kernels of a handle of shape `p` (cfg, L, P, N, R, S, CAP, ICAP) on a
+// device with `max_smem` bytes of opt-in shared memory per block.  False: an environment does not fit.  No CUDA calls.
+static bool plan_launches(const NmParams &p, int max_smem, const NmHooks &hk, NmPlan &pl) {
+  auto r128 = [](size_t x) { return (x + 127) & ~(size_t)127; };
+  // Two kernel families (csrc/nmmo_step.cu): environments of up to 256 players / 512 entities / 255^2 tiles run out of
+  // shared memory, 256 threads each; larger ones (BASELINE.json configs[4]: 1024 players, 2048 NPCs, 544^2 tiles) keep
+  // their tables in HBM / L2 and get 1024 threads
+  pl.big = (hk.force_big || p.P > NM_STEP_THREADS || p.R > 2 * NM_STEP_THREADS || p.S > 255) ? 1 : 0;
+  const NmStepBytes one = pl.big ? step_bytes<VBig>(p) : step_bytes<VSmall>(p);
+  pl.obs_smem = pl.big ? obs_bytes<OBig>(p) : obs_bytes<OSmall>(p);
+  if (one.smem > (size_t)max_smem || pl.obs_smem > (size_t)max_smem) return false;
+  NmStepBytes b = one;
+  bool step_std, obs_std;
+  if (pl.big) {
+    pl.envs_per_cta = 1; pl.threads_per_env = VBig::kThreads;
+    pl.step_full = NM_KERNEL(nmmo_step_big_kernel); pl.step_lean = NM_KERNEL(nmmo_step_big_std_kernel);
+    pl.obs_full = NM_KERNEL(nmmo_obs_big_kernel); pl.obs_lean = NM_KERNEL(nmmo_obs_big_std_kernel);
+    step_std = obs_std = has_std_shape<StdShape5>(p) && p.cfg[NC_VISION] == StdShape5::VIS && !hk.no_std_step;
+  } else {
+    // four environments per CTA (VSmall4) when they fit, else three (item table and event ring in place in HBM / L2),
+    // else two (they walk the code together), else one
+    const NmStepBytes four = step_bytes<VSmall4>(p), three = step_bytes<VSmall3>(p);
+    const int want = hk.envs_per_cta;
+    if (want == 4 && p.P <= VSmall4::kThreads && p.R <= 2 * VSmall4::kThreads && 4 * r128(four.smem) <= (size_t)max_smem) {
+      pl.envs_per_cta = 4; pl.threads_per_env = VSmall4::kThreads; b = four;
+      pl.step_full = NM_KERNEL(nmmo_step4_kernel); pl.step_lean = NM_KERNEL(nmmo_step4_std_kernel);
+    } else if (want >= 3 && 3 * r128(three.smem) <= (size_t)max_smem) {
+      pl.envs_per_cta = 3; pl.threads_per_env = VSmall3::kThreads; b = three;
+      pl.step_full = NM_KERNEL(nmmo_step3_kernel); pl.step_lean = NM_KERNEL(nmmo_step3_std_kernel);
+    } else {
+      pl.envs_per_cta = (want != 1 && 2 * r128(one.smem) <= (size_t)max_smem) ? 2 : 1; pl.threads_per_env = VSmall::kThreads;
+      pl.step_full = pl.step_lean = NM_KERNEL(nmmo_step_kernel);
+    }
+    pl.obs_full = NM_KERNEL(nmmo_obs_kernel); pl.obs_lean = NM_KERNEL(nmmo_obs_std_kernel);
+    const bool std_shape = has_std_shape<StdShape>(p);
+    step_std = std_shape && !hk.no_std_step;
+    obs_std = std_shape && p.ICAP == StdShape::ICAP && p.cfg[NC_VISION] == StdShape::VIS && !hk.no_std_obs;
+  }
+  if (!step_std) pl.step_lean = pl.step_full;
+  if (!obs_std) pl.obs_lean = pl.obs_full;
+  pl.half_smem = (int)r128(b.smem); pl.ws_bytes = b.ws;
+  pl.obs_parts = pl.big ? (p.P + NM_BIG_OBS_AGENTS - 1) / NM_BIG_OBS_AGENTS : 1;
+  return true;
+}
+
+// The opt-in limit is a property of the kernel, not of the handle: several handles of different shapes may be alive in
+// one process, so it only ever grows (per kernel and device)
+static int raise_smem_limit(const NmKernel &k, int device, size_t bytes) {
+  static std::map<std::pair<void (*)(NmParams), int>, size_t> limit;
+  size_t &cur = limit[{k.fn, device}];
+  if (bytes > cur) { CU(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes)); cur = bytes; }
+  return NM_OK;
+}
+
 struct nmmo_handle {
   NmParams prm;
   int device;
@@ -35,8 +195,7 @@ struct nmmo_handle {
   cudaStream_t h2d_stream = nullptr;
   cudaEvent_t ev_entry = nullptr, ev_h2d[2] = {nullptr, nullptr};
   int h2d_split_min = 1024;                   // handles with fewer environments copy in one piece
-  size_t step_smem, obs_smem;
-  bool obs_std = false, step_std = false, big_std = false;      // the handle has the reference's default shape: the *_std kernels (compile-time shape and layout)
+  NmPlan plan;                                // kernels and launch shapes (plan_launches)
   std::vector<void *> allocs;
   int32_t *d_actions;             // staging for the host-buffer path
   int16_t *d_actions16;           // ... and for its int16 variant
@@ -54,89 +213,6 @@ struct nmmo_handle {
   // disjoint entries); allocated with the staging
   int32_t *ev_off = nullptr;
 };
-
-static size_t a16(size_t x) { return (x + 15) & ~(size_t)15; }
-
-// big family: shared memory and per-env HBM workspace of nmmo_step_big_kernel (same carve order as step_body<VBig>)
-static size_t step_big_smem_bytes(const NmParams &p) {
-  size_t s = 0;
-  int NINV = p.cfg[NC_N_INV];
-  s += a16((size_t)((p.S * p.S + 31) / 32) * 4); s += 2 * a16((size_t)((p.CAP + 31) / 32) * 4);
-  s += a16((size_t)p.P * NINV * 2); s += a16(p.P);
-  s += a16(p.N); s += a16((size_t)p.N * 2); s += a16((size_t)p.P * 4) * 2;
-  s += a16((size_t)VBig::kNpcHash * 2);
-  s += a16(std::max<size_t>(4096, (size_t)p.R * 8) + 32 * VBig::kChunkIters * 4); s += a16((size_t)p.R * (sizeof(VBig::tile_t) + 2));
-  s += a16((size_t)VBig::kTblSlots * 4); s += a16(p.P); s += a16((size_t)p.P * 4); s += a16(32 * 4); s += 16;
-  return s + 128;
-}
-// observation kernels: cell index (per-cell list ends, rows grouped by cell) and the per-warp row bitmaps
-static size_t obs_cell_bytes(const NmParams &p, int NW) {
-  const int ncx = (p.S + NM_OBS_CELL - 1) / NM_OBS_CELL, R32 = (p.R + 31) & ~31;
-  return a16((size_t)(ncx * ncx + 1) * 4) + a16((size_t)R32 * 2) + a16((size_t)NW * (R32 / 32) * 4);
-}
-// observation kernels, per warp: visible-row list, batched-sampler mask words / agents / picks, Entity row buffer
-static size_t obs_warp_bytes(const NmParams &p, int NW) {
-  return a16((size_t)NW * a16((size_t)p.L.n_ent * 2)) + a16((size_t)NW * NM_OBS_BATCH * 33 * 4) + a16((size_t)NW * NM_OBS_BATCH * 2) +
-         a16((size_t)NW * NM_OBS_BATCH * AC_N * 2) + (p.big ? 0 : a16((size_t)NW * NM_OBS_EROWS * 64));
-}
-// observation kernels: per-agent lists and target bits of the pre-pass (where it can run; same condition as in obs_body)
-static size_t obs_pre_bytes(const NmParams &p, int AP, int NW) {
-  const int RW = ((p.R + 31) & ~31) / 32;
-  const bool pre_ok = RW <= 32 && (size_t)AP * RW * 4 <= (size_t)NW * NM_OBS_BATCH * 33 * 4;
-  return pre_ok ? a16((size_t)AP * 33 * 2) + a16((size_t)AP * 3 * 4) : 0;
-}
-static size_t step_big_ws_bytes(const NmParams &p) {
-  return a16((size_t)12 * p.P * 2) + a16((size_t)VBig::kEvCap * 8) + a16((size_t)p.P * 16) + a16((size_t)p.P * 8) + 128;
-}
-static size_t obs_big_smem_bytes(const NmParams &p) {
-  size_t s = 0;
-  int NINV = p.cfg[NC_N_INV];
-  int NW = NM_OBS_THREADS / 32, AP = std::min(p.P, NM_BIG_OBS_AGENTS);
-  s += a16((size_t)p.L.n_mkt * IA_N_OBS * 2); s += a16((size_t)p.L.n_mkt * 2);
-  s += a16((size_t)AP * NINV * 2); s += a16((size_t)AP * 4); s += a16(64 * 4);
-  s += obs_warp_bytes(p, NW); s += 16;
-  s += a16((3 * AC_N + 2) * 4); s += a16((size_t)AP * 4); s += a16((size_t)AP * 8) + obs_pre_bytes(p, AP, NW); s += a16((size_t)((p.R + 31) & ~31) * 4);
-  s += obs_cell_bytes(p, NW) + 64 * 4 + a16((size_t)AP * 8);
-  return s + 128;
-}
-
-static size_t step_smem_bytes(const NmParams &p, bool items_in_place = false) {
-  size_t s = 0;
-  int NINV = p.cfg[NC_N_INV];
-  s += a16((size_t)EA_N * p.R * 2); s += items_in_place ? 0 : a16((size_t)IS_N * p.CAP * 2); s += a16((size_t)p.S * p.S / 2);
-  s += a16((size_t)((p.S * p.S + 31) / 32) * 4); s += 2 * a16((size_t)((p.CAP + 31) / 32) * 4);
-  s += a16((size_t)p.P * NINV * 2); s += a16(p.P); s += a16((size_t)12 * p.P * 2);
-  s += a16(p.N); s += a16((size_t)p.N * 2); s += items_in_place ? 0 : a16(NM_EV_CAP * 8); s += a16((size_t)p.P * 4) * 2; s += a16(64); s += 16;
-  s += a16(1024); s += a16((size_t)p.P * 16); s += a16((size_t)p.P * 8); s += a16(std::max<size_t>(4096, (size_t)p.R * 8) + 128); s += a16((size_t)p.R * 4); s += a16(NM_DEPL_CAP * 2); s += 4096; s += a16(p.P); s += a16((size_t)p.P * 4) + 64;
-  return s + 128;
-}
-// four environments per CTA (VSmall4): shared memory of one environment, and its HBM workspace (the carve_ws arrays of
-// step_body<VSmall4>, incl. the event ring); the scratch also holds the Move position index, and the depleted-tile
-// list is used in place
-static size_t step4_smem_bytes(const NmParams &p) {
-  size_t s = 0;
-  s += a16((size_t)EA_N * p.R * 2); s += a16((size_t)p.S * p.S / 2);
-  s += a16((size_t)((p.S * p.S + 31) / 32) * 4); s += 2 * a16((size_t)((p.CAP + 31) / 32) * 4);
-  s += a16(p.P); s += a16(p.N); s += a16((size_t)p.N * 2); s += a16((size_t)VSmall4::kNpcHash * 2);
-  s += a16(std::max<size_t>(4096, (size_t)p.R * 8)); s += a16((size_t)p.R * 4); s += a16(32 * 4); s += 16;
-  return s + 128;
-}
-static size_t step4_ws_bytes(const NmParams &p) {
-  return a16((size_t)p.P * p.cfg[NC_N_INV] * 2) + a16((size_t)12 * p.P * 2) + a16((size_t)NM_EV_CAP * 8) + a16((size_t)p.P * 4) +
-         a16((size_t)p.P * 16) + a16((size_t)p.P * 8) + a16(p.P);
-}
-static size_t obs_smem_bytes(const NmParams &p) {
-  size_t s = 0;
-  int NINV = p.cfg[NC_N_INV];
-  int NW = NM_OBS_THREADS / 32;
-  s += a16((size_t)EA_N_OBS * (p.R + NM_OBS_ENT_SKEW) * 2); s += a16((size_t)p.R * 2); s += a16((size_t)IS_N * p.ICAP * 2); s += a16((size_t)p.S * p.S / 2);
-  s += a16((size_t)p.L.n_mkt * IA_N_OBS * 2); s += a16((size_t)p.L.n_mkt * 2);
-  s += a16((size_t)p.P * NINV * 2); s += a16((size_t)p.P * 4); s += a16(64 * 4);
-  s += obs_warp_bytes(p, NW); s += 16;
-  s += a16((3 * AC_N + 2) * 4); s += a16((size_t)p.P * 4); s += a16((size_t)p.P * 8) + obs_pre_bytes(p, p.P, NW); s += a16((size_t)((p.R + 31) & ~31) * 4);
-  s += obs_cell_bytes(p, NW) + 64 * 4 + a16((size_t)p.P * 8);
-  return s + 64;
-}
 
 template <typename T>
 static int dalloc(nmmo_handle *h, T **ptr, size_t count, bool zero = true) {
@@ -211,6 +287,7 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   if (!cfg || !fcfg || !maps || !tasks || !task_embed || !out) return fail(NM_ERR_ARG, "null argument");
   if (n_cfg != NC_COUNT || n_fcfg != NF_COUNT) return fail(NM_ERR_ARG, "config vector length does not match nmmo_spec.h");
   if (n_envs <= 0 || n_maps <= 0 || n_tasks <= 0) return fail(NM_ERR_ARG, "n_envs, n_maps, n_tasks must be positive");
+  const NmHooks hk{};
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(NM_ERR_CUDA, "no CUDA device: nmmo_b200 has no CPU fallback");
@@ -230,15 +307,7 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   p.E = n_envs; p.P = cfg[NC_N_PLAYERS]; p.N = cfg[NC_N_NPCS]; p.R = p.P + p.N; p.S = cfg[NC_MAP_SIZE]; p.CAP = cfg[NC_ITEM_CAP];
   p.n_maps = n_maps; p.n_tasks = n_tasks; p.env_base = env_base;
   p.ICAP = std::min(p.CAP, 256);      // item rows the observation kernel keeps in shared memory; rows beyond are read in HBM
-  if (const char *ov = getenv("NMMO_B200_ICAP")) {      // test hook: force the HBM tail path with a tiny staged prefix
-    int v = atoi(ov);
-    if (v >= 8 && v % 8 == 0) p.ICAP = std::min(p.CAP, v);
-  }
-  // Two kernel families (csrc/nmmo_step.cu): environments of up to 256 players / 512 entities / 255^2 tiles run out of
-  // shared memory, 256 threads each; larger ones (BASELINE.json configs[4]: 1024 players, 2048 NPCs, 544^2 tiles) keep
-  // their tables in HBM / L2 and get 1024 threads
-  p.big = (p.P > NM_STEP_THREADS || p.R > 2 * NM_STEP_THREADS || p.S > 255) ? 1 : 0;
-  if (const char *ov = getenv("NMMO_B200_FORCE_BIG")) { if (atoi(ov) == 1) p.big = 1; }      // test hook: big family on a small env
+  if (hk.icap >= 8 && hk.icap % 8 == 0) p.ICAP = std::min(p.CAP, hk.icap);
   if (p.P <= 0 || p.P > NM_BIG_THREADS) { return fail(NM_ERR_LIMIT, "PLAYER_N must be in 1..1024"); }
   if (p.R % 8 || p.CAP % 8 || (p.S * p.S) % 32) { return fail(NM_ERR_LIMIT, "P+N and item cap must be multiples of 8, S*S of 32 (bulk copies)"); }
   if (p.R > VBig::kRowsPerThread * NM_BIG_THREADS) { return fail(NM_ERR_LIMIT, "P+N must be <= 3072"); }
@@ -251,78 +320,20 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
     return fail(NM_ERR_ARG, "SPAWN_PATCH^2 must hold PLAYER_N players and fit inside the map centre");
   if (p.cfg[NC_SPAWN_PATCH] == 0 && !p.cfg[NC_ALLOW_OCCUPIED] && p.P > 4 * p.cfg[NC_MAP_CENTER])
     return fail(NM_ERR_ARG, "border-ring spawn with one entity per tile needs PLAYER_N <= 4 * MAP_CENTER");
-  h->step_smem = p.big ? step_big_smem_bytes(p) : step_smem_bytes(p);
-  h->obs_smem = p.big ? obs_big_smem_bytes(p) : obs_smem_bytes(p);
   int max_smem = 0;
   CU(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
-  if ((int)h->step_smem > max_smem || (int)h->obs_smem > max_smem) { return fail(NM_ERR_LIMIT, "environment does not fit in shared memory"); }
-  // the small step kernel runs two environments per CTA (they walk the code together) when both fit
-  p.half_smem = (int)((h->step_smem + 127) & ~(size_t)127);
-  p.envs_per_cta = (!p.big && 2 * p.half_smem <= max_smem) ? 2 : 1;
-  // four environments per CTA (VSmall4) when they fit, else three (item table and event ring in place in HBM / L2)
-  int want = 4;
-  if (const char *ov = getenv("NMMO_B200_ENVS_PER_CTA")) want = atoi(ov);      // test hook: 1 / 2 / 3 / 4
-  const size_t s4 = (step4_smem_bytes(p) + 127) & ~(size_t)127, s3 = (step_smem_bytes(p, true) + 127) & ~(size_t)127;
-  if (!p.big && want == 4 && p.P <= VSmall4::kThreads && p.R <= 2 * VSmall4::kThreads && 4 * s4 <= (size_t)max_smem) {
-    p.envs_per_cta = 4; p.half_smem = (int)s4; h->step_smem = s4;
-  } else if (!p.big && want >= 3 && 3 * s3 <= (size_t)max_smem) {
-    p.envs_per_cta = 3; p.half_smem = (int)s3; h->step_smem = s3;
-  }
-  if (getenv("NMMO_B200_NO_DEPL_LIST")) p.no_depl_list = 1;      // test hook
+  NmPlan &pl = h->plan;
+  if (!plan_launches(p, max_smem, hk, pl)) { return fail(NM_ERR_LIMIT, "environment does not fit in shared memory"); }
+  p.big = pl.big; p.envs_per_cta = pl.envs_per_cta; p.half_smem = pl.half_smem; p.ws_bytes = pl.ws_bytes;
+  for (const NmKernel *k : {&pl.step_lean, &pl.step_full}) { int rc = raise_smem_limit(*k, device, (size_t)pl.envs_per_cta * pl.half_smem); if (rc) return rc; }
+  for (const NmKernel *k : {&pl.obs_lean, &pl.obs_full}) { int rc = raise_smem_limit(*k, device, pl.obs_smem); if (rc) return rc; }
+  p.no_depl_list = hk.no_depl_list;
   p.ev_cap = p.big ? VBig::kEvCap : VSmall::kEvCap;
-  if (const char *ov = getenv("NMMO_B200_EV_CAP")) { int v = atoi(ov); if (v > 0 && v < p.ev_cap) p.ev_cap = v; }      // test hook: provoke overflow
-  if (const char *ov = getenv("NMMO_B200_ENVS_PER_CTA")) {      // test hook
-    if (!p.big && atoi(ov) == 1) { p.envs_per_cta = 1; p.half_smem = (int)((step_smem_bytes(p) + 127) & ~(size_t)127); h->step_smem = p.half_smem; }
-  }
-  {   // the opt-in limit is a property of the kernel, not of the handle: several handles of different shapes may
-      // be alive in one process, so it only ever grows (per device)
-    static int step_attr[4][64] = {{0}}, obs_attr[2][64] = {{0}};
-    const int need_step = p.envs_per_cta * p.half_smem, need_obs = (int)h->obs_smem, d = device & 63, b = p.big;
-    const int sk = b ? 1 : (p.envs_per_cta == 3 ? 2 : p.envs_per_cta == 4 ? 3 : 0);
-    if (need_step > step_attr[sk][d]) {
-      if (sk == 1) CU(cudaFuncSetAttribute(nmmo_step_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
-      else if (sk == 2) CU(cudaFuncSetAttribute(nmmo_step3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
-      else if (sk == 3) CU(cudaFuncSetAttribute(nmmo_step4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
-      else CU(cudaFuncSetAttribute(nmmo_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
-      step_attr[sk][d] = need_step;
-    }
-    if (need_obs > obs_attr[b][d]) {
-      if (b) CU(cudaFuncSetAttribute(nmmo_obs_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_obs));
-      else {
-        CU(cudaFuncSetAttribute(nmmo_obs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_obs));
-        CU(cudaFuncSetAttribute(nmmo_obs_std_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_obs));
-      }
-      obs_attr[b][d] = need_obs;
-    }
-    {
-      constexpr nm_obs_layout sl = nm_std_layout();
-      bool std_cfg = true;      // the engine defaults the *_std kernels fold in (nm_cfg_std_value)
-      for (int i = 0; i < NC_COUNT; i++)
-        if (nm_cfg_std_value(i) != NM_CFG_RUNTIME && p.cfg[i] != nm_cfg_std_value(i)) std_cfg = false;
-      const bool std_shape = std_cfg && !b && memcmp(&p.L, &sl, sizeof(sl)) == 0 && p.P == StdShape::P && p.N == StdShape::N && p.R == StdShape::R &&
-                             p.S == StdShape::S && p.CAP == StdShape::CAP && p.cfg[NC_N_INV] == StdShape::NINV;
-      h->obs_std = std_shape && p.ICAP == StdShape::ICAP && p.cfg[NC_VISION] == StdShape::VIS;
-      h->step_std = std_shape && p.envs_per_cta >= 3;
-      if (const char *ov = getenv("NMMO_B200_NO_STD_OBS")) { if (atoi(ov) == 1) h->obs_std = false; }      // test hooks: the generic kernels on the default shape
-      if (const char *ov = getenv("NMMO_B200_NO_STD_STEP")) { if (atoi(ov) == 1) h->step_std = false; }
-      if (h->step_std) CU(cudaFuncSetAttribute(p.envs_per_cta == 4 ? nmmo_step4_std_kernel : nmmo_step3_std_kernel,
-                                               cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
-      // big family: the configs[4] shape
-      h->big_std = std_cfg && b && memcmp(&p.L, &sl, sizeof(sl)) == 0 && p.P == StdShape5::P && p.N == StdShape5::N && p.R == StdShape5::R &&
-                   p.S == StdShape5::S && p.CAP == StdShape5::CAP && p.cfg[NC_N_INV] == StdShape5::NINV && p.cfg[NC_VISION] == StdShape5::VIS;
-      if (const char *ov = getenv("NMMO_B200_NO_STD_STEP")) { if (atoi(ov) == 1) h->big_std = false; }
-      if (h->big_std) {
-        CU(cudaFuncSetAttribute(nmmo_step_big_std_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_step));
-        CU(cudaFuncSetAttribute(nmmo_obs_big_std_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, need_obs));
-      }
-    }
-  }
+  if (hk.ev_cap > 0 && hk.ev_cap < p.ev_cap) p.ev_cap = hk.ev_cap;
   size_t E = p.E, P = p.P;
   const size_t ent_i16 = p.big ? (size_t)NM_BIG_ENT_STRIDE * p.R : (size_t)EA_N * p.R;      // int16 per env
   DA(p.ent, E * ent_i16); DA(p.item, E * IS_N * p.CAP); DA(p.map, E * p.S * p.S / 2);
-  if (p.big) { p.ws_bytes = step_big_ws_bytes(p); DA(p.ws, E * p.ws_bytes); }
-  else if (p.envs_per_cta == 4) { p.ws_bytes = step4_ws_bytes(p); DA(p.ws, E * p.ws_bytes); }
-  else if (p.envs_per_cta == 3) { p.ws_bytes = a16((size_t)NM_EV_CAP * 8); DA(p.ws, E * p.ws_bytes); }
+  if (p.ws_bytes) DA(p.ws, E * p.ws_bytes);
   uint8_t *dmaps; DA(dmaps, (size_t)n_maps * p.S * p.S); p.maps = dmaps;
   CU(cudaMemcpy(dmaps, maps, (size_t)n_maps * p.S * p.S, cudaMemcpyHostToDevice));
   DA(p.scalars, E * NM_SC_N); DA(p.seed, E); DA(p.danger, E * p.N);
@@ -347,7 +358,7 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   std::vector<int32_t> sc(E * NM_SC_N, 0);
   for (size_t e = 0; e < E; e++) sc[e * NM_SC_N + SC_DONE] = 1;
   CU(cudaMemcpy(p.scalars, sc.data(), sizeof(int32_t) * sc.size(), cudaMemcpyHostToDevice));
-  if (const char *ov = getenv("NMMO_B200_H2D_SPLIT_MIN")) { int v = atoi(ov); if (v >= 1) h->h2d_split_min = v; }      // test hook
+  if (hk.h2d_split_min >= 1) h->h2d_split_min = hk.h2d_split_min;
   {
     uint64_t d = 0x6E6D6D6F53544154ULL;
     d = digest_bytes(d, cfg, sizeof(int32_t) * NC_COUNT);
@@ -377,33 +388,28 @@ extern "C" int nmmo_destroy(nmmo_handle *h) {
   return NM_OK;
 }
 
+// The plan entry a launch with `prm` uses: the *_std instantiations have no phase profiler and (step kernels) no
+// injected-draw lookup
+static bool lean(const NmParams &prm, bool step) { return !prm.prof && !(step && prm.inj_off); }
+static const NmKernel &step_kernel(const nmmo_handle *h, const NmParams &prm) { return lean(prm, true) ? h->plan.step_lean : h->plan.step_full; }
+static const NmKernel &obs_kernel(const nmmo_handle *h, const NmParams &prm) { return lean(prm, false) ? h->plan.obs_lean : h->plan.obs_full; }
+
 // step kernel over env range [lo, hi) on `st`
 static int launch_step_kernel(nmmo_handle *h, NmParams &prm, cudaStream_t st, int lo, int hi) {
-  const int epc = h->prm.envs_per_cta, n = hi - lo;
+  const NmPlan &pl = h->plan;
   prm.env_lo = lo; prm.env_hi = hi;
-  // the *_std instantiations have no profile counters and no injected-draw lookup
-  const bool lean_ok = !prm.prof && !prm.inj_off;
-  if (prm.big && h->big_std && lean_ok) nmmo_step_big_std_kernel<<<n, NM_BIG_THREADS, (size_t)prm.half_smem, st>>>(prm);
-  else if (prm.big) nmmo_step_big_kernel<<<n, NM_BIG_THREADS, (size_t)prm.half_smem, st>>>(prm);
-  else if (epc == 4 && h->step_std && lean_ok) nmmo_step4_std_kernel<<<(n + 3) / 4, 4 * NM_STEP4_THREADS, (size_t)4 * prm.half_smem, st>>>(prm);
-  else if (epc == 4) nmmo_step4_kernel<<<(n + 3) / 4, 4 * NM_STEP4_THREADS, (size_t)4 * prm.half_smem, st>>>(prm);
-  else if (epc == 3 && h->step_std && lean_ok) nmmo_step3_std_kernel<<<(n + 2) / 3, 3 * NM_STEP_THREADS, (size_t)3 * prm.half_smem, st>>>(prm);
-  else if (epc == 3) nmmo_step3_kernel<<<(n + 2) / 3, 3 * NM_STEP_THREADS, (size_t)3 * prm.half_smem, st>>>(prm);
-  else nmmo_step_kernel<<<(n + epc - 1) / epc, epc * NM_STEP_THREADS, (size_t)epc * prm.half_smem, st>>>(prm);
+  const auto fn = step_kernel(h, prm).fn;
+  fn<<<(hi - lo + pl.envs_per_cta - 1) / pl.envs_per_cta, pl.envs_per_cta * pl.threads_per_env, (size_t)pl.envs_per_cta * pl.half_smem, st>>>(prm);
   CU(cudaGetLastError());
   return NM_OK;
 }
 
 // observation kernel over env range [lo, hi) on `st`
 static int launch_obs_kernel(nmmo_handle *h, NmParams &prm, cudaStream_t st, int lo, int hi) {
-  const int n = hi - lo;
+  const NmPlan &pl = h->plan;
   prm.env_lo = lo; prm.env_hi = hi;
-  if (prm.big) {
-    const int ap = std::min(prm.P, NM_BIG_OBS_AGENTS), parts = (prm.P + ap - 1) / ap;
-    if (h->big_std && !prm.prof) nmmo_obs_big_std_kernel<<<n * parts, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
-    else nmmo_obs_big_kernel<<<n * parts, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
-  } else if (h->obs_std && !prm.prof) nmmo_obs_std_kernel<<<n, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
-  else nmmo_obs_kernel<<<n, NM_OBS_THREADS, h->obs_smem, st>>>(prm);
+  const auto fn = obs_kernel(h, prm).fn;
+  fn<<<(hi - lo) * pl.obs_parts, NM_OBS_THREADS, pl.obs_smem, st>>>(prm);
   CU(cudaGetLastError());
   return NM_OK;
 }
@@ -680,18 +686,8 @@ extern "C" void *nmmo_info_valid_ptr(nmmo_handle *h) { return h->prm.info_valid;
 extern "C" void *nmmo_episode_done_ptr(nmmo_handle *h) { return h->prm.episode_done; }
 extern "C" void *nmmo_task_id_ptr(nmmo_handle *h) { return h->prm.task_id; }
 extern "C" void *nmmo_task_embed_ptr(nmmo_handle *h) { return (void *)h->prm.embed; }
-// which instantiation this handle launches (bench / profiling: kernel names as ncu lists them)
-extern "C" const char *nmmo_step_kernel_name(nmmo_handle *h) {
-  const bool lean_ok = !h->prm.prof && !h->prm.inj_off;      // same rule as launch_step
-  if (h->prm.big) return (h->big_std && lean_ok) ? "nmmo_step_big_std_kernel" : "nmmo_step_big_kernel";
-  if (h->prm.envs_per_cta == 4) return (h->step_std && lean_ok) ? "nmmo_step4_std_kernel" : "nmmo_step4_kernel";
-  if (h->prm.envs_per_cta == 3) return (h->step_std && lean_ok) ? "nmmo_step3_std_kernel" : "nmmo_step3_kernel";
-  return "nmmo_step_kernel";
-}
-extern "C" const char *nmmo_obs_kernel_name(nmmo_handle *h) {
-  if (h->prm.big) return (h->big_std && !h->prm.prof) ? "nmmo_obs_big_std_kernel" : "nmmo_obs_big_kernel";
-  return (h->obs_std && !h->prm.prof) ? "nmmo_obs_std_kernel" : "nmmo_obs_kernel";
-}
+extern "C" const char *nmmo_step_kernel_name(nmmo_handle *h) { return step_kernel(h, h->prm).name; }
+extern "C" const char *nmmo_obs_kernel_name(nmmo_handle *h) { return obs_kernel(h, h->prm).name; }
 extern "C" int nmmo_obs_stride(nmmo_handle *h) { return h->prm.L.stride; }
 extern "C" int nmmo_num_envs(nmmo_handle *h) { return h->prm.E; }
 extern "C" int nmmo_num_agents(nmmo_handle *h) { return h->prm.P; }

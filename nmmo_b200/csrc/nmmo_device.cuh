@@ -239,6 +239,14 @@ struct NmCfg {
   }
 };
 
+// Observation kernel: whether the per-agent pre-pass runs for R table rows and AP agents per CTA -- at most 32 row-bitmap
+// words per agent, and room for the AP agents' bitmaps in the built-in policy's batch words.  obs_body carves its
+// per-agent lists where it does, and nmmo_create sizes the kernel's shared memory by it.
+__host__ __device__ __forceinline__ bool nm_obs_pre_ok(int R, int AP) {
+  const int RW = ((R + 31) & ~31) >> 5;
+  return RW <= 32 && (size_t)AP * RW * 4 <= (size_t)(NM_OBS_THREADS >> 5) * NM_OBS_BATCH * 33 * 4;
+}
+
 // ------------------------------------------------------------------------- rng ------
 __host__ __device__ __forceinline__ uint64_t nm_mix64(uint64_t z) {
   z += 0x9E3779B97F4A7C15ULL;

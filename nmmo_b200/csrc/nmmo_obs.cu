@@ -157,8 +157,8 @@ __device__ __forceinline__ void obs_body(const NmParams &prm) {
   uint64_t *s_work = (uint64_t *)carve((size_t)AP * 8);
   // per agent (pre-pass, a quad of threads per agent): up to 32 visible rows in table order (+ their count in slot 32;
   // row stride 33 halfwords so that the quads of a warp hit different banks) and the Attack / Give target bits of those rows
-  // (only where the pre-pass can run: at most 32 bitmap words per agent, and room for the bitmaps in the batch words)
-  const bool pre_ok = RW <= 32 && (size_t)AP * RW * 4 <= (size_t)NW * NM_OBS_BATCH * 33 * 4;
+  // (only where the pre-pass can run)
+  const bool pre_ok = nm_obs_pre_ok(R, AP);
   uint16_t *s_va = pre_ok ? (uint16_t *)carve((size_t)AP * 33 * 2) : nullptr;
   uint32_t *s_tg = pre_ok ? (uint32_t *)carve((size_t)AP * 3 * 4) : nullptr;
   uint64_t *bar = (uint64_t *)carve(16);
