@@ -98,6 +98,11 @@ enum nm_cfg {
                             environment.py:48); teams are consecutive id ranges, the first member is the leader */
   NC_SAMPLE_MOVE_PCT,    /* built-in action sampler only: percent probability that the Move head picks a valid
                             direction other than Stay (0 = uniform over the valid entries, config 2) */
+  /* death fog (nmmo/entity/player.py Player.update) [UPSTREAM] */
+  NC_DEATH_FOG,          /* PLAYER_DEATH_FOG: first tick of the fog, -1 = None (off)  config.yaml:75-86 death_fog_tick,
+                            environment.py:36-39 */
+  NC_DEATH_FOG_SPEED,    /* PLAYER_DEATH_FOG_SPEED 1: damage added per tick of fog */
+  NC_DEATH_FOG_FINAL_SIZE,  /* PLAYER_DEATH_FOG_FINAL_SIZE 8: Chebyshev radius around the map centre the fog never enters */
   NC_COUNT
 };
 

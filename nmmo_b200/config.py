@@ -87,6 +87,16 @@ def default_wrapper_args(agent: str = "takeru", **over) -> Namespace:
     return Namespace(**d)
 
 
+def death_fog_onset(tick) -> int:
+    """``env.death_fog_tick`` (environment.py:36-39 -> PLAYER_DEATH_FOG) as NC_DEATH_FOG: None -> -1 (no fog), an int
+    >= 0 -> the first tick of the fog.  Anything else is refused here, before a handle is created."""
+    if tick is None:
+        return -1
+    if isinstance(tick, (bool, np.bool_)) or not isinstance(tick, (int, np.integer)) or tick < 0 or tick > 2**31 - 1:
+        raise ValueError(f"death_fog_tick must be None or an int >= 0, got {tick!r}")
+    return int(tick)
+
+
 def make_config(env_args: Namespace = None, wrapper_args: Namespace = None, agent: str = "takeru",
                 **engine_over) -> Tuple[np.ndarray, np.ndarray]:
     """Build (cfg int32, fcfg float64).  ``engine_over`` overrides raw NC_* entries (tests)."""
@@ -152,6 +162,9 @@ def make_config(env_args: Namespace = None, wrapper_args: Namespace = None, agen
     c[S["NC_BASE_GOLD"]] = 1
     c[S["NC_LISTING_DURATION"]] = 3
     c[S["NC_ALLOW_OCCUPIED"]] = 0
+    c[S["NC_DEATH_FOG"]] = death_fog_onset(getattr(env_args, "death_fog_tick", None))
+    c[S["NC_DEATH_FOG_SPEED"]] = 1
+    c[S["NC_DEATH_FOG_FINAL_SIZE"]] = 8
     c[S["NC_WRAPPER"]] = WRAPPERS.get(agent, S["NW_BASE"])
     c[S["NC_EARLY_STOP_N"]] = int(getattr(wrapper_args, "early_stop_agent_num", 0))
     c[S["NC_EVAL_MODE"]] = int(bool(getattr(wrapper_args, "eval_mode", False)))

@@ -287,6 +287,8 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   if (!cfg || !fcfg || !maps || !tasks || !task_embed || !out) return fail(NM_ERR_ARG, "null argument");
   if (n_cfg != NC_COUNT || n_fcfg != NF_COUNT) return fail(NM_ERR_ARG, "config vector length does not match nmmo_spec.h");
   if (n_envs <= 0 || n_maps <= 0 || n_tasks <= 0) return fail(NM_ERR_ARG, "n_envs, n_maps, n_tasks must be positive");
+  if (cfg[NC_DEATH_FOG] < -1 || cfg[NC_DEATH_FOG_SPEED] < 0 || cfg[NC_DEATH_FOG_FINAL_SIZE] < 0)
+    return fail(NM_ERR_ARG, "DEATH_FOG must be -1 (off) or a tick >= 0; DEATH_FOG_SPEED and DEATH_FOG_FINAL_SIZE must be >= 0");
   const NmHooks hk{};
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)

@@ -60,7 +60,9 @@ enum nm_scalar { SC_TICK = 0, SC_DONE, SC_NEXT_NPC_ID, SC_N_DANGER, SC_MAP_ID, S
                  SC_N_DEPL /* entries of the depleted-tile list; -1 = unknown, rebuild it from a map scan */ };
 
 struct NmParams {
-  int32_t cfg[NC_COUNT];
+  // the config vector, rounded up to whole 16-byte words: the members after it keep their offsets modulo 16 whatever
+  // NC_COUNT is, and with them the kernels' merged parameter loads (e.g. two reward weights per 128-bit constant load)
+  int32_t cfg[(NC_COUNT + 3) & ~3];
   double fcfg[NF_COUNT];
   nm_obs_layout L;
   int E, P, N, R, S, CAP, n_maps, n_tasks;
@@ -221,6 +223,11 @@ __host__ __device__ constexpr int nm_cfg_std_value(int i) {
     case NC_ALLOW_OCCUPIED: return 0;      // one entity per tile (DESIGN.md section 7); the reference's Config never sets it
     case NC_BASE_GOLD: return 1;
     case NC_LISTING_DURATION: return 3;
+    // death fog: off (None) in every configuration the reference ships, so the *_std kernels compile it out; a handle with
+    // fog on fails has_std_shape and runs the generic instantiation of the same source
+    case NC_DEATH_FOG: return -1;
+    case NC_DEATH_FOG_SPEED: return 1;
+    case NC_DEATH_FOG_FINAL_SIZE: return 8;
     default: return NM_CFG_RUNTIME;      // shape entries (PLAYER_N, NPC_N, MAP_CENTER, MAP_SIZE, ITEM_CAP), HORIZON, RESILIENT_N,
                                          // SPAWN_IMMUNITY, the wrapper arguments and the workload knobs stay run-time
   }

@@ -1616,9 +1616,11 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
 
   PHASE();
   // ---- phase 2: players.update (order-free part), npcs.update -------------------------
+  // s_list[p]: 1 = p harvests in the id-ordered part below, 2 = the death fog killed p and its items are destroyed there
+  // (item rows are allocated lowest-free-first, so freeing them is ordered against the other players' drops)
   #pragma unroll 1
   for (int p = tid; p < P; p += T) {
-    bool seq = false;
+    bool seq = false, fog_items = false;
     if (ENT(EA_STATUS, p) == ES_ALIVE) {
       if (ENT(EA_DAMAGE, p) == 0) ENT(EA_ATTACKER_ID, p) = 0;
       int il = 0;
@@ -1628,36 +1630,53 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
       if (ENT(EA_FREEZE, p) > 0) ENT(EA_FREEZE, p) -= 1;
       ENT(EA_DAMAGE, p) = 0;
       ENT(EA_TIME_ALIVE, p) += 1;
-      int hp = ENT(EA_HEALTH, p), org = hp, food = ENT(EA_FOOD, p), water = ENT(EA_WATER, p);
-      if (food > c[NC_RES_REGEN_THRESH] && water > c[NC_RES_REGEN_THRESH]) hp = min(c[NC_RES_BASE], hp + c[NC_RES_HEALTH_RESTORE]);
-      int res = ENT(EA_RESILIENT, p);
-      if (food == 0) { int d = c[NC_RES_STARVATION]; if (res) d /= 2; hp = max(0, hp - d); }
-      if (water == 0) { int d = c[NC_RES_DEHYDRATION]; if (res) d /= 2; hp = max(0, hp - d); }
-      ENT(EA_HEALTH, p) = (int16_t)hp;
-      ENT(EA_HEALTH_RESTORE, p) = (int16_t)(hp - org);
-      int r = ENT(EA_ROW, p), cc = ENT(EA_COL, p);
-      water = max(0, water - c[NC_RES_DEPLETION]);
-      int up = tile_at(ctx, r - 1, cc), dn = tile_at(ctx, r + 1, cc), lf = tile_at(ctx, r, cc - 1), rt = tile_at(ctx, r, cc + 1);
-      if (up == MT_WATER || dn == MT_WATER || lf == MT_WATER || rt == MT_WATER) {
-        water = min(c[NC_RES_BASE], water + c[NC_RES_HARVEST_RESTORE]);
-        emit(ctx, p, EV_DRINK_WATER, 0, 0, 0, 0, 0);
+      // death fog (Player.update, DESIGN.md 7): off (-1) in every *_std instantiation, where this block compiles out
+      bool fog_dead = false;
+      if (c[NC_DEATH_FOG] >= 0 && ctx.tick >= c[NC_DEATH_FOG]) {
+        const int cent = c[NC_MAP_BORDER] + c[NC_MAP_CENTER] / 2;
+        const int dist = max(abs(ENT(EA_ROW, p) - cent), abs(ENT(EA_COL, p) - cent));
+        if (dist > c[NC_DEATH_FOG_FINAL_SIZE]) {
+          const int dmg = max(0, dist - c[NC_MAP_CENTER] / 2 + c[NC_DEATH_FOG_SPEED] * (ctx.tick - c[NC_DEATH_FOG] + 1));
+          ENT(EA_DMG_RECEIVED, p) = (int16_t)min(32767, ENT(EA_DMG_RECEIVED, p) + dmg);
+          ENT(EA_DAMAGE, p) = (int16_t)dmg;
+          const int left = max(0, ENT(EA_HEALTH, p) - dmg);
+          ENT(EA_HEALTH, p) = (int16_t)left;
+          fog_dead = left == 0;      // no Resources / Skills update this tick
+          fog_items = fog_dead && ctx.invn[p] > 0;
+        }
       }
-      ENT(EA_WATER, p) = (int16_t)water;
-      food = max(0, food - c[NC_RES_DEPLETION]);
-      int here = tile_at(ctx, r, cc);
-      if (here == MT_FOILAGE && !c[NC_ALLOW_OCCUPIED]) {
-        // with one entity per tile nobody else can eat this tile: no ordering needed
-        tile_dec(ctx, r * S + cc);
-        food = min(c[NC_RES_BASE], food + c[NC_RES_HARVEST_RESTORE]);
-        emit(ctx, p, EV_EAT_FOOD, 0, 0, 0, 0, 0);
-        here = MT_SCRUB;
+      if (!fog_dead) {
+        int hp = ENT(EA_HEALTH, p), org = hp, food = ENT(EA_FOOD, p), water = ENT(EA_WATER, p);
+        if (food > c[NC_RES_REGEN_THRESH] && water > c[NC_RES_REGEN_THRESH]) hp = min(c[NC_RES_BASE], hp + c[NC_RES_HEALTH_RESTORE]);
+        int res = ENT(EA_RESILIENT, p);
+        if (food == 0) { int d = c[NC_RES_STARVATION]; if (res) d /= 2; hp = max(0, hp - d); }
+        if (water == 0) { int d = c[NC_RES_DEHYDRATION]; if (res) d /= 2; hp = max(0, hp - d); }
+        ENT(EA_HEALTH, p) = (int16_t)hp;
+        ENT(EA_HEALTH_RESTORE, p) = (int16_t)(hp - org);
+        int r = ENT(EA_ROW, p), cc = ENT(EA_COL, p);
+        water = max(0, water - c[NC_RES_DEPLETION]);
+        int up = tile_at(ctx, r - 1, cc), dn = tile_at(ctx, r + 1, cc), lf = tile_at(ctx, r, cc - 1), rt = tile_at(ctx, r, cc + 1);
+        if (up == MT_WATER || dn == MT_WATER || lf == MT_WATER || rt == MT_WATER) {
+          water = min(c[NC_RES_BASE], water + c[NC_RES_HARVEST_RESTORE]);
+          emit(ctx, p, EV_DRINK_WATER, 0, 0, 0, 0, 0);
+        }
+        ENT(EA_WATER, p) = (int16_t)water;
+        food = max(0, food - c[NC_RES_DEPLETION]);
+        int here = tile_at(ctx, r, cc);
+        if (here == MT_FOILAGE && !c[NC_ALLOW_OCCUPIED]) {
+          // with one entity per tile nobody else can eat this tile: no ordering needed
+          tile_dec(ctx, r * S + cc);
+          food = min(c[NC_RES_BASE], food + c[NC_RES_HARVEST_RESTORE]);
+          emit(ctx, p, EV_EAT_FOOD, 0, 0, 0, 0, 0);
+          here = MT_SCRUB;
+        }
+        ENT(EA_FOOD, p) = (int16_t)food;
+        seq = here == MT_FOILAGE || here == MT_HERB || here == MT_ORE || here == MT_TREE || here == MT_CRYSTAL ||
+              up == MT_FISH || dn == MT_FISH || lf == MT_FISH || rt == MT_FISH;
       }
-      ENT(EA_FOOD, p) = (int16_t)food;
-      seq = here == MT_FOILAGE || here == MT_HERB || here == MT_ORE || here == MT_TREE || here == MT_CRYSTAL ||
-            up == MT_FISH || dn == MT_FISH || lf == MT_FISH || rt == MT_FISH;
     }
-    s_list[p] = seq ? 1 : 0;
-    if (seq) atomicOr(&ctx.sc[23], 32);
+    s_list[p] = seq ? 1 : (fog_items ? 2 : 0);
+    if (seq || fog_items) atomicOr(&ctx.sc[23], 32);
   }
   #pragma unroll 1
   for (int r = P + tid; r < R; r += T)
@@ -1671,7 +1690,7 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
   HSYNC();
   PHASE();
   const int todo = ctx.sc[23];      // env-uniform: bit per phase that has work (Use, Buy, Give, Destroy, Sell, harvest)
-  // id-ordered part: tile depletion and drops
+  // id-ordered part: tile depletion and drops, and the items of players the death fog killed
   if (todo & 32) {
   if (warp == 0) {
     #pragma unroll 1
@@ -1681,7 +1700,14 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
       #pragma unroll 1
       while (m) {
         int l = __ffs(m) - 1; m &= m - 1;
-        if (lane == l) player_harvest(ctx, p);
+        if (lane == l) {
+          if (c[NC_DEATH_FOG] >= 0 && s_list[p] == 2) {
+            #pragma unroll 1
+            while (ctx.invn[p] > 0) item_destroy(ctx, ctx.inv[p * NINV + ctx.invn[p] - 1]);
+          } else {
+            player_harvest(ctx, p);
+          }
+        }
         __syncwarp();
       }
     }
