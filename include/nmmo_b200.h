@@ -144,14 +144,15 @@ int nmmo_task_state(nmmo_handle *h, int env, int32_t *task_id, int32_t *complete
                     double *max_progress);
 
 /* Episode statistics of finished agents since the last clear: sums[IN_N], counts[IN_N] (means
- * are sums/counts, clean_pufferl.py:381-390), counters[4] = slot-steps, agent-steps (mask
- * sum), finished episodes, event-ring overflows, bytes moved by the observation kernel, 3 spare
- * (counters has 8 entries).  Plain sums so ranks can all-reduce them. */
+ * are sums/counts, clean_pufferl.py:381-390), counters[8] = slot-steps, agent-steps (mask
+ * sum), finished episodes, event-ring overflows, bytes moved by the observation kernel, rejected
+ * next-episode entries (nmmo_set_next_episodes), 2 spare.  Plain sums so ranks can all-reduce them. */
 int nmmo_stats(nmmo_handle *h, double *sums, double *counts, uint64_t *counters, int clear);
 
 /* Device-side error state (synchronises): NM_ERR_STATE when an environment produced more events in one tick than its
  * event ring holds (events were dropped: statistics and event-driven task progress of that env are wrong) since the
- * counters were last cleared.  nmmo_step is asynchronous and cannot report it; the host-buffer calls do. */
+ * counters were last cleared.  nmmo_step is asynchronous and cannot report it; the host-buffer calls do.  Also
+ * NM_ERR_STATE when an automatic reset rejected an out-of-range pending next-episode entry (nmmo_set_next_episodes). */
 int nmmo_check(nmmo_handle *h);
 
 /* Environment state (DESIGN.md 2.3): one fixed-size blob per env, `bytes` long (header included, a multiple of 128), that
@@ -193,6 +194,31 @@ int nmmo_set_event_log(nmmo_handle *h, int enable);
  * empty, reversed or out-of-bounds range, cap < 0, or a NULL or not 4-byte-aligned pointer (rows_dev may be NULL when
  * cap = 0). */
 int nmmo_events(nmmo_handle *h, int env_lo, int env_hi, int32_t *rows_dev, int cap, int32_t *count_dev, void *stream);
+
+/* Pending next-episode values (DESIGN.md 2.5): what an env's next AUTOMATIC reset takes instead of deriving it, so that
+ * a curriculum (in torch on the device, or on the host) steers every episode, not only the first.
+ * enable = 1 allocates the buffers below (E * (13 + 4 * P) bytes) with every flag 0 (also when already on); 0 frees them.
+ * Synchronises the device, so it is ordered after every range step in flight.  The accessors return NULL while off.
+ *   flags  uint8  [E]     bits nm_next (nmmo_spec.h): NM_NEXT_SEED 1 | NM_NEXT_MAP 2 | NM_NEXT_TASKS 4
+ *   seed   uint64 [E]     the next episode's env seed
+ *   map    int32  [E]     its map id
+ *   task   int32  [E][P]  its task-table rows, one per agent slot
+ * When: only at an env's automatic reset inside a step call (nmmo_step, nmmo_step_envs, the nmmo_step_host calls: the
+ * step after the one that ended its episode).  nmmo_reset and nmmo_load_envs neither use the values nor clear them.
+ * What: a field is taken only when its bit is set; otherwise it is derived as without this feature: the seed is
+ * nm_mix64(seed + 0x632BE59BD9B4E019) of the ending episode's seed, the map and the tasks are drawn from the new seed.
+ * Consumption: the reset sets the env's flags byte to 0 and leaves the value arrays as they are, so a curriculum finds
+ * the envs that need a new entry by flags == 0, on the device.  Teams (NC_TEAM_SIZE > 1): agent p takes the entry of its
+ * team leader, the row the task draw is keyed by, so a team's tasks are uniform.  Out of range: a map id outside
+ * [0, n_maps) or a team's task row outside [0, n_tasks) is never read through; that field (that team's task) is drawn as
+ * if unset, counters[5] of nmmo_stats counts it and nmmo_check returns NM_ERR_STATE.  The values belong to the slot: they
+ * are not part of a state blob.  Writes by the caller must be ordered before the step call that should see them and
+ * after the one that last cleared the flags (e.g. on the stream the env is stepped on). */
+int nmmo_set_next_episodes(nmmo_handle *h, int enable);
+void *nmmo_next_flags_ptr(nmmo_handle *h);
+void *nmmo_next_seed_ptr(nmmo_handle *h);
+void *nmmo_next_map_ptr(nmmo_handle *h);
+void *nmmo_next_task_ptr(nmmo_handle *h);
 
 /* Per-kernel device timing (CUDA events recorded on the launching stream around the step kernel
  * and the observation kernel): enable, run steps, read the mean milliseconds per launch. */

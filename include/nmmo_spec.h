@@ -273,6 +273,10 @@ enum nm_task_flag {
                                CanSeeAgent -> that team's leader, CanSeeGroup / AllDead -> that team (AllDead p1 = 1: its leader) */
 };
 
+/* Pending next-episode values (nmmo_set_next_episodes): bits of an env's flags byte, one per field its next automatic
+ * reset takes from the device buffers instead of deriving it */
+enum nm_next { NM_NEXT_SEED = 1, NM_NEXT_MAP = 2, NM_NEXT_TASKS = 4 };
+
 /* ------------------------------------------------------------------------ rng ------- */
 /* Draw sites.  A draw is addressed by (env seed, tick, site, idx, k) so that a parallel
  * device step and a sequential CPU step consume the same values in any order; recorded

@@ -386,6 +386,7 @@ extern "C" int nmmo_destroy(nmmo_handle *h) {
   if (h->h2d_stream) { cudaStreamDestroy(h->h2d_stream); cudaEventDestroy(h->ev_entry); cudaEventDestroy(h->ev_h2d[0]); cudaEventDestroy(h->ev_h2d[1]); }
   if (h->copy_stream) { cudaStreamDestroy(h->copy_stream); cudaEventDestroy(h->ev_step_done); cudaEventDestroy(h->ev_copy_done); cudaFreeHost(h->h_overflow); }
   if (h->prm.ev_log) { cudaFree(h->prm.ev_log); cudaFree(h->prm.ev_n); cudaFree(h->ev_off); }
+  if (h->prm.next_flags) { cudaFree(h->prm.next_flags); cudaFree(h->prm.next_seed); cudaFree(h->prm.next_map); cudaFree(h->prm.next_task); }
   delete h;
   return NM_OK;
 }
@@ -564,16 +565,20 @@ static int finish_step_host(nmmo_handle *h, float *rew_out, uint8_t *term_out, u
   return NM_OK;
 }
 
-// Device-side error state (synchronises): NM_ERR_STATE when any environment dropped events (its SC_ERROR bit is set)
-// since the counters were last cleared.  The asynchronous nmmo_step cannot report it; callers poll this at their
+// Device-side error state (synchronises): NM_ERR_STATE when any environment dropped events (its SC_ERROR bit is set), or an
+// automatic reset rejected an out-of-range pending next-episode entry, since the counters were last cleared.  The asynchronous nmmo_step cannot report it; callers poll this at their
 // logging cadence (B200VecEnv.stats does).
 extern "C" int nmmo_check(nmmo_handle *h) {
   if (!h) return fail(NM_ERR_ARG, "null handle");
   CU(cudaSetDevice(h->device));
   CU(cudaDeviceSynchronize());
-  unsigned long long n = 0;
-  CU(cudaMemcpy(&n, h->prm.counters + 3, sizeof(n), cudaMemcpyDeviceToHost));
-  if (n) return fail(NM_ERR_STATE, "event ring overflow in " + std::to_string(n) + " env-tick(s): more events in one tick than the ring holds");
+  unsigned long long n[3] = {0, 0, 0};
+  CU(cudaMemcpy(n, h->prm.counters + 3, sizeof(n), cudaMemcpyDeviceToHost));
+  if (n[0]) return fail(NM_ERR_STATE, "event ring overflow in " + std::to_string(n[0]) + " env-tick(s): more events in one tick than the ring holds");
+  if (n[2])
+    return fail(NM_ERR_STATE, std::to_string(n[2]) + " pending next-episode entr" + (n[2] == 1 ? "y was" : "ies were") +
+                              " out of range (a next_map id outside [0, " + std::to_string(h->prm.n_maps) + ") or a team's next_task row outside [0, " +
+                              std::to_string(h->prm.n_tasks) + ")): automatic resets drew those fields as if they were unset");
   return NM_OK;
 }
 
@@ -979,3 +984,39 @@ extern "C" int nmmo_events(nmmo_handle *h, int env_lo, int env_hi, int32_t *rows
   CU(cudaGetLastError());
   return NM_OK;
 }
+
+// ------------------------------------------------------------------------------------ next-episode values ----
+extern "C" int nmmo_set_next_episodes(nmmo_handle *h, int enable) {
+  if (!h) return fail(NM_ERR_ARG, "null handle");
+  CU(cudaSetDevice(h->device));
+  CU(cudaDeviceSynchronize());      // no step in flight may read or clear the flags while they change
+  NmParams &p = h->prm;
+  if (!enable) {
+    if (p.next_flags) { CU(cudaFree(p.next_flags)); CU(cudaFree(p.next_seed)); CU(cudaFree(p.next_map)); CU(cudaFree(p.next_task)); }
+    p.next_flags = nullptr; p.next_seed = nullptr; p.next_map = nullptr; p.next_task = nullptr;
+    return NM_OK;
+  }
+  const size_t E = p.E, P = p.P;
+  if (!p.next_flags) {
+    uint8_t *f = nullptr; uint64_t *sd = nullptr; int32_t *m = nullptr, *t = nullptr;
+    cudaError_t e = cudaMalloc((void **)&f, E);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&sd, E * sizeof(uint64_t));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&m, E * sizeof(int32_t));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&t, E * P * sizeof(int32_t));
+    if (e != cudaSuccess) {
+      cudaFree(f); cudaFree(sd); cudaFree(m); cudaFree(t);
+      return fail(NM_ERR_CUDA, std::string("next-episode buffers: ") + cudaGetErrorString(e));
+    }
+    p.next_flags = f; p.next_seed = sd; p.next_map = m; p.next_task = t;
+    CU(cudaMemset(p.next_seed, 0, E * sizeof(uint64_t)));
+    CU(cudaMemset(p.next_map, 0, E * sizeof(int32_t)));
+    CU(cudaMemset(p.next_task, 0, E * P * sizeof(int32_t)));
+  }
+  CU(cudaMemset(p.next_flags, 0, E));
+  CU(cudaDeviceSynchronize());
+  return NM_OK;
+}
+extern "C" void *nmmo_next_flags_ptr(nmmo_handle *h) { return h->prm.next_flags; }
+extern "C" void *nmmo_next_seed_ptr(nmmo_handle *h) { return h->prm.next_seed; }
+extern "C" void *nmmo_next_map_ptr(nmmo_handle *h) { return h->prm.next_map; }
+extern "C" void *nmmo_next_task_ptr(nmmo_handle *h) { return h->prm.next_task; }

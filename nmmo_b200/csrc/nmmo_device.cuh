@@ -108,6 +108,12 @@ struct NmParams {
   // emitted, and their count (0 for an env the call resets); nmmo_events turns them into rows (nmmo_events.cu)
   uint2 *ev_log;               // [E][ev_cap]
   int32_t *ev_n;               // [E]
+  // pending next-episode values (nmmo_set_next_episodes; NULL = off): an env's automatic reset takes the fields whose
+  // nm_next bit is set in its flags byte from here, then clears the byte
+  uint8_t *next_flags;         // [E]
+  uint64_t *next_seed;         // [E]
+  int32_t *next_map;           // [E]
+  int32_t *next_task;          // [E][P] task-table rows (agent p reads its team leader's entry)
 };
 
 // The reference's default shape (config 2: 128 players, 256 NPCs, 160^2 map, N_ent 100, N_mkt 384, 12 inventory rows,

@@ -1184,17 +1184,26 @@ __device__ void write_info(const Ctx<V> &ctx, int p, bool terminated, double cum
 #endif
 template <class V>
 __device__ NM_RESET_INLINE void reset_env(const NmParams &P_, int env, uint64_t seed, bool explicit_map, bool explicit_tasks,
-                          int *s_slot /* >= 2*P ints of shared memory */) {
+                          int *s_slot /* >= 2*P ints of shared memory */, bool automatic) {
   const int32_t *c = P_.cfg;
   int tid = threadIdx.x % V::kThreads, T = V::kThreads;
   const int half_id = threadIdx.x / V::kThreads;
   int P = P_.P, R = P_.R, S = P_.S;
   int32_t *sc = P_.scalars + (size_t)env * NM_SC_N;
+  // automatic reset: the env's pending next-episode values (nmmo_set_next_episodes).  Every thread reads the flags before
+  // the barrier below; thread 0 clears them after it.  A map id or task row out of range is drawn as if unset.
+  const int nf = automatic && P_.next_flags ? P_.next_flags[env] : 0;
+  if (nf & NM_NEXT_SEED) seed = P_.next_seed[env];
   // injected draws are keyed by tick 0 here
   Ctx<V> ctx;
   ctx.p = &P_; ctx.c = NmCfg<V::kStd>{c}; ctx.env = env; ctx.seed = seed; ctx.tick = 0;
   ctx.inj_lo = P_.inj_off ? P_.inj_off[env] : 0; ctx.inj_hi = P_.inj_off ? P_.inj_off[env + 1] : 0;
-  int map_id = explicit_map ? sc[SC_MAP_ID] : nm_bounded(draw(ctx, RS_MAP, 0, 0), P_.n_maps);
+  int map_id = (nf & NM_NEXT_MAP) ? P_.next_map[env] : -1;
+  if (explicit_map) map_id = sc[SC_MAP_ID];
+  else if ((unsigned)map_id >= (unsigned)P_.n_maps) {
+    if ((nf & NM_NEXT_MAP) && tid == 0) atomicAdd(&P_.counters[5], 1ULL);
+    map_id = nm_bounded(draw(ctx, RS_MAP, 0, 0), P_.n_maps);
+  }
   // map copy, table clears
   {
     // source maps are one byte per tile; the live map packs two tiles per byte
@@ -1261,8 +1270,16 @@ __device__ NM_RESET_INLINE void reset_env(const NmParams &P_, int env, uint64_t 
     GENT(EA_STATUS) = ES_ALIVE;
 #undef GENT
     size_t a = (size_t)env * P + p;
-    // one task per team: the draw is keyed by the team leader's row (team size 1: by the agent's own)
-    if (!explicit_tasks) P_.task_id[a] = nm_bounded(draw(ctx, RS_TASK, (uint32_t)(p - p % max(1, c[NC_TEAM_SIZE])), 0), P_.n_tasks);
+    // one task per team: the draw and the pending entry are the team leader's (team size 1: the agent's own)
+    if (!explicit_tasks) {
+      const int lead = p - p % max(1, c[NC_TEAM_SIZE]);
+      int t = (nf & NM_NEXT_TASKS) ? P_.next_task[(size_t)env * P + lead] : -1;
+      if ((unsigned)t >= (unsigned)P_.n_tasks) {
+        if ((nf & NM_NEXT_TASKS) && p == lead) atomicAdd(&P_.counters[5], 1ULL);
+        t = nm_bounded(draw(ctx, RS_TASK, (uint32_t)lead, 0), P_.n_tasks);
+      }
+      P_.task_id[a] = t;
+    }
     P_.rew[a] = 0.0f; P_.term[a] = 0; P_.trunc[a] = 0; P_.mask[a] = 1; P_.info_valid[a] = 0;
     P_.obs_meta[a] &= ~OM_TASK;        // new episode, new task embedding
   }
@@ -1272,6 +1289,7 @@ __device__ NM_RESET_INLINE void reset_env(const NmParams &P_, int env, uint64_t 
     sc[SC_FRESH] = 1; sc[SC_ITEM_HI] = 0; sc[SC_N_DEPL] = 0; sc[SC_NEED_RESET] = 0; sc[SC_EXPLICIT_MAP] = 0; sc[SC_EXPLICIT_TASKS] = 0;
     P_.episode_done[env] = 0;
     if (P_.ev_n) P_.ev_n[env] = 0;      // a reset env has no events in the event log
+    if (nf) P_.next_flags[env] = 0;     // consumed; the value arrays keep what they hold
   }
 }
 
@@ -1321,7 +1339,7 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
   // ---- reset paths -------------------------------------------------------------------
   if (prm.mode == 1) {
     if (!gsc[SC_NEED_RESET]) return;
-    reset_env<V>(prm, env, prm.seed[env], gsc[SC_EXPLICIT_MAP] != 0, gsc[SC_EXPLICIT_TASKS] != 0, (int *)smem);
+    reset_env<V>(prm, env, prm.seed[env], gsc[SC_EXPLICIT_MAP] != 0, gsc[SC_EXPLICIT_TASKS] != 0, (int *)smem, false);
     return;
   }
 
@@ -1466,7 +1484,7 @@ __device__ __forceinline__ void step_body(const NmParams &prm) {
     }
     HSYNC();
     if (tid == 0) { gsc[SC_EPISODE] += 1; atomicAdd(&prm.counters[2], 1ULL); }
-    reset_env<V>(prm, env, nm_mix64(ctx.seed + 0x632BE59BD9B4E019ULL), false, false, (int *)smem);
+    reset_env<V>(prm, env, nm_mix64(ctx.seed + 0x632BE59BD9B4E019ULL), false, false, (int *)smem, true);
     return;
   }
   // Decode the player actions against the observation record they were chosen on (the ids are read

@@ -21,7 +21,8 @@ EXPORTS = [
     "nmmo_obs_ptr", "nmmo_reward_ptr", "nmmo_terminated_ptr", "nmmo_truncated_ptr", "nmmo_mask_ptr",
     "nmmo_info_ptr", "nmmo_info_valid_ptr", "nmmo_episode_done_ptr", "nmmo_task_id_ptr", "nmmo_task_embed_ptr", "nmmo_obs_stride", "nmmo_num_envs",
     "nmmo_num_agents", "nmmo_step_kernel_name", "nmmo_obs_kernel_name", "nmmo_inject_rng", "nmmo_snapshot", "nmmo_task_state", "nmmo_stats", "nmmo_check", "nmmo_timing", "nmmo_timing_read", "nmmo_profile", "nmmo_set_obs_full", "nmmo_set_autosample",
-    "nmmo_state_bytes", "nmmo_save_envs", "nmmo_load_envs", "nmmo_set_event_log", "nmmo_events", "nmmo_last_error",
+    "nmmo_state_bytes", "nmmo_save_envs", "nmmo_load_envs", "nmmo_set_event_log", "nmmo_events", "nmmo_set_next_episodes",
+    "nmmo_next_flags_ptr", "nmmo_next_seed_ptr", "nmmo_next_map_ptr", "nmmo_next_task_ptr", "nmmo_last_error",
     "nmmo_rollout_create", "nmmo_rollout_create_compact", "nmmo_rollout_store_compact", "nmmo_rollout_expand", "nmmo_rollout_destroy", "nmmo_rollout_reset", "nmmo_rollout_store", "nmmo_rollout_store_range", "nmmo_rollout_ptr",
     "nmmo_rollout_gae", "nmmo_rollout_buffer", "nmmo_rollout_last_error",
 ]
@@ -107,6 +108,11 @@ def load(build_if_missing: bool = True):
     L.nmmo_set_event_log.argtypes = [vp, C.c_int]
     L.nmmo_events.restype = C.c_int
     L.nmmo_events.argtypes = [vp, C.c_int, C.c_int, vp, C.c_int, vp, vp]
+    L.nmmo_set_next_episodes.restype = C.c_int
+    L.nmmo_set_next_episodes.argtypes = [vp, C.c_int]
+    for n in ("nmmo_next_flags_ptr", "nmmo_next_seed_ptr", "nmmo_next_map_ptr", "nmmo_next_task_ptr"):
+        getattr(L, n).restype = vp
+        getattr(L, n).argtypes = [vp]
     L.nmmo_last_error.restype = C.c_char_p
     L.nmmo_rollout_create.restype = C.c_int
     L.nmmo_rollout_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
@@ -197,6 +203,8 @@ class Simulator:
         self.E = int(n_envs)
         self.P = int(cfg[SPEC["NC_N_PLAYERS"]]); self.N = int(cfg[SPEC["NC_N_NPCS"]])
         self.cap = int(cfg[SPEC["NC_ITEM_CAP"]]); self.S = S
+        self.n_maps, self.n_tasks = int(maps.shape[0]), int(task_table.shape[0])
+        self.next_flags = self.next_seed = self.next_map = self.next_task = None      # set_next_episodes
         h = C.c_void_p()
         rc = self.L.nmmo_create(_p(self.cfg), len(self.cfg), _p(self.fcfg), len(self.fcfg), self.E, self.device,
                                 int(env_base), _p(maps), maps.shape[0], _p(task_table), _p(task_embed),
@@ -319,6 +327,89 @@ class Simulator:
                                        C.c_void_p(count.data_ptr()), self._stream()))
         return out, count
 
+    def set_next_episodes(self, enable: bool = True):
+        """Pending next-episode values on (DESIGN.md 2.5; synchronises the device) or off.  While on, every automatic
+        reset of an env (the step after its episode ended) takes the fields whose bit is set in ``next_flags[env]`` from
+        these views, instead of deriving them, and sets the byte to 0:
+
+        - ``next_flags`` uint8 [E]: SPEC NM_NEXT_SEED | NM_NEXT_MAP | NM_NEXT_TASKS;
+        - ``next_seed`` int64 [E]: the env seed, as the bits of the uint64 the engine uses;
+        - ``next_map`` int32 [E]: the map id;
+        - ``next_task`` int32 [E, P]: task-table rows per agent slot (agent p takes its team leader's entry).
+
+        An unset field is what it would be without this feature.  Explicit resets (reset, load_envs) neither use nor clear
+        the values, and they are not part of a saved state.  Switching on again zeroes every flag."""
+        t = self.torch
+        self._check(self.L.nmmo_set_next_episodes(self.h, int(bool(enable))))
+        if not enable:
+            self.next_flags = self.next_seed = self.next_map = self.next_task = None
+            return
+        dev = t.device("cuda", self.device)
+
+        def view(fn, shape, typestr):
+            return t.as_tensor(_DevView(getattr(self.L, fn)(self.h), shape, typestr, self), device=dev)
+
+        with t.cuda.device(dev):
+            self.next_flags = view("nmmo_next_flags_ptr", (self.E,), "|u1")
+            self.next_seed = view("nmmo_next_seed_ptr", (self.E,), "<i8")
+            self.next_map = view("nmmo_next_map_ptr", (self.E,), "<i4")
+            self.next_task = view("nmmo_next_task_ptr", (self.E, self.P), "<i4")
+
+    def set_next(self, env_ids, seeds=None, maps=None, tasks=None):
+        """Write next-episode values of envs `env_ids` and OR the bits of the fields given into their flags, with torch
+        ops on the current stream (set_next_episodes must be on).  seeds [n] (uint64 or int64 bits), maps [n],
+        tasks [n] (one row for every agent of the env) or [n, P].  Host inputs (lists, numpy arrays, CPU tensors) are
+        checked first: a ValueError leaves the handle unchanged.  CUDA inputs are not checked and cost no host
+        synchronisation; env ids must then be in range, and an out-of-range map or task is drawn as if unset at the
+        reset (check() reports it)."""
+        t = self.torch
+        if self.next_flags is None:
+            raise RuntimeError("pending next-episode values are off: call set_next_episodes() first")
+        dev = self.next_flags.device
+
+        def host(x):      # a host input as a numpy array (None for a CUDA tensor or an absent input)
+            if x is None or (t.is_tensor(x) and x.is_cuda):
+                return None
+            return np.asarray(x.cpu() if t.is_tensor(x) else x)
+
+        h_ids, h_sd, h_mp, h_tk = host(env_ids), host(seeds), host(maps), host(tasks)
+        n = int(h_ids.size) if h_ids is not None else env_ids.numel()
+        if h_ids is not None and (h_ids.ndim > 1 or ((h_ids < 0) | (h_ids >= self.E)).any()):
+            raise ValueError(f"env ids must be a 1-d list of envs in [0, {self.E})")
+        if h_sd is not None and (h_sd.shape != (n,) or (h_sd.dtype.kind == "i" and (h_sd < 0).any())):
+            raise ValueError(f"seeds must be [{n}] values >= 0 (or uint64)")
+        if h_mp is not None and (h_mp.shape != (n,) or ((h_mp < 0) | (h_mp >= self.n_maps)).any()):
+            raise ValueError(f"maps must be [{n}] map ids in [0, {self.n_maps})")
+        if h_tk is not None and (h_tk.shape not in ((n,), (n, self.P)) or ((h_tk < 0) | (h_tk >= self.n_tasks)).any()):
+            raise ValueError(f"tasks must be [{n}] or [{n}, {self.P}] task rows in [0, {self.n_tasks})")
+
+        def dev_t(x, h, dtype):
+            if x is None:
+                return None
+            if h is None:
+                return x.view(t.int64) if x.dtype == t.uint64 else x.to(dtype)
+            h = np.ascontiguousarray(h)
+            h = h.view(np.int64) if h.dtype == np.uint64 else h.astype(np.int64 if dtype == t.int64 else np.int32)
+            return t.as_tensor(h, device=dev)
+
+        ids = dev_t(env_ids, h_ids, t.int64).reshape(n)
+        sd = dev_t(seeds, h_sd, t.int64)
+        mp = dev_t(maps, h_mp, t.int32)
+        tk = dev_t(tasks, h_tk, t.int32)
+        bits = 0
+        if sd is not None:
+            self.next_seed.index_copy_(0, ids, sd)
+            bits |= SPEC["NM_NEXT_SEED"]
+        if mp is not None:
+            self.next_map.index_copy_(0, ids, mp)
+            bits |= SPEC["NM_NEXT_MAP"]
+        if tk is not None:
+            tk = tk.reshape(n, 1).expand(n, self.P) if tk.dim() == 1 else tk.reshape(n, self.P)
+            self.next_task.index_copy_(0, ids, tk.contiguous())
+            bits |= SPEC["NM_NEXT_TASKS"]
+        if bits:
+            self.next_flags.index_copy_(0, ids, self.next_flags.index_select(0, ids) | bits)
+
     def step_host(self, actions: np.ndarray, want_obs: bool = False):
         """Host-buffer call: actions [E,P,12] in host memory (pinned = async copies) as int32, int16 (half the
         bytes over the host link) or uint8 packed by ``pack_actions_u8`` (a quarter)."""
@@ -381,7 +472,8 @@ class Simulator:
         return self.L.nmmo_step_kernel_name(self.h).decode(), self.L.nmmo_obs_kernel_name(self.h).decode()
 
     def check(self):
-        """Raises NmmoError if any environment dropped events (event ring overflow) since the last stats clear."""
+        """Raises NmmoError if any environment dropped events (event ring overflow), or an automatic reset rejected an
+        out-of-range next-episode entry, since the last stats clear."""
         self._check(self.L.nmmo_check(self.h))
 
     def timing(self, enable: bool):

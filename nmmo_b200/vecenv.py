@@ -127,6 +127,10 @@ class _BatchedSimulator(Simulator):
         self.join_batches()
         return super().set_event_log(*args, **kwargs)
 
+    def set_next_episodes(self, *args, **kwargs):
+        self.join_batches()
+        return super().set_next_episodes(*args, **kwargs)
+
 
 class B200VecEnv:
     def __init__(self, env_creator=None, env_args=None, env_kwargs: Optional[Dict] = None, num_envs: int = 1,
@@ -208,6 +212,7 @@ class B200VecEnv:
         self._info_cap = int(min(info_cap, b * self.agents_per_env))
         self._next_batch = 0
         self.batch_env_range = (0, self.num_envs)      # envs [lo, hi) of the batch the last recv() returned
+        self._idle = True                # no batch stepped since the last reset / load: every env takes next-episode values
         if self.num_batches > 1:
             dev = self.sim.obs.device
             self._streams = [torch.cuda.Stream(device=dev) for _ in range(self.num_batches)]
@@ -233,6 +238,7 @@ class B200VecEnv:
         self._export_all_events()
         self._info_q = None
         self._pending = True
+        self._idle = True
         self._next_batch = 0
 
     def reset_envs(self, env_indices, seeds, new_tasks=None):
@@ -248,6 +254,30 @@ class B200VecEnv:
         self.sim.reset(sd, task_ids=task_ids, env_mask=mask)
         self._export_all_events()
         self._pending = True
+        self._idle = True
+
+    def set_next_episodes(self, env_indices, seeds=None, maps=None, tasks=None):
+        """Seed, map and / or tasks of the NEXT episode of envs `env_indices` (DESIGN.md 2.5): each env's next automatic
+        reset (the step after its episode ends) takes the fields given here instead of deriving them from the seed, and
+        then forgets them; fields not given stay derived.  tasks: one task-table row per env for all of its agents (as
+        the reference's Syllabus curriculum assigns them, syllabus_wrapper.py:129-150) or [n, agents_per_env].  Inputs
+        are Simulator.set_next's: host inputs are checked (ValueError), CUDA inputs cost no host synchronisation.
+
+        The first call switches the feature on, which synchronises the device once.  With an env pool only envs of the
+        batch the last recv() returned are accepted (the other batches may be stepping and consuming their entries), or
+        any env between a reset / load and the next send(); entries written between a batch's recv() and send() take
+        effect at that batch's next automatic resets.  The envs with no pending entry are those with
+        ``pool.sim.next_flags == 0``."""
+        t = self._torch
+        if self.sim.next_flags is None:
+            self.sim.set_next_episodes(True)
+        if self.num_batches > 1 and not self._idle and not (t.is_tensor(env_indices) and env_indices.is_cuda):
+            ids = np.asarray(env_indices.cpu() if t.is_tensor(env_indices) else env_indices, np.int64).reshape(-1)
+            lo, hi = self.batch_env_range
+            if ((ids < lo) | (ids >= hi)).any():
+                raise ValueError(f"envs {ids[(ids < lo) | (ids >= hi)].tolist()} are not in the batch the last recv() returned "
+                                 f"(envs [{lo}, {hi})): the other batches may be stepping")
+        self.sim.set_next(env_indices, seeds=seeds, maps=maps, tasks=tasks)
 
     def save_envs(self, env_indices):
         """Saved state of envs `env_indices` -> uint8 CUDA tensor [n, sim.state_bytes] (DESIGN.md 2.3).  Call it where
@@ -263,6 +293,7 @@ class B200VecEnv:
         self.sim.load_envs(env_indices, states)
         self._export_all_events()
         self._pending = True
+        self._idle = True
 
     def events(self):
         """(rows int32 CUDA [event_log_cap, 9], count int32 CUDA [1]): the player events of the step whose outputs the
@@ -392,6 +423,7 @@ class B200VecEnv:
         t = self._torch
         a = actions if t.is_tensor(actions) else t.as_tensor(np.asarray(actions))
         a = a.to(device=self.sim.obs.device, dtype=t.int32).reshape(self.envs_per_batch, self.agents_per_env, 12).contiguous()
+        self._idle = False
         if self.num_batches == 1:
             self.sim.step(a)
             if self._ev is not None:
