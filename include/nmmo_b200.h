@@ -37,7 +37,11 @@ enum nm_err { NM_OK = 0, NM_ERR_ARG = -1, NM_ERR_CUDA = -2, NM_ERR_LIMIT = -3, N
  * env / reward_wrapper namespaces).  maps: uint8 [n_maps][S][S] host memory (the reference loads
  * them from PATH_MAPS, environment.py:41).  tasks / task_embed: the curriculum
  * (environment.py:49) as int32 [n_tasks][NM_TASK_COLS] predicate rows (nmmo_spec.h: 12 columns) + fp16 [n_tasks][task_dim].
- * env_base: global index of this handle's env 0 (env sharding across GPUs). */
+ * env_base: global index of this handle's env 0 (env sharding across GPUs).
+ * NM_ERR_LIMIT, before anything is allocated on the device, for a record layout the kernels cannot write:
+ * N_ENT_OBS outside 1..255, N_INV outside 1..16, N_MKT_OBS or N_PRICE < 1, the twelve ActionTargets heads
+ * together > 1024 entries, TASK_DIM not a positive multiple of 8, or VISION outside 0..MAP_BORDER-1 (tile windows are
+ * read unclamped, and the far side of the spawn ring is MAP_BORDER tiles from the map edge). */
 int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, int n_fcfg, int n_envs, int device,
                 int env_base, const uint8_t *maps, int n_maps, const int32_t *tasks,
                 const uint16_t *task_embed, int n_tasks, nmmo_handle **out);
@@ -99,7 +103,8 @@ int nmmo_sample_actions(nmmo_handle *h, uint64_t seed, int32_t *actions_dev, voi
 
 /* Scripted survival policy for long benchmark runs (uniform-random agents starve within ~35 ticks): every agent walks
  * to the nearest water / foliage tile of its observation window when hungry, explores otherwise, never fights or
- * trades.  Reads only the observation records; writes DEVICE int32 [E][P][12]. */
+ * trades.  Reads only the observation records; writes DEVICE int32 [E][P][12].  NM_ERR_LIMIT for a tile window of more
+ * than 256 tiles (VISION > 7). */
 int nmmo_forage_actions(nmmo_handle *h, uint64_t seed, int32_t *actions_dev, void *stream);
 
 /* Built-in random policy: with a non-NULL DEVICE buffer int32 [E][P][12], every reset/step also

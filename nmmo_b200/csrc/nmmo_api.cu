@@ -317,6 +317,13 @@ extern "C" int nmmo_create(const int32_t *cfg, int n_cfg, const double *fcfg, in
   if (p.N > VBig::kNpcHash / 2) { return fail(NM_ERR_LIMIT, "NPC_N must be <= 2048"); }
   if (p.cfg[NC_NPC_SPAWN_ATTEMPTS] > 32) { return fail(NM_ERR_LIMIT, "NPC_SPAWN_ATTEMPTS must be <= 32"); }
   if (p.L.n_ent > 255 || p.cfg[NC_N_INV] > 16) { return fail(NM_ERR_LIMIT, "N_ENT_OBS <= 255, N_INV <= 16"); }
+  if (p.L.n_ent < 1 || p.L.n_mkt < 1 || p.L.n_inv < 1 || p.L.n_price < 1)
+    return fail(NM_ERR_LIMIT, "N_ENT_OBS, N_MKT_OBS, N_INV and N_PRICE must be >= 1");
+  // the Task block is copied in 16-byte vectors from embed + task_id * task_dim
+  if (p.L.task_dim <= 0 || p.L.task_dim % 8) return fail(NM_ERR_LIMIT, "TASK_DIM must be a positive multiple of 8");
+  // tile windows are read unclamped, and players stand on rows / columns MAP_BORDER .. MAP_BORDER + MAP_CENTER
+  // (= MAP_SIZE - MAP_BORDER, the far side of the spawn ring): a window wider than the border leaves the map
+  if (p.cfg[NC_VISION] < 0 || p.cfg[NC_VISION] >= p.cfg[NC_MAP_BORDER]) return fail(NM_ERR_LIMIT, "VISION must be in 0..MAP_BORDER-1");
   if (p.L.m_end > 1024) { return fail(NM_ERR_LIMIT, "the ActionTargets masks must total <= 1024 entries (one 32-entry word per lane)"); }
   if (p.cfg[NC_SPAWN_PATCH] > 0 && (p.cfg[NC_SPAWN_PATCH] * p.cfg[NC_SPAWN_PATCH] < p.P || p.cfg[NC_SPAWN_PATCH] > p.cfg[NC_MAP_CENTER]))
     return fail(NM_ERR_ARG, "SPAWN_PATCH^2 must hold PLAYER_N players and fit inside the map centre");
@@ -673,6 +680,7 @@ extern "C" int nmmo_sample_actions(nmmo_handle *h, uint64_t seed, int32_t *actio
 extern "C" int nmmo_forage_actions(nmmo_handle *h, uint64_t seed, int32_t *actions_dev, void *stream) {
   if (!h || !actions_dev) return fail(NM_ERR_ARG, "null argument");
   if ((uintptr_t)actions_dev & 15) return fail(NM_ERR_ARG, "actions must be 16-byte aligned");
+  if (h->prm.L.win * h->prm.L.win > 256) return fail(NM_ERR_LIMIT, "the forager searches tile windows of <= 256 tiles (VISION <= 7)");
   CU(cudaSetDevice(h->device));
   NmParams prm = h->prm;
   const int threads = 256, NW = threads / 32;

@@ -43,6 +43,63 @@ def build_world(agent="takeru", n_maps=4, map_seed=7, task_dim=None, env_over=No
     return cfg, fcfg, maps, tab, emb
 
 
+# Record layouts away from the reference's (100 entities, 384 market rows, 12 inventory rows, 99 prices, vision 7):
+# name -> (N_ENT_OBS, N_MKT_OBS, N_INV, N_PRICE, VISION, task_dim, world shape).  Widths of 31 / 32 / 33 mask entries
+# put a head's no-op on either side of a 32-entry mask word; "many entities" lets an agent see more than 32 entities.
+RECORD_LAYOUTS = {
+    "minimal": (1, 1, 1, 1, 3, 8, SMALL),
+    "truncating": (8, 8, 4, 5, 5, 24, SMALL),
+    "word_edges": (31, 31, 16, 31, 7, 64, SMALL),
+    "word_edges_plus_1": (32, 63, 15, 32, 8, 64, SMALL),
+    "many_entities": (255, 16, 4, 4, 9, 16, dict(NC_N_PLAYERS=64, NC_N_NPCS=64, NC_MAP_CENTER=24)),
+    "wide_buy": (60, 600, 12, 80, 4, 64, SMALL),
+}
+# agents that live long enough to pick up, list and buy items
+LONG_LIVED = dict(NC_RES_DEPLETION=1, NC_SPAWN_IMMUNITY=3)
+# with fill_market's actions, a world whose market outgrows a few rows: nobody starves, every harvest drops a weapon,
+# listings stay up for 400 ticks, NPCs are passive
+MARKET_FILLING = dict(NC_LISTING_DURATION=400, NC_RES_DEPLETION=0, NC_SPAWN_IMMUNITY=3, NC_WEAPON_DROP_THR=-1,
+                      NC_NPC_AGGR_PCT=200, NC_NPC_NEUT_PCT=200)
+
+
+def fill_market(acts, obs, L, rng):
+    """Edit random valid actions acts [E, P, 12] in place, given the records obs [E, P, stride] they were drawn from:
+    most agents list their first sellable item at a random price, nobody destroys or uses items, and only one agent in
+    four buys -- uniform-random play never lists more than a few items at a time; this outgrows a small Market block."""
+    so, sn = L.masks["Sell.InventoryItem"]
+    for e in range(acts.shape[0]):
+        for p in range(acts.shape[1]):
+            sellable = np.flatnonzero(obs[e, p, so:so + sn - 1])
+            if len(sellable) and rng.random() < 0.9:
+                acts[e, p, 9] = sellable[0]; acts[e, p, 10] = rng.integers(0, L.n_price)
+            acts[e, p, 3] = acts[e, p, 11] = L.n_inv
+            if p % 4:
+                acts[e, p, 2] = L.n_mkt
+    return acts
+
+
+def random_layouts(n, seed=2024):
+    """n record layouts drawn uniformly within what nmmo_create accepts: every width >= 1, N_ENT_OBS <= 255,
+    N_INV <= 16, N_PRICE <= 256, VISION < MAP_BORDER (16), TASK_DIM a multiple of 8, the twelve mask heads <= 1024."""
+    rng = np.random.default_rng(seed)
+    cfg = np.zeros(SPEC["NC_COUNT"], np.int32)
+    out = []
+    while len(out) < n:
+        n_ent, n_mkt, n_inv = int(rng.integers(1, 256)), int(rng.integers(1, 1000)), int(rng.integers(1, 17))
+        n_price, vision, task_dim = int(rng.integers(1, 257)), int(rng.integers(0, 16)), 8 * int(rng.integers(1, 65))
+        for k, v in zip(("NC_N_ENT_OBS", "NC_N_MKT_OBS", "NC_N_INV", "NC_N_PRICE"), (n_ent, n_mkt, n_inv, n_price)):
+            cfg[SPEC[k]] = v
+        if ObsLayout(cfg).m_end <= 1024:
+            out.append((n_ent, n_mkt, n_inv, n_price, vision, task_dim, SMALL))
+    return out
+
+
+def layout_world(layout, **engine_over):
+    n_ent, n_mkt, n_inv, n_price, vision, task_dim, shape = layout
+    return build_world(task_dim=task_dim, **shape, NC_N_ENT_OBS=n_ent, NC_N_MKT_OBS=n_mkt, NC_N_INV=n_inv,
+                       NC_N_PRICE=n_price, NC_VISION=vision, **engine_over)
+
+
 def describe_obs_mismatch(cfg, a, b):
     """Human-readable location of the first differing byte between two obs records."""
     L = ObsLayout(cfg)
